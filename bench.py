@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: image pairs/sec at 1920x1080 (BASELINE.json), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 A "step" = one pass of the whole hot path (pyramid, polynomial expansion, update-matrices, window blur + solve
 iterations, span sampling + classification) over one batch of B (default 32) synthetic 1920x1080 pairs with the reference's
@@ -201,17 +201,49 @@ class Resident:
         dist.barrier()
         return dist.reduce_max(float(ms.value))
 
-    def statuses(self):
+    def fetch(self):
+        """-> (results, vectors, cap) of the last run as tw_batch_fetch hands them to a caller (pair i's vectors at i * cap)."""
         cap = ((self.w + self.span - 1) // self.span) * ((self.h + self.span - 1) // self.span)
         vec = (self.tw.tw_vector * (cap * self.B))()
         res = (self.tw.tw_result * self.B)()
         self.check(self.lib.tw_batch_fetch(self.of.ctx, self.B, vec, cap, res), "fetch")
-        return [res[i].status for i in range(self.B)]
+        return res, vec, cap
+
+    def statuses(self):
+        return [r.status for r in self.fetch()[0]]
 
     def close(self):
         self.of.close()
         for pa, pb in self.pinned:
             self.lib.tw_host_free(pa); self.lib.tw_host_free(pb)
+
+
+DUMP_BYTES = 60 << 20  # all files of --dump-outputs together, .npy headers included: below 64 MB however counted
+
+
+def dump_outputs(out_dir, R, dense):
+    """Writes what the last step of the timed pass handed its caller, as .npy files a second build's run can be compared with:
+    status.npy and n_vectors.npy (one entry per pair), vectors.npy (pair, x, y, dx, dy per row, scan order) and, with the dense last
+    iteration, flow.npy (pair, pixel, dx / dy) at the pixels listed in flow_pixels.npy (row-major indices).  The pixels, and the
+    vectors if they would not fit, are a seeded sample so that the files stay within DUMP_BYTES."""
+    os.makedirs(out_dir, exist_ok=True)
+    res, vec, cap = R.fetch()
+    n = [min(r.n_vectors, cap) for r in res]
+    out = {"status": np.array([r.status for r in res], np.float64), "n_vectors": np.array([r.n_vectors for r in res], np.float64)}
+    if dense:
+        npx = R.w * R.h
+        px = np.sort(np.random.default_rng(0).choice(npx, min(npx, (DUMP_BYTES // 2) // (8 * R.B)), replace=False))
+        out["flow_pixels"] = px.astype(np.float64)
+        out["flow"] = np.stack([np.stack([f.ravel()[px] for f in R.of.batch_flow(i, R.w, R.h)], 1) for i in range(R.B)])
+    v = np.ctypeslib.as_array(vec).reshape(R.B, cap)
+    rows = np.concatenate([np.stack([np.full(k, i, np.float64), v[i, :k]["x"], v[i, :k]["y"], v[i, :k]["dx"], v[i, :k]["dy"]], 1)
+                           for i, k in enumerate(n)])
+    room = (DUMP_BYTES - sum(a.nbytes for a in out.values())) // (5 * 8)
+    if len(rows) > room:
+        rows = rows[np.sort(np.random.default_rng(1).choice(len(rows), room, replace=False))]
+    out["vectors"] = rows
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_pool(tw, lib, devices, B, cp, pinned, n_req, warm):
@@ -314,7 +346,7 @@ def main():
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=300)
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--batch", type=int, default=32, help="pairs per step = the dispatcher's batch (16 -> 32: +3 % pairs/s; 5.6 GB of device buffers)")
+    ap.add_argument("--batch", type=int, default=32, help="pairs per step = the dispatcher's batch (16 -> 32: +3 %% pairs/s; 5.6 GB of device buffers)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true", help="skip the e2e, variants and configs legs (profilers)")
@@ -326,7 +358,10 @@ def main():
     ap.add_argument("--last", default="sparse", choices=["sparse", "dense"],
                     help="last iteration of the finest scale: 'sparse' = evaluated at the sampled positions only (what the dispatcher "
                          "does: the Response carries vectors, not the field; bit-identical vectors), 'dense' = full flow field")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the b200 arm; the reference arm keeps none")
     if args.impl == "b200":
         args.warmup = max(args.warmup, 3)
 
@@ -358,10 +393,14 @@ def main():
     statuses = R.statuses()  # sanity: the warm-up results are real
     l0 = of.launch_count()
     sampler = ClockSampler(local_rank)
-    elapsed_ms = R.timed(args.steps, 0, dist)
-    clocks = sampler.stop()
+    try:
+        elapsed_ms = R.timed(args.steps, 0, dist)
+    finally:
+        clocks = sampler.stop()  # also on failure: the sampler must not outlive this process
     launches = of.launch_count() - l0
     value = tw.dist.whole_job_throughput(B * args.steps, world, elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, R, args.last == "dense")
 
     # ---- per-kernel-family pass: the same steps again with a CUDA event pair around every launch (the graph replay above
     # has no per-kernel events; with profiling on the library issues the identical launch sequence eagerly) ----
