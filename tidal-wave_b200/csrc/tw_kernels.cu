@@ -1209,8 +1209,11 @@ cudaError_t launch_first_update(cudaStream_t s, const FirstUpdateArgs &a)
     dim3 grid((a.d.w + 31) / 32, (a.d.h + 7) / 8, a.batch);
     if (a.ufma) return cudaErrorNotSupported; // "update_fma" was removed from the library (see launch_gauss_mr)
     {
-        if (a.d.pitch == 2048) first_update_kernel<2048, false><<<grid, dim3(32, 8), 0, s>>>(a);
-        else if (a.d.pitch == 4096) first_update_kernel<4096, false><<<grid, dim3(32, 8), 0, s>>>(a);
+        // the compile-time pitch stands for both levels: only when the coarse flow has the same row pitch ("tight_pitch" gives
+        // every level its own, e.g. 2048 over 1024)
+        const bool one_pitch = !a.coarse || a.cd.pitch == a.d.pitch;
+        if (one_pitch && a.d.pitch == 2048) first_update_kernel<2048, false><<<grid, dim3(32, 8), 0, s>>>(a);
+        else if (one_pitch && a.d.pitch == 4096) first_update_kernel<4096, false><<<grid, dim3(32, 8), 0, s>>>(a);
         else first_update_kernel<0, false><<<grid, dim3(32, 8), 0, s>>>(a);
     }
     return cudaGetLastError();

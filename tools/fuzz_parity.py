@@ -12,8 +12,27 @@ n = int(sys.argv[1]) if len(sys.argv) > 1 else 60
 rng = np.random.default_rng(int(sys.argv[2]) if len(sys.argv) > 2 else 1)
 O = RefOracle()
 bad = 0
+
+
+def draw_size():
+    """Mostly ordinary frames; one in eight smaller than the window (a one-scale pyramid below 32 px), one in eight around
+    the row-pitch classes: 2048 / 4096 (W = pitch: no padding after the last column) and above 4096 (runtime pitch, a multiple
+    of 32 or ragged), short so the oracle stays fast."""
+    r = int(rng.integers(8))
+    if r == 0:
+        w, h = int(rng.integers(1, 33)), int(rng.integers(1, 300))
+        return (w, h) if rng.integers(2) else (h, w)
+    if r == 1:
+        if rng.integers(2):
+            w = int(rng.choice([2048, 4096])) + int(rng.integers(-1, 2))
+        else:
+            w = 32 * int(rng.integers(129, 241)) + (int(rng.integers(1, 32)) if rng.integers(2) else 0)
+        return w, int(rng.integers(16, 160))
+    return int(rng.integers(33, 720)), int(rng.integers(33, 520))
+
+
 for case in range(n):
-    w, h = int(rng.integers(33, 720)), int(rng.integers(33, 520))
+    w, h = draw_size()
     kw = {}
     kind = int(rng.integers(6))
     if kind == 0:
@@ -26,7 +45,7 @@ for case in range(n):
         kw = dict(pyrScale=float(rng.choice([0.5, 0.6, 0.8])), pyrLevels=int(rng.integers(1, 5)))
     batch = int(rng.integers(1, 4))
     opts = {"window_tiles": int(rng.integers(2)), "sparse_last": int(rng.integers(2)), "box_unfused": int(rng.integers(2)) if kind == 0 else 0,
-            "polyexp_tma": int(rng.integers(2)), "level_generic": 1 if rng.integers(8) == 0 else 0}
+            "polyexp_tma": int(rng.integers(2)), "level_generic": 1 if rng.integers(8) == 0 else 0, "tight_pitch": int(rng.integers(2))}
     thr, span = float(rng.choice([0.3, 0.6, 5.0])), int(rng.choice([7, 10, 16]))
     pairs = [tw.synth.make_pair("S" if rng.integers(2) else "T", w, h, int(rng.integers(1000)), defect=bool(rng.integers(2))) for _ in range(batch)]
     p = tw.OpticalFlowParameter(**kw)
