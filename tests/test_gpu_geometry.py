@@ -11,20 +11,20 @@ cfg3 only, everything else is faithful whatever a says):
 
   case (W x H, options, switches)                      instantiation reached
   ---------------------------------------------------  ---------------------------------------------------------------------
-  4097 / 5120 / 7680, default, a = 0, window_tiles 1   gauss_iter2_kernel<15, 0, false, 0>, polyexp_fast_kernel<7, 0>
-  4097 / 5120 / 7680, default, a = 1, window_tiles 1   gauss_iter2_kernel<15, 2, false, 0>, polyexp_mixed_kernel<7, 0>
+  4097 / 5120 / 7680, default, a = 0, window_tiles 1   gauss_iter2_kernel<15, 0, 0>, polyexp_fast_kernel<7, 0>
+  4097 / 5120 / 7680, default, a = 1, window_tiles 1   gauss_iter2_kernel<15, 2, 0>, polyexp_mixed_kernel<7, 0>
                                  (polyexp_tma 1 / 0)   polyexp_mixed_kernel<7, 0> with and without the TMA input tile
   4097 / 5120 / 7680, default, window_tiles 0          gauss_strip_kernel<0|2, *> with tensor-map strides of pitch 4128 /
                                                        5120 / 7680 (5120, 7680: zero slack)
   2049 / 4096, default, window_tiles 0                 gauss_strip_kernel at pitch 4096 (4096: zero slack)
-  2048 / 4096, default                                 gauss_iter2_kernel<15, *, false, 2048 / 4096> at zero slack
-  4096, g15n5                                          gauss_iter2_kernel<7, 0, false, 4096>, polyexp_fast_kernel<5, 4096>
-  5120 / 7680, g15n5                                   gauss_iter2_kernel<7, 0, false, 0>, polyexp_fast_kernel<5, 0>,
+  2048 / 4096, default                                 gauss_iter2_kernel<15, *, 2048 / 4096> at zero slack
+  4096, g15n5                                          gauss_iter2_kernel<7, 0, 4096>, polyexp_fast_kernel<5, 4096>
+  5120 / 7680, g15n5                                   gauss_iter2_kernel<7, 0, 0>, polyexp_fast_kernel<5, 0>,
                                  (sparse_last 1)       one-row gauss_last_sparse_kernel (radius 7) at runtime pitch
   4096 / 5120 / 7680, cfg4 and box31, box_unfused 0    box_ckpt_kernel + box_band_kernel at pitch 4096 / runtime pitch
                                       box_unfused 1    box_vsum_kernel + box_hscan_kernel (+ first_update_kernel) likewise
   4097 / 5120, winSize 20                              gauss_iter_generic_kernel at runtime pitch
-  every W > 4096                                       first_update_kernel<0, false>
+  every W > 4096                                       first_update_kernel<0>
   every W > 4096, default, sparse_last 1               gauss_last_sparse3_kernel at runtime pitch
   2048 / 2049 / 4096 / 4097, tight_pitch 1             per-level pitches (e.g. 2048 | 1024 | 512 | 256 at W = 2048): the
                                                        coarse levels run the PITCH = 0 instantiations of every kernel above

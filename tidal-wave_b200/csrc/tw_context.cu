@@ -40,6 +40,30 @@ struct Scale {
     TileMap imap = {};      // tensor map of the level images (poly-exp input tiles by TMA)
 };
 
+// The run-time switches that change the launch sequence of a plan without rebuilding it: part of the graph key.
+struct LaunchOptions {
+    int arith = 1;        // 0 = faithful (App. A operation order), 1 = relaxed where validated (relaxed_in_effect)
+    int sparse_last = 0;  // 1: last iteration of the finest scale only at the span-grid points (no dense flow field)
+    int window_tiles = 1; // 1 (default): the tile-per-CTA window kernel (gauss_iter2_kernel); 0: the persistent TMA-fed strip kernel (tw_window.cu),
+                          // bit-identical and measured 1-7 % slower (DESIGN.md section 4.2)
+    int box_unfused = 0;  // 1: the three-launch box iteration (V plane through HBM), kept for the parity tests
+    int level_generic = 0, level_unfused = 0;
+    bool operator==(const LaunchOptions &o) const
+    {
+        return arith == o.arith && sparse_last == o.sparse_last && window_tiles == o.window_tiles && box_unfused == o.box_unfused &&
+               level_generic == o.level_generic && level_unfused == o.level_unfused;
+    }
+};
+
+// A plan's CUDA graph of the launch sequence (enqueue) is captured for one (n, threshold, span, options, result buffer) key
+struct GraphKey {
+    int n = 0; double thr = 0; int span = 0; LaunchOptions opt; const void *vectors = nullptr; int dev_cap = 0;
+    bool operator==(const GraphKey &o) const
+    {
+        return n == o.n && thr == o.thr && span == o.span && opt == o.opt && vectors == o.vectors && dev_cap == o.dev_cap;
+    }
+};
+
 struct Plan {
     bool valid = false;
     int W = 0, H = 0, batch = 0, keep = 0;
@@ -53,6 +77,11 @@ struct Plan {
     double *V = nullptr; // box only
     float *T = nullptr;  // long pre-blur levels only: row-pass intermediate of launch_level_image_big
     bool fused_levels = false;
+    // captured launch sequence (run_sequence): graph_exec replays graph_key; seen_key is the key of the last eager run
+    GraphKey graph_key, seen_key;
+    cudaGraphExec_t graph_exec = nullptr;
+    long long graph_launches = 0;
+    unsigned long long last_use = 0; // in the plan cache: the least recently used plan is evicted first
 };
 
 } // namespace
@@ -64,39 +93,16 @@ struct tw_ctx {
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr, ev_r0 = nullptr, ev_r1 = nullptr;
     Plan plan;
     int keep_levels = 0;
-    int opt_sparse_last = 0; // 1: last iteration of the finest scale only at the span-grid points (no dense flow field)
     bool last_sparse = false; // the previous run left no dense field
-    int opt_update_fma = 0; // studied opt-in (oracle relax bit 6), never part of "arithmetic" = 1
-    int opt_gauss_fma = 0, opt_gauss_scalar = 0, opt_level_generic = 0, opt_level_unfused = 0, opt_tight_pitch = 0;
+    LaunchOptions opt;
+    int opt_graph = 1;  // replay the launch sequence of a batch from a captured CUDA graph
+    // options that change how plans are built: setting one rebuilds the plan
+    int opt_tight_pitch = 0;
     int opt_poly_no_tma = 1;  // 0 ("polyexp_tma" = 1, TW_POLY_TMA=1): interior input tiles of the relaxed poly-exp staged by one TMA tile copy --
                               // bit-identical, measured 5 % slower than the per-thread loads (0.697 vs 0.662 ms per step), hence opt-in
-    int opt_box_unfused = 0;  // 1: the three-launch box iteration (V plane through HBM), kept for the parity tests
-    int opt_window_tiles = 1; // 1 (default): the tile-per-CTA window kernel (gauss_iter2_kernel); 0: the persistent TMA-fed strip kernel (tw_window.cu),
-                              // bit-identical and measured 1-7 % slower (DESIGN.md section 4.2)
-    int opt_arith = 1;  // 0 = faithful (App. A operation order), 1 = relaxed where validated (relaxed_in_effect)
-    int opt_graph = 1;  // replay the launch sequence of a batch from a captured CUDA graph
-    // CUDA graph of the launch sequence (enqueue) for one (plan, n, threshold, span, options) key
-    struct GraphKey {
-        unsigned long long plan_gen = 0; int n = 0; double thr = 0; int span = 0; int opts = 0; const void *vectors = nullptr; int dev_cap = 0;
-        bool operator==(const GraphKey &o) const
-        {
-            return plan_gen == o.plan_gen && n == o.n && thr == o.thr && span == o.span && opts == o.opts && vectors == o.vectors && dev_cap == o.dev_cap;
-        }
-    };
-    GraphKey graph_key, seen_key;
-    cudaGraphExec_t graph_exec = nullptr;
-    long long graph_launches = 0;
-    unsigned long long plan_gen = 0, next_gen = 0;
     // Plans (all device buffers, tables and tensor maps of one (size, parameters)) that are not the current one, each with its
     // captured graph: screenshot directories mix page sizes, and rebuilding a plan costs tens of cudaMalloc / cudaFree calls.
-    struct PlanSlot {
-        Plan plan;
-        GraphKey graph_key, seen_key;
-        cudaGraphExec_t graph_exec = nullptr;
-        long long graph_launches = 0;
-        unsigned long long gen = 0, last_use = 0;
-    };
-    std::vector<PlanSlot> plan_cache;
+    std::vector<Plan> plan_cache;
     unsigned long long use_tick = 0;
     int plan_cache_max = 3; // + the current plan (TW_PLAN_CACHE)
     // results
@@ -159,54 +165,42 @@ bool set_err(tw_ctx *c, const char *what, cudaError_t e)
         if (e_ != cudaSuccess) { set_err(ctx, #call, e_); return false; } \
     } while (0)
 
-void drop_graph(tw_ctx *ctx)
+void drop_graph(Plan &pl)
 {
-    if (ctx->graph_exec) { cudaGraphExecDestroy(ctx->graph_exec); ctx->graph_exec = nullptr; }
-    ctx->graph_key = tw_ctx::GraphKey();
-    ctx->seen_key = tw_ctx::GraphKey();
+    if (pl.graph_exec) { cudaGraphExecDestroy(pl.graph_exec); pl.graph_exec = nullptr; }
+    pl.graph_key = GraphKey();
+    pl.seen_key = GraphKey();
 }
 
-void free_plan(tw_ctx *ctx)
+// Frees the plan's device buffers and its graph (stream idle).
+void free_plan(Plan &pl)
 {
-    drop_graph(ctx);
-    ctx->plan_gen = ++ctx->next_gen;
-    for (void *p : ctx->plan.allocs) cudaFree(p);
-    ctx->plan = Plan();
-}
-
-void free_slot(tw_ctx::PlanSlot &s)
-{
-    if (s.graph_exec) cudaGraphExecDestroy(s.graph_exec);
-    for (void *p : s.plan.allocs) cudaFree(p);
-    s = tw_ctx::PlanSlot();
+    drop_graph(pl);
+    for (void *p : pl.allocs) cudaFree(p);
+    pl = Plan();
 }
 
 // Frees every cached plan (stream idle): options that change how plans are built, out-of-memory, destruction.
 void flush_plan_cache(tw_ctx *ctx)
 {
-    for (auto &s : ctx->plan_cache) free_slot(s);
+    for (Plan &pl : ctx->plan_cache) free_plan(pl);
     ctx->plan_cache.clear();
 }
 
 // The current plan (valid or not) leaves ctx->plan: into the cache with its graph, or freed.  Stream idle.
 void stash_plan(tw_ctx *ctx)
 {
-    if (!ctx->plan.valid || ctx->plan_cache_max < 1) { free_plan(ctx); return; }
+    if (!ctx->plan.valid || ctx->plan_cache_max < 1) { free_plan(ctx->plan); return; }
     while ((int)ctx->plan_cache.size() >= ctx->plan_cache_max) { // evict the least recently used
         size_t lru = 0;
         for (size_t i = 1; i < ctx->plan_cache.size(); i++)
             if (ctx->plan_cache[i].last_use < ctx->plan_cache[lru].last_use) lru = i;
-        free_slot(ctx->plan_cache[lru]);
+        free_plan(ctx->plan_cache[lru]);
         ctx->plan_cache.erase(ctx->plan_cache.begin() + lru);
     }
-    tw_ctx::PlanSlot s;
-    s.plan = std::move(ctx->plan);
-    s.graph_key = ctx->graph_key; s.seen_key = ctx->seen_key; s.graph_exec = ctx->graph_exec; s.graph_launches = ctx->graph_launches;
-    s.gen = ctx->plan_gen; s.last_use = ++ctx->use_tick;
-    ctx->plan_cache.push_back(std::move(s));
+    ctx->plan.last_use = ++ctx->use_tick;
+    ctx->plan_cache.push_back(std::move(ctx->plan));
     ctx->plan = Plan();
-    ctx->graph_exec = nullptr; ctx->graph_key = tw_ctx::GraphKey(); ctx->seen_key = tw_ctx::GraphKey(); ctx->graph_launches = 0;
-    ctx->plan_gen = ++ctx->next_gen;
 }
 
 template <typename T>
@@ -375,19 +369,21 @@ bool same_param(const tw_flow_param &a, const tw_flow_param &b)
            a.pyrIterations == b.pyrIterations && a.polyN == b.polyN && a.polySigma == b.polySigma && a.flags == b.flags;
 }
 
+// Whether pl is a valid plan for W x H frames, parameters p and the context's batch size and keep_levels.
+bool plan_fits(const tw_ctx *ctx, const Plan &pl, int W, int H, const tw_flow_param &p)
+{
+    return pl.valid && pl.W == W && pl.H == H && pl.batch == ctx->max_batch && pl.keep == ctx->keep_levels && same_param(pl.p, p);
+}
+
 bool build_plan(tw_ctx *ctx, int W, int H, const tw_flow_param &p)
 {
     Plan &pl = ctx->plan;
-    if (pl.valid && pl.W == W && pl.H == H && pl.batch == ctx->max_batch && pl.keep == ctx->keep_levels && same_param(pl.p, p))
-        return true;
+    if (plan_fits(ctx, pl, W, H, p)) return true;
     CK(cudaStreamSynchronize(ctx->stream));
     stash_plan(ctx);
     for (size_t i = 0; i < ctx->plan_cache.size(); i++) { // a plan of this size and these parameters from before?
-        tw_ctx::PlanSlot &s = ctx->plan_cache[i];
-        if (s.plan.valid && s.plan.W == W && s.plan.H == H && s.plan.batch == ctx->max_batch && s.plan.keep == ctx->keep_levels && same_param(s.plan.p, p)) {
-            ctx->plan = std::move(s.plan);
-            ctx->graph_key = s.graph_key; ctx->seen_key = s.seen_key; ctx->graph_exec = s.graph_exec; ctx->graph_launches = s.graph_launches;
-            ctx->plan_gen = s.gen;
+        if (plan_fits(ctx, ctx->plan_cache[i], W, H, p)) {
+            pl = std::move(ctx->plan_cache[i]);
             ctx->plan_cache.erase(ctx->plan_cache.begin() + i);
             return true;
         }
@@ -592,7 +588,7 @@ bool ensure_results(tw_ctx *ctx, int cap)
 // always run the faithful kernels.
 bool relaxed_in_effect(const tw_ctx *ctx, const tw_flow_param &p)
 {
-    return ctx->opt_arith == 1 && (p.flags & 256) && p.winSize >= 30 && p.polyN == 7;
+    return ctx->opt.arith == 1 && (p.flags & 256) && p.winSize >= 30 && p.polyN == 7;
 }
 
 // Whether a run with this span ends in the sparse last iteration (K5s): then no dense flow field exists afterwards.
@@ -600,7 +596,7 @@ bool sparse_in_effect(const tw_ctx *ctx, int span)
 {
     const Plan &pl = ctx->plan;
     const tw_flow_param &p = pl.p;
-    if (!(span > 0 && ctx->opt_sparse_last && (p.flags & 256) && p.pyrIterations > 0 && (pl.win.m == 15 || pl.win.m == 7))) return false;
+    if (!(span > 0 && ctx->opt.sparse_last && (p.flags & 256) && p.pyrIterations > 0 && (pl.win.m == 15 || pl.win.m == 7))) return false;
     IterArgs ia{};
     ia.span = span;
     return gauss_last_sparse_ok(ia, pl.win);
@@ -621,7 +617,7 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
         cudaError_t e = cudaMemsetAsync(ctx->d_counts, 0, sizeof(int) * n, ctx->stream);
         if (e != cudaSuccess) { set_err(ctx, "memset counts", e); return false; }
     }
-    const bool fused_levels = pl.fused_levels && !ctx->opt_level_generic && !ctx->opt_level_unfused;
+    const bool fused_levels = pl.fused_levels && !ctx->opt.level_generic && !ctx->opt.level_unfused;
     const size_t fbase = ns >= 4 ? ns - 4 : 0; // first scale produced by the fused kernel
     if (fused_levels) {
         float *dst[4]; LevelDims dd[4];
@@ -647,8 +643,8 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
         // I planes of a batch are laid out [B][2]: the u8 source is [B][2] too, so image index = blockIdx.z.
         if (!fused_levels || si < fbase) {
             LaunchScope ls_(ctx, F_LEVEL, n * (2 * P0 + 8 * Pl));
-            cudaError_t e_ = ctx->opt_level_generic ? cudaErrorNotSupported : launch_level_image_fast(ctx->stream, la, s.host_taps.data(), s.int_scale);
-            if (e_ == cudaErrorNotSupported && !ctx->opt_level_generic && pl.T && level_image_big_ok(la)) e_ = launch_level_image_big(ctx->stream, la, pl.T);
+            cudaError_t e_ = ctx->opt.level_generic ? cudaErrorNotSupported : launch_level_image_fast(ctx->stream, la, s.host_taps.data(), s.int_scale);
+            if (e_ == cudaErrorNotSupported && !ctx->opt.level_generic && pl.T && level_image_big_ok(la)) e_ = launch_level_image_big(ctx->stream, la, pl.T);
             if (e_ == cudaErrorNotSupported) e_ = launch_level_image(ctx->stream, la);
             if (e_ != cudaSuccess) { set_err(ctx, "launch_level_image", e_); return false; }
         }
@@ -661,7 +657,6 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
         }
         fa.inv_scale = (float)(1. / p.pyrScale);
         fa.R = s.R; fa.d = s.d; fa.batch = n;
-        fa.ufma = (relaxed && ctx->opt_update_fma) ? 1 : 0;
         fa.M = p.pyrIterations > 0 ? s.M0 : nullptr;
         fa.flow_out = p.pyrIterations > 0 ? nullptr : s.flow;
         double cbytes = si > 0 ? 8.0 * pl.scales[si - 1].d.w * pl.scales[si - 1].d.h : 0.0;
@@ -673,19 +668,17 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
             ia.Min = Min; ia.Mout = Mout; ia.R = s.R; ia.flow = s.flow; ia.d = s.d; ia.batch = n;
             ia.last = (it == p.pyrIterations - 1);
             if (fused_count && ia.last && si + 1 == ns) { ia.span = span; ia.thr2 = threshold * threshold; ia.counts = ctx->d_counts; }
-            ia.fma = relaxed ? 2 : (ctx->opt_gauss_fma ? 1 : 0);
-            ia.ufma = (ia.fma == 2 && ctx->opt_update_fma) ? 1 : 0;
-            ia.scalar = ctx->opt_gauss_scalar;
+            ia.fma = relaxed ? 2 : 0;
             double bytes = n * (ia.last ? 28 : 80) * Pl;
             if (ia.span > 0 && sparse_in_effect(ctx, span)) {
                 // classification only: blur + solve at the sampled positions (one pass over M, no flow plane written)
                 LAUNCH(F_GLAST, n * 20.0 * Pl, launch_gauss_last_sparse(ctx->stream, ia, pl.win));
-            } else if ((p.flags & 256) && ctx->opt_window_tiles == 0 && gauss_strip_ok(ia, pl.win) &&
+            } else if ((p.flags & 256) && ctx->opt.window_tiles == 0 && gauss_strip_ok(ia, pl.win) &&
                        s.maps[Min == s.M1 ? 1 : 0].valid) {
                 LAUNCH(ia.last ? F_GLAST : F_GITER, bytes, launch_gauss_strip(ctx->stream, ia, pl.win, s.maps[Min == s.M1 ? 1 : 0]));
             } else if (p.flags & 256) {
                 LAUNCH(ia.last ? F_GLAST : F_GITER, bytes, launch_gauss_iter(ctx->stream, ia, pl.win));
-            } else if (!ctx->opt_box_unfused && box_fused_ok(s.d, p.winSize / 2)) {
+            } else if (!ctx->opt.box_unfused && box_fused_ok(s.d, p.winSize / 2)) {
                 // fused box iteration: band checkpoints of the vertical running sums, then blur + solve + update in one kernel
                 LAUNCH(F_BVSUM, n * 20.0 * Pl, launch_box_ckpt(ctx->stream, Min, pl.V, s.d, n, p.winSize / 2));
                 LAUNCH(ia.last ? F_BLAST : F_BITER, n * (ia.last ? 28.0 : 80.0) * Pl - n * 20.0 * Pl,
@@ -696,7 +689,6 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
                 if (!ia.last) {
                     FirstUpdateArgs ua{};
                     ua.flow_in = s.flow; ua.R = s.R; ua.M = Mout; ua.d = s.d; ua.batch = n; ua.inv_scale = 1.f;
-                    ua.ufma = 0;
                     LAUNCH(F_BUPD, 0.0, launch_first_update(ctx->stream, ua));
                 }
             }
@@ -722,24 +714,24 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
 bool run_sequence(tw_ctx *ctx, int n, double threshold, int span)
 {
     if (!ctx->opt_graph || ctx->profiling) return enqueue(ctx, n, threshold, span);
-    tw_ctx::GraphKey key;
-    key.plan_gen = ctx->plan_gen; key.n = n; key.thr = threshold; key.span = span;
-    key.opts = ctx->opt_gauss_fma | ctx->opt_gauss_scalar << 1 | ctx->opt_level_generic << 2 | ctx->opt_level_unfused << 3 | ctx->opt_arith << 4 | ctx->opt_update_fma << 5 | ctx->opt_sparse_last << 6 | ctx->opt_window_tiles << 7 | ctx->opt_box_unfused << 9;
+    Plan &pl = ctx->plan;
+    GraphKey key;
+    key.n = n; key.thr = threshold; key.span = span; key.opt = ctx->opt;
     key.vectors = ctx->d_vectors; key.dev_cap = ctx->dev_cap; // the captured sample kernel bakes both in
-    if (ctx->graph_exec && key == ctx->graph_key) {
-        cudaError_t e = cudaGraphLaunch(ctx->graph_exec, ctx->stream);
+    if (pl.graph_exec && key == pl.graph_key) {
+        cudaError_t e = cudaGraphLaunch(pl.graph_exec, ctx->stream);
         if (e != cudaSuccess) { set_err(ctx, "cudaGraphLaunch", e); return false; }
-        ctx->launches += ctx->graph_launches;
+        ctx->launches += pl.graph_launches;
         return true;
     }
-    if (!(key == ctx->seen_key)) { // first run of this key: eager
+    if (!(key == pl.seen_key)) { // first run of this key: eager
         if (!enqueue(ctx, n, threshold, span)) return false;
-        ctx->seen_key = key;
-        ctx->seen_key.vectors = ctx->d_vectors; ctx->seen_key.dev_cap = ctx->dev_cap; // enqueue may have (re)allocated the result buffer
+        pl.seen_key = key;
+        pl.seen_key.vectors = ctx->d_vectors; pl.seen_key.dev_cap = ctx->dev_cap; // enqueue may have (re)allocated the result buffer
         return true;
     }
     // second run: capture, instantiate, launch
-    if (ctx->graph_exec) { cudaGraphExecDestroy(ctx->graph_exec); ctx->graph_exec = nullptr; }
+    if (pl.graph_exec) { cudaGraphExecDestroy(pl.graph_exec); pl.graph_exec = nullptr; }
     const long long before = ctx->launches;
     cudaGraph_t graph = nullptr;
     cudaError_t e = cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal);
@@ -759,17 +751,17 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span)
         if (!ok) return false;
         return enqueue(ctx, n, threshold, span);
     }
-    e = cudaGraphInstantiate(&ctx->graph_exec, graph, 0);
+    e = cudaGraphInstantiate(&pl.graph_exec, graph, 0);
     cudaGraphDestroy(graph);
     if (e != cudaSuccess) {
         cudaGetLastError();
-        ctx->graph_exec = nullptr;
+        pl.graph_exec = nullptr;
         ctx->opt_graph = 0;
         return enqueue(ctx, n, threshold, span);
     }
-    ctx->graph_key = key;
-    ctx->graph_launches = captured;
-    e = cudaGraphLaunch(ctx->graph_exec, ctx->stream);
+    pl.graph_key = key;
+    pl.graph_launches = captured;
+    e = cudaGraphLaunch(pl.graph_exec, ctx->stream);
     if (e != cudaSuccess) { set_err(ctx, "cudaGraphLaunch", e); return false; }
     ctx->launches += captured;
     return true;
@@ -834,11 +826,11 @@ tw_ctx *tw_create(int device, int max_w, int max_h, int max_batch, char *err, in
     }
     tw_ctx *ctx = new tw_ctx();
     ctx->device = device; ctx->max_w = max_w; ctx->max_h = max_h; ctx->max_batch = max_batch < 1 ? 1 : max_batch;
-    ctx->opt_arith = default_arith();
+    ctx->opt.arith = default_arith();
     if (const char *g = getenv("TW_GRAPH")) ctx->opt_graph = atoi(g) ? 1 : 0; // TW_GRAPH=0: eager launches (profilers)
     if (const char *g = getenv("TW_PLAN_CACHE")) ctx->plan_cache_max = atoi(g) < 0 ? 0 : atoi(g);
     if (const char *g = getenv("TW_POLY_TMA")) ctx->opt_poly_no_tma = atoi(g) ? 0 : 1;
-    if (const char *g = getenv("TW_WINDOW")) ctx->opt_window_tiles = !strcmp(g, "strip") ? 0 : 1; // TW_WINDOW=strip|tiles
+    if (const char *g = getenv("TW_WINDOW")) ctx->opt.window_tiles = !strcmp(g, "strip") ? 0 : 1; // TW_WINDOW=strip|tiles
     if ((e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess) { delete ctx; return fail(cudaGetErrorString(e)); }
     cudaEventCreate(&ctx->ev_t0); cudaEventCreate(&ctx->ev_t1); cudaEventCreate(&ctx->ev_r0); cudaEventCreate(&ctx->ev_r1);
     if ((e = cudaMalloc(&ctx->d_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
@@ -856,7 +848,7 @@ void tw_destroy(tw_ctx *ctx)
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     drain_profile(ctx);
-    free_plan(ctx);
+    free_plan(ctx->plan);
     flush_plan_cache(ctx);
     for (auto e : ctx->ev_pool) cudaEventDestroy(e);
     if (ctx->d_counts) cudaFree(ctx->d_counts);
@@ -981,7 +973,7 @@ int tw_batch_run(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, d
     if (span < 0) { ctx->err = "bad span"; return TW_BAD_PARAMETER; }
     cudaSetDevice(ctx->device);
     Plan &pl = ctx->plan;
-    if (!(pl.valid && pl.W == w && pl.H == h && pl.batch == ctx->max_batch && pl.keep == ctx->keep_levels)) {
+    if (!plan_fits(ctx, pl, w, h, pl.p)) { // images of this size resident (under whichever parameters)
         ctx->err = "tw_batch_run: no uploaded images of this size";
         return TW_BAD_PARAMETER;
     }
@@ -1122,8 +1114,7 @@ int tw_pipe_submit(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8
     for (int i = 0; i < n; i++)
         if (!expect[i] || !target[i]) { ctx->err = "null image"; return TW_BAD_IMAGE_FORMAT; }
     cudaSetDevice(ctx->device);
-    const Plan &pl0 = ctx->plan;
-    const bool same_plan = pl0.valid && pl0.W == w && pl0.H == h && pl0.batch == ctx->max_batch && pl0.keep == ctx->keep_levels && same_param(pl0.p, *param);
+    const bool same_plan = plan_fits(ctx, ctx->plan, w, h, *param);
     if (!same_plan && pp.count > 0) { ctx->err = "tw_pipe_submit: size / parameters changed, collect the pending batch first"; return TW_BAD_PARAMETER; }
     if (!build_plan(ctx, w, h, *param)) return TW_CUDA_ERROR;
     Plan &pl = ctx->plan;
@@ -1330,14 +1321,14 @@ long long tw_launch_count(tw_ctx *ctx) { return ctx ? ctx->launches : 0; }
 int tw_set_option(tw_ctx *ctx, const char *name, int value)
 {
     if (!ctx || !name) return TW_BAD_PARAMETER;
-    if (!strcmp(name, "arithmetic")) { ctx->opt_arith = value ? 1 : 0; return TW_OK; }
-    if (!strcmp(name, "graph")) { ctx->opt_graph = value ? 1 : 0; if (!value) drop_graph(ctx); return TW_OK; }
+    if (!strcmp(name, "arithmetic")) { ctx->opt.arith = value ? 1 : 0; return TW_OK; }
+    if (!strcmp(name, "graph")) { ctx->opt_graph = value ? 1 : 0; if (!value) drop_graph(ctx->plan); return TW_OK; }
     if (!strcmp(name, "gauss_fma") || !strcmp(name, "update_fma") || !strcmp(name, "gauss_scalar")) {
         // studied and rejected relaxations (oracle relax bits 0 / 6) and the scalar v1 window kernel: no longer in the library
         if (value) { ctx->err = std::string(name) + ": removed from the library (DESIGN.md section 2)"; return TW_UNSUPPORTED; }
         return TW_OK;
     }
-    if (!strcmp(name, "sparse_last")) { ctx->opt_sparse_last = value ? 1 : 0; return TW_OK; }
+    if (!strcmp(name, "sparse_last")) { ctx->opt.sparse_last = value ? 1 : 0; return TW_OK; }
     if (!strcmp(name, "polyexp_tma")) { // takes effect when the next plan is built (the tensor maps are made with the plan)
         ctx->opt_poly_no_tma = value ? 0 : 1;
         ctx->plan.valid = false;
@@ -1345,10 +1336,10 @@ int tw_set_option(tw_ctx *ctx, const char *name, int value)
         flush_plan_cache(ctx);
         return TW_OK;
     }
-    if (!strcmp(name, "box_unfused")) { ctx->opt_box_unfused = value ? 1 : 0; return TW_OK; }
-    if (!strcmp(name, "window_tiles")) { ctx->opt_window_tiles = value ? 1 : 0; return TW_OK; }
-    if (!strcmp(name, "level_generic")) { ctx->opt_level_generic = value ? 1 : 0; return TW_OK; }
-    if (!strcmp(name, "level_unfused")) { ctx->opt_level_unfused = value ? 1 : 0; return TW_OK; }
+    if (!strcmp(name, "box_unfused")) { ctx->opt.box_unfused = value ? 1 : 0; return TW_OK; }
+    if (!strcmp(name, "window_tiles")) { ctx->opt.window_tiles = value ? 1 : 0; return TW_OK; }
+    if (!strcmp(name, "level_generic")) { ctx->opt.level_generic = value ? 1 : 0; return TW_OK; }
+    if (!strcmp(name, "level_unfused")) { ctx->opt.level_unfused = value ? 1 : 0; return TW_OK; }
     if (!strcmp(name, "tight_pitch")) {
         ctx->opt_tight_pitch = value ? 1 : 0;
         ctx->plan.valid = false;

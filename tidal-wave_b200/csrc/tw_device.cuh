@@ -37,10 +37,10 @@ __device__ __forceinline__ const float *M_channel(const float *Mb, int pitch, in
 }
 
 
-// UF = validated relaxation (oracle relax bit 6): fmaf chains in the bilinear blend, the flow terms and the outer
-// products (same association order as App. A.4); UF = false keeps the oracle's mul / add sequence (-fmad=false TU).
+// The oracle's mul / add sequence of App. A.4 (-fmad=false TU: no contraction).  BORDER = false: the caller knows the pixel
+// is outside the damped 5-pixel frame border.
 // pt / pb = R1 at rows y1 / y1+1, columns (x1, x1+1); q = R0 at (x, y).
-template <bool UF, bool BORDER = true>
+template <bool BORDER = true>
 __device__ __forceinline__ void upd_core(const float q[5], const float pt[5][2], const float pb[5][2], bool inside, float fx, float fy,
                                          int w, int h, int x, int y, float dx, float dy, float m[5])
 {
@@ -48,10 +48,7 @@ __device__ __forceinline__ void upd_core(const float q[5], const float pt[5][2],
     if (inside) {
         const float a00 = (1.f - fx) * (1.f - fy), a01 = fx * (1.f - fy), a10 = (1.f - fx) * fy, a11 = fx * fy;
 #pragma unroll
-        for (int c = 0; c < 5; c++) {
-            if (UF) r[c] = fmaf(a11, pb[c][1], fmaf(a10, pb[c][0], fmaf(a01, pt[c][1], a00 * pt[c][0])));
-            else r[c] = a00 * pt[c][0] + a01 * pt[c][1] + a10 * pb[c][0] + a11 * pb[c][1];
-        }
+        for (int c = 0; c < 5; c++) r[c] = a00 * pt[c][0] + a01 * pt[c][1] + a10 * pb[c][0] + a11 * pb[c][1];
         r[2] = (q[2] + r[2]) * 0.5f;
         r[3] = (q[3] + r[3]) * 0.5f;
         r[4] = (q[4] + r[4]) * 0.25f;
@@ -62,32 +59,18 @@ __device__ __forceinline__ void upd_core(const float q[5], const float pt[5][2],
         r[4] = q[4] * 0.5f;
     }
     float r2 = (q[0] - r[0]) * 0.5f, r3 = (q[1] - r[1]) * 0.5f, r4 = r[2], r5 = r[3], r6 = r[4];
-    if (UF) {
-        r2 = fmaf(r4, dy, fmaf(r6, dx, r2));
-        r3 = fmaf(r6, dy, fmaf(r5, dx, r3));
-    } else {
-        r2 = r2 + (r4 * dy + r6 * dx);
-        r3 = r3 + (r6 * dy + r5 * dx);
-    }
+    r2 = r2 + (r4 * dy + r6 * dx);
+    r3 = r3 + (r6 * dy + r5 * dx);
     if (BORDER && ((unsigned)(x - 5) >= (unsigned)(w - 10) || (unsigned)(y - 5) >= (unsigned)(h - 10))) {
         float sc = (x < 5 ? border_tab(x) : 1.f) * (x >= w - 5 ? border_tab(w - x - 1) : 1.f) * (y < 5 ? border_tab(y) : 1.f) *
                    (y >= h - 5 ? border_tab(h - y - 1) : 1.f);
         r2 *= sc; r3 *= sc; r4 *= sc; r5 *= sc; r6 *= sc;
     }
-    if (UF) {
-        const float r66 = r6 * r6;
-        m[0] = fmaf(r4, r4, r66);
-        m[1] = (r4 + r5) * r6;
-        m[2] = fmaf(r5, r5, r66);
-        m[3] = fmaf(r4, r2, r6 * r3);
-        m[4] = fmaf(r6, r2, r5 * r3);
-    } else {
-        m[0] = r4 * r4 + r6 * r6;
-        m[1] = (r4 + r5) * r6;
-        m[2] = r5 * r5 + r6 * r6;
-        m[3] = r4 * r2 + r6 * r3;
-        m[4] = r6 * r2 + r5 * r3;
-    }
+    m[0] = r4 * r4 + r6 * r6;
+    m[1] = (r4 + r5) * r6;
+    m[2] = r5 * r5 + r6 * r6;
+    m[3] = r4 * r2 + r6 * r3;
+    m[4] = r6 * r2 + r5 * r3;
 }
 
 
@@ -154,7 +137,7 @@ __device__ __forceinline__ float2 tw_sub2(float2 a, float2 b)
 }
 
 // A.4 for TWO pixels at once (packed f32x2: .x / .y = the two pixels), both "inside" and both outside the damped 5-pixel frame
-// border: the operation sequence of upd_core<false, false> with inside = true, every half of every packed instruction one
+// border: the operation sequence of upd_core<false> with inside = true, every half of every packed instruction one
 // IEEE-754 operation, so the result is bit-identical to the scalar code.  A rounded sum whose second operand is a product is
 // issued as fma(product, one, first) with `one` the RUNTIME 1.0f (see tw_fma2): ptxas would otherwise contract the packed
 // multiply into the packed add.

@@ -1129,22 +1129,20 @@ __device__ __forceinline__ void upd_load(const float *__restrict__ R0, const flo
     }
 }
 
-template <bool UF>
 __device__ __forceinline__ void upd_compute(const UpdLoad &L, int w, int h, int x, int y, float dx, float dy, float m[5])
 {
     float pt[5][2], pb[5][2];
 #pragma unroll
     for (int c = 0; c < 5; c++) { pt[c][0] = L.p[c][0]; pt[c][1] = L.p[c][1]; pb[c][0] = L.p[c][2]; pb[c][1] = L.p[c][3]; }
-    upd_core<UF>(L.q, pt, pb, L.inside, L.fx, L.fy, w, h, x, y, dx, dy, m);
+    upd_core(L.q, pt, pb, L.inside, L.fx, L.fy, w, h, x, y, dx, dy, m);
 }
 
-template <bool UF>
 __device__ __forceinline__ void update_matrices_px(const float *__restrict__ R0, const float *__restrict__ R1,
                                                    int pitch, int w, int h, int x, int y, float dx, float dy, float m[5])
 {
     UpdLoad L;
     upd_load(R0, R1, pitch, w, h, x, y, dx, dy, L);
-    upd_compute<UF>(L, w, h, x, y, dx, dy, m);
+    upd_compute(L, w, h, x, y, dx, dy, m);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1174,7 +1172,7 @@ __device__ __forceinline__ void upsample_flow_px(const FirstUpdateArgs &a, int b
     dy = (t0 * gy + t1 * fy) * a.inv_scale;
 }
 
-template <int PITCH, bool UF>
+template <int PITCH>
 __global__ void __launch_bounds__(256, 6) first_update_kernel(FirstUpdateArgs a)
 {
     // one pixel per thread and <= 42 registers: 48 warps / SM keep enough loads in flight for this HBM-latency-bound
@@ -1199,7 +1197,7 @@ __global__ void __launch_bounds__(256, 6) first_update_kernel(FirstUpdateArgs a)
     if (a.M) {
         const float *R0 = a.R + (size_t)b * 10 * a.d.plane, *R1 = R0 + 5 * a.d.plane;
         float m[5];
-        update_matrices_px<UF>(R0, R1, a.d.pitch, a.d.w, a.d.h, x, y, dx, dy, m);
+        update_matrices_px(R0, R1, a.d.pitch, a.d.w, a.d.h, x, y, dx, dy, m);
         store_M(a.M + (size_t)b * 5 * a.d.plane, a.d.pitch, y, x, m);
     }
 }
@@ -1207,15 +1205,12 @@ __global__ void __launch_bounds__(256, 6) first_update_kernel(FirstUpdateArgs a)
 cudaError_t launch_first_update(cudaStream_t s, const FirstUpdateArgs &a)
 {
     dim3 grid((a.d.w + 31) / 32, (a.d.h + 7) / 8, a.batch);
-    if (a.ufma) return cudaErrorNotSupported; // "update_fma" was removed from the library (see launch_gauss_mr)
-    {
-        // the compile-time pitch stands for both levels: only when the coarse flow has the same row pitch ("tight_pitch" gives
-        // every level its own, e.g. 2048 over 1024)
-        const bool one_pitch = !a.coarse || a.cd.pitch == a.d.pitch;
-        if (one_pitch && a.d.pitch == 2048) first_update_kernel<2048, false><<<grid, dim3(32, 8), 0, s>>>(a);
-        else if (one_pitch && a.d.pitch == 4096) first_update_kernel<4096, false><<<grid, dim3(32, 8), 0, s>>>(a);
-        else first_update_kernel<0, false><<<grid, dim3(32, 8), 0, s>>>(a);
-    }
+    // the compile-time pitch stands for both levels: only when the coarse flow has the same row pitch ("tight_pitch" gives
+    // every level its own, e.g. 2048 over 1024)
+    const bool one_pitch = !a.coarse || a.cd.pitch == a.d.pitch;
+    if (one_pitch && a.d.pitch == 2048) first_update_kernel<2048><<<grid, dim3(32, 8), 0, s>>>(a);
+    else if (one_pitch && a.d.pitch == 4096) first_update_kernel<4096><<<grid, dim3(32, 8), 0, s>>>(a);
+    else first_update_kernel<0><<<grid, dim3(32, 8), 0, s>>>(a);
     return cudaGetLastError();
 }
 
@@ -1248,8 +1243,6 @@ __global__ void __launch_bounds__(256) gauss_iter_generic_kernel(IterArgs a, Win
             float v = Mc[gy * rs + gx] * t.k[0];
             if (a.fma == 2) {
                 for (int k = 1; k <= m; k++) { v = fmaf(Mc[max(gy - k, 0) * rs + gx], t.k[k], v); v = fmaf(Mc[min(gy + k, h - 1) * rs + gx], t.k[k], v); }
-            } else if (a.fma) {
-                for (int k = 1; k <= m; k++) v = fmaf(Mc[min(gy + k, h - 1) * rs + gx] + Mc[max(gy - k, 0) * rs + gx], t.k[k], v);
             } else {
                 for (int k = 1; k <= m; k++) v = v + (Mc[min(gy + k, h - 1) * rs + gx] + Mc[max(gy - k, 0) * rs + gx]) * t.k[k];
             }
@@ -1263,8 +1256,6 @@ __global__ void __launch_bounds__(256) gauss_iter_generic_kernel(IterArgs a, Win
             float v = p[0] * t.k[0];
             if (a.fma == 2) {
                 for (int k = 1; k <= m; k++) { v = fmaf(t.k[k], p[-k], v); v = fmaf(t.k[k], p[k], v); }
-            } else if (a.fma) {
-                for (int k = 1; k <= m; k++) v = fmaf(t.k[k], p[-k] + p[k], v);
             } else {
                 for (int k = 1; k <= m; k++) v = v + t.k[k] * (p[-k] + p[k]);
             }
@@ -1285,7 +1276,7 @@ __global__ void __launch_bounds__(256) gauss_iter_generic_kernel(IterArgs a, Win
             f[o] = fx; f[o + plane] = fy;
         } else {
             float mm[5];
-            update_matrices_px<false>(R0, R1, pitch, w, h, x, y, fx, fy, mm);
+            update_matrices_px(R0, R1, pitch, w, h, x, y, fx, fy, mm);
             store_M(a.Mout + (size_t)b * 5 * plane, pitch, y, x, mm);
         }
     }
@@ -1294,16 +1285,15 @@ __global__ void __launch_bounds__(256) gauss_iter_generic_kernel(IterArgs a, Win
 // ------------------------------------------------------------------------------------------------
 // K4/K5 (window radius MR = 15 or 7)  register-blocked Gaussian window blur + solve + update.
 //   tile 96 x 32 outputs, 256 threads, 2 CTAs / SM.
-//   phase V: thread = (column, 16-row group); 16+2*MR inputs in registers (coalesced global loads, row/column
-//            replicate = clamped addresses), 16 outputs, taps summed in the oracle's order; -> shared Vb[5][32][132]
-//   phase H: lane = row (pitch 132 = 4 mod 32 words: conflict-free LDS.128), warp = 12-column segment, 3 groups of
-//            4 pixels x 5 channels; 2x2 solve in double; flow -> shared Fb[2][32][97]
+//   phase V: vertical tap sums of the tile's 128 columns (coalesced global loads, row / column replicate = clamped
+//            addresses) -> shared
+//   phase H: lane = row, warp = 12-column segment, 3 groups of 4 pixels x 5 channels; 2x2 solve in double;
+//            flow -> shared Fb[2][32][97]
 //   phase U: lane = x (coalesced): next update-matrices (A.4) or, last iteration, the flow write.
-// FMA = validated relaxation (fmaf in the tap sums, SURVEY App. B.5: <= 2e-4 px on the default options); the
-// default build keeps the oracle's add-mul-add order bit for bit.
+// FMA = 0 keeps the oracle's add-mul-add tap order bit for bit; FMA = 2 is the validated relaxation, the direct-form fmaf
+// taps (oracle relax bit 7; SURVEY App. B.5).
 // ------------------------------------------------------------------------------------------------
-constexpr int GK_TW = 96, GK_TH = 32, GK_VW = 128, GK_VP = 132, GK_FP = 97, GK_RV = 16;
-constexpr size_t GK_SMEM = sizeof(float) * (5 * GK_TH * GK_VP + 2 * GK_TH * GK_FP);
+constexpr int GK_TW = 96, GK_TH = 32, GK_FP = 97;
 
 #ifdef TW_TIMELINE // development builds only (tools/timeline.py): per-CTA phase timestamps of the level-0 window kernel
 __device__ unsigned long long g_timeline[16384 * 24];
@@ -1334,7 +1324,6 @@ __device__ int g_dev_flags; // experiments: 1 = no R prefetch, 2 = no M prefetch
 // Per-pixel path of phase U for one thread's run of 4 vertically adjacent pixels (motion boundaries, frame borders,
 // partial tiles): two pixels' 2 x 25 loads in flight at a time.  Kept out of line so that its registers do not
 // weigh on the shared-row path.
-template <bool UF>
 __device__ __noinline__ void upd_run_slow(const float *__restrict__ R0, const float *__restrict__ R1, float *__restrict__ M,
                                           const float *__restrict__ Fb, int pitch, int w, int h, int x, int yb, int rowb, int col)
 {
@@ -1353,14 +1342,13 @@ __device__ __noinline__ void upd_run_slow(const float *__restrict__ R0, const fl
         for (int u = 0; u < 2; u++) {
             if (!ok[u]) continue;
             float mm[5];
-            upd_compute<UF>(L[u], w, h, x, yb + hf + u, fxs[u], fys[u], mm);
+            upd_compute(L[u], w, h, x, yb + hf + u, fxs[u], fys[u], mm);
             store_M(M, pitch, yb + hf + u, x, mm);
         }
     }
 }
 
 // phase U of K4/K5: lane = x, coalesced.  Last iteration: write the flow tile; otherwise the next update-matrices.
-template <bool UF>
 __device__ __forceinline__ void gauss_epilogue(const IterArgs &a, const float *__restrict__ Fb, int tid, int x0, int y0, int b, int pitch)
 {
     const int w = a.d.w, h = a.d.h;
@@ -1448,133 +1436,23 @@ __device__ __forceinline__ void gauss_epilogue(const IterArgs &a, const float *_
                 const float fxu = Fb[(rowb + u) * GK_FP + col2], fyu = Fb[(GK_TH + rowb + u) * GK_FP + col2];
                 const float px = (float)x + fxu, py = (float)(yb + u) + fyu;
                 float mm[5];
-                upd_core<UF, false>(q[u], rr[u], rr[u + 1], true, px - (float)X1, py - (float)(Y1 + u), w, h, x, yb + u, fxu, fyu, mm);
+                upd_core<false>(q[u], rr[u], rr[u + 1], true, px - (float)X1, py - (float)(Y1 + u), w, h, x, yb + u, fxu, fyu, mm);
                 store_M(M, pitch, yb + u, x, mm);
                 asm volatile("" ::: "memory"); // one pixel at a time: interleaving the four pixels' arithmetic costs more registers than there are
             }
         } else {
-            upd_run_slow<UF>(R0, R1, M, Fb, pitch, w, h, x, yb, rowb, col);
+            upd_run_slow(R0, R1, M, Fb, pitch, w, h, x, yb, rowb, col);
         }
         TW_TL(4 + k)
     }
 }
 
-template <int MR, int FMA, bool INTERIOR>
-__device__ __forceinline__ void gauss_v_phase(const float *__restrict__ Min, float *__restrict__ Vb, const WinTaps &t, int tid, int x0,
-                                              int y0, int w, int h, int pitch, size_t plane)
-{
-    const int j = tid & (GK_VW - 1), g = tid >> 7;
-    const int gx = clampi(x0 - 16 + j, 0, w - 1);
-    const int ybase = y0 + g * GK_RV - MR;
-#pragma unroll 1
-    for (int c = 0; c < 5; c++) {
-        int es;
-        const float *Mc = M_channel(Min, pitch, c, es) + (size_t)gx * es;
-        const size_t rs = (size_t)pitch * 5;
-        float in[GK_RV + 2 * MR];
-        if (INTERIOR) {
-            const float *p = Mc + (size_t)ybase * rs;
-#pragma unroll
-            for (int r = 0; r < GK_RV + 2 * MR; r++) in[r] = __ldg(p + (size_t)r * rs);
-        } else {
-#pragma unroll
-            for (int r = 0; r < GK_RV + 2 * MR; r++) in[r] = __ldg(Mc + (size_t)clampi(ybase + r, 0, h - 1) * rs);
-        }
-        float *dst = Vb + (c * GK_TH + g * GK_RV) * GK_VP + j;
-#pragma unroll
-        for (int o = 0; o < GK_RV; o++) {
-            float v = in[o + MR] * t.k[0];
-#pragma unroll
-            for (int i = 1; i <= MR; i++) {
-                if (FMA == 2) { v = fmaf(in[o + MR - i], t.k[i], v); v = fmaf(in[o + MR + i], t.k[i], v); }
-                else if (FMA) v = fmaf(in[o + MR + i] + in[o + MR - i], t.k[i], v);
-                else v = v + (in[o + MR + i] + in[o + MR - i]) * t.k[i];
-            }
-            dst[o * GK_VP] = v;
-        }
-    }
-}
-
-template <int MR, int FMA, bool UF>
-__global__ void __launch_bounds__(256, 2) gauss_iter_kernel(IterArgs a, WinTaps t)
-{
-    extern __shared__ __align__(16) float gk_smem[];
-    float *Vb = gk_smem;
-    float *Fb = gk_smem + 5 * GK_TH * GK_VP;
-    const int tid = threadIdx.x, lane = tid & 31;
-    const int x0 = blockIdx.x * GK_TW, y0 = blockIdx.y * GK_TH, b = blockIdx.z;
-    const int w = a.d.w, h = a.d.h, pitch = a.d.pitch;
-    const size_t plane = a.d.plane;
-    const float *Min = a.Min + (size_t)b * 5 * plane;
-
-    // The epilogue's R0 / R1 reads are latency-bound: pull the tile's lines into L2 while the blur runs.
-    if (!a.last) {
-        const float *Rb = a.R + (size_t)b * 10 * plane;
-        for (int i = tid; i < 10 * GK_TH * 3; i += 256) {
-            const int pl = i / (GK_TH * 3), rem = i - pl * (GK_TH * 3), row = rem / 3, seg = rem - row * 3;
-            const int y = min(y0 + row, h - 1), x = min(x0 + seg * 32, w - 1);
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(Rb + (size_t)(pl / 5) * 5 * plane + ((size_t)y * 5 + pl % 5) * pitch + x));
-        }
-    }
-
-    // ---- phase V ----
-    if ((y0 - MR >= 0) && (y0 + GK_TH + MR - 1 <= h - 1)) // block-uniform: no row clamping needed
-        gauss_v_phase<MR, FMA, true>(Min, Vb, t, tid, x0, y0, w, h, pitch, plane);
-    else
-        gauss_v_phase<MR, FMA, false>(Min, Vb, t, tid, x0, y0, w, h, pitch, plane);
-    __syncthreads();
-
-    // ---- phase H + solve ----
-    {
-        const int seg = tid >> 5; // 12-column segment
-        constexpr int LO = (16 - MR) & ~3;                // first needed index, 16B-aligned
-        constexpr int NV = ((3 + 16 + MR) | 3) + 1 - LO;  // floats loaded per channel per group (multiple of 4)
-#pragma unroll 1
-        for (int grp = 0; grp < 3; grp++) {
-            const int cbase = seg * 12 + grp * 4; // output column of pixel 0; V column = cbase + 16
-            float res[5][4];
-#pragma unroll
-            for (int c = 0; c < 5; c++) {
-                const float4 *src = reinterpret_cast<const float4 *>(Vb + (c * GK_TH + lane) * GK_VP + cbase + LO);
-                float v[NV];
-#pragma unroll
-                for (int q = 0; q < NV / 4; q++) {
-                    float4 u = src[q];
-                    v[4 * q] = u.x; v[4 * q + 1] = u.y; v[4 * q + 2] = u.z; v[4 * q + 3] = u.w;
-                }
-#pragma unroll
-                for (int p = 0; p < 4; p++) {
-                    const int ctr = p + 16 - LO;
-                    float s = v[ctr] * t.k[0];
-#pragma unroll
-                    for (int i = 1; i <= MR; i++) {
-                        if (FMA == 2) { s = fmaf(t.k[i], v[ctr - i], s); s = fmaf(t.k[i], v[ctr + i], s); }
-                        else if (FMA) s = fmaf(t.k[i], v[ctr - i] + v[ctr + i], s);
-                        else s = s + t.k[i] * (v[ctr - i] + v[ctr + i]);
-                    }
-                    res[c][p] = s;
-                }
-            }
-#pragma unroll
-            for (int p = 0; p < 4; p++) {
-                float fx, fy;
-                solve2x2(res[0][p], res[1][p], res[2][p], res[3][p], res[4][p], fx, fy);
-                Fb[lane * GK_FP + cbase + p] = fx;
-                Fb[(GK_TH + lane) * GK_FP + cbase + p] = fy;
-            }
-        }
-    }
-    __syncthreads();
-
-    gauss_epilogue<UF>(a, Fb, tid, x0, y0, b, pitch);
-}
-
 
 // ------------------------------------------------------------------------------------------------
-// K4/K5 v2: the same tile / phase structure as gauss_iter_kernel, with the tap sums issued as PACKED f32x2
-// instructions (FADD2 / FMUL2 / FFMA2, sm_100+).  Each half of a packed op is an independent IEEE-754 op, so the
-// result stays bit-identical to the oracle's scalar add-mul-add order while the FP32 instruction count halves
-// (measured, tools/ubench2.cu: the faithful tap runs 1.41x faster packed than scalar).
+// K4/K5 gauss_iter2_kernel: the tap sums are issued as PACKED f32x2 instructions (FADD2 / FMUL2 / FFMA2, sm_100+).
+// Each half of a packed op is an independent IEEE-754 op, so the result stays bit-identical to the oracle's scalar
+// add-mul-add order while the FP32 instruction count halves (measured, tools/ubench2.cu: the faithful tap runs 1.41x
+// faster packed than scalar).
 //   Packing: phase V pairs the CHANNELS (G11,G12) and (G22,h1) of one pixel column, and for h2 two adjacent
 //   columns; phase H reads them back as float2 (pitch 130 float2 = conflict-free LDS.128 with lane = row) and
 //   pairs h2 over adjacent pixels.  Shared: P01[32][130] float2, P23[32][130] float2, P4[32][132] float, flow tile.
@@ -1620,8 +1498,7 @@ __device__ __forceinline__ void gauss_v_item2(const float2 *__restrict__ src, in
 #pragma unroll
             for (int o = 0; o < G2_RV; o++) {
                 const float2 sum = tw_add2(in[o + MR + i], in[o + MR - i]);
-                if (FMA) v[o] = tw_fma2(sum, kk, v[o]);
-                else v[o] = tw_fma2(tw_mul2(sum, kk), one2, v[o]); // = v + round(sum * k): see tw_fma2 note
+                v[o] = tw_fma2(tw_mul2(sum, kk), one2, v[o]); // = v + round(sum * k): see tw_fma2 note
             }
         }
     }
@@ -1675,8 +1552,7 @@ __device__ __forceinline__ void gauss_v_walk2(const float2 *__restrict__ src, in
 #pragma unroll
                 for (int o = 0; o < G2_RV; o++) {
                     const float2 sum = tw_add2(win[o + MR + i], win[o + MR - i]);
-                    if (FMA) v[o] = tw_fma2(sum, kk, v[o]);
-                    else v[o] = tw_fma2(tw_mul2(sum, kk), one2, v[o]);
+                    v[o] = tw_fma2(tw_mul2(sum, kk), one2, v[o]);
                 }
             }
         }
@@ -1736,7 +1612,6 @@ __device__ __forceinline__ void gauss_v_phase2(const float *__restrict__ Min, fl
                     const float2 sum = tw_add2(in[o + MR + i], in[o + MR - i]);
                     const float2 kk = make_float2(t.k[i], t.k[i]);
                     if (FMA == 2) v = tw_fma2(in[o + MR + i], kk, tw_fma2(in[o + MR - i], kk, v));
-                    else if (FMA) v = tw_fma2(sum, kk, v);
                     else v = tw_fma2(tw_mul2(sum, kk), one2, v);
                 }
                 dst[o * (G2_P4 / 2)] = v;
@@ -1748,7 +1623,7 @@ __device__ __forceinline__ void gauss_v_phase2(const float *__restrict__ Min, fl
 // PITCH > 0: the row pitch is a compile-time constant (the plan pads every level to 2048 or 4096 floats), so the
 // unrolled row addresses become LDG immediates instead of 3-4 integer instructions per load.
 
-template <int MR, int FMA, bool UF, int PITCH>
+template <int MR, int FMA, int PITCH>
 __global__ void __launch_bounds__(256, 2) gauss_iter2_kernel(IterArgs a, WinTaps t)
 {
     extern __shared__ __align__(16) float gk_smem[];
@@ -1850,8 +1725,7 @@ __global__ void __launch_bounds__(256, 2) gauss_iter2_kernel(IterArgs a, WinTaps
                         for (int p = 0; p < 4; p++) {
                             const int ctr = p + 16 - LO;
                             const float2 sum = tw_add2(v[ctr - i], v[ctr + i]);
-                            if (FMA) sacc[p] = tw_fma2(kk, sum, sacc[p]);
-                            else sacc[p] = tw_fma2(tw_mul2(kk, sum), one2, sacc[p]);
+                            sacc[p] = tw_fma2(tw_mul2(kk, sum), one2, sacc[p]);
                         }
                     }
                 }
@@ -1878,8 +1752,7 @@ __global__ void __launch_bounds__(256, 2) gauss_iter2_kernel(IterArgs a, WinTaps
                             sacc = tw_fma2(kk, make_float2(v[ctr + i], v[ctr + 1 + i]), sacc);
                         } else {
                             const float2 sum = tw_add2(make_float2(v[ctr - i], v[ctr + 1 - i]), make_float2(v[ctr + i], v[ctr + 1 + i]));
-                            if (FMA) sacc = tw_fma2(kk, sum, sacc);
-                            else sacc = tw_fma2(tw_mul2(kk, sum), one2, sacc);
+                            sacc = tw_fma2(tw_mul2(kk, sum), one2, sacc);
                         }
                     }
                     r4[p] = sacc.x; r4[p + 1] = sacc.y;
@@ -1900,57 +1773,51 @@ __global__ void __launch_bounds__(256, 2) gauss_iter2_kernel(IterArgs a, WinTaps
     // on the tile's mean flow -- in the 83 KB the dead planes leave, with 16-byte coalesced loads and the corners read by
     // LDS.  The extra barrier and the exposed window load cost more than the gathers save, because phase U is paced by
     // the co-resident CTA's hold on the FMA pipe / issue slots rather than by its own loads; DESIGN.md 4.1.)
-    gauss_epilogue<UF>(a, Fb, tid, x0, y0, b, pitch);
+    gauss_epilogue(a, Fb, tid, x0, y0, b, pitch);
 #ifdef TW_TIMELINE
     __syncthreads();
 #endif
     TW_TL(7)
 }
 
-template <int MR, int FMA, bool UF, int PITCH>
+template <int MR, int FMA, int PITCH>
 static cudaError_t launch_gauss_fast2p(cudaStream_t s, const IterArgs &a, const WinTaps &t)
 {
     static std::atomic<bool> configured_dev[kMaxDevices];
     std::atomic<bool> &configured = configured_dev[current_device()];
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(gauss_iter2_kernel<MR, FMA, UF, PITCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM);
+        cudaError_t e = cudaFuncSetAttribute(gauss_iter2_kernel<MR, FMA, PITCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G2_SMEM);
         if (e != cudaSuccess) return e;
         configured = true;
     }
     dim3 grid((a.d.w + GK_TW - 1) / GK_TW, (a.d.h + GK_TH - 1) / GK_TH, a.batch);
-    gauss_iter2_kernel<MR, FMA, UF, PITCH><<<grid, 256, G2_SMEM, s>>>(a, t);
+    gauss_iter2_kernel<MR, FMA, PITCH><<<grid, 256, G2_SMEM, s>>>(a, t);
     return cudaGetLastError();
 }
 
-template <int MR, int FMA, bool UF>
+template <int MR, int FMA>
 static cudaError_t launch_gauss_fast2(cudaStream_t s, const IterArgs &a, const WinTaps &t)
 {
-    if (a.d.pitch == 2048) return launch_gauss_fast2p<MR, FMA, UF, 2048>(s, a, t);
-    if (a.d.pitch == 4096) return launch_gauss_fast2p<MR, FMA, UF, 4096>(s, a, t);
-    return launch_gauss_fast2p<MR, FMA, UF, 0>(s, a, t);
+    if (a.d.pitch == 2048) return launch_gauss_fast2p<MR, FMA, 2048>(s, a, t);
+    if (a.d.pitch == 4096) return launch_gauss_fast2p<MR, FMA, 4096>(s, a, t);
+    return launch_gauss_fast2p<MR, FMA, 0>(s, a, t);
 }
 
-// (window mode, ufma) combinations that exist: faithful (0,0), the gauss_fma opt-in (1,0), relaxed = direct form (2,0),
-// relaxed + the update_fma opt-in (2,1).
+// The two arithmetics of the library: faithful (IterArgs::fma = 0) and relaxed = direct form (2).
 template <int MR>
 static cudaError_t launch_gauss_mr(cudaStream_t s, const IterArgs &a, const WinTaps &t)
 {
 #ifdef TW_DEV_ONE // development builds: one instantiation only (fast compile while tuning the kernel)
-    if (MR == 15 && a.d.pitch == 2048 && a.fma == 2 && !a.ufma) return launch_gauss_fast2p<15, 2, false, 2048>(s, a, t);
+    if (MR == 15 && a.d.pitch == 2048 && a.fma == 2) return launch_gauss_fast2p<15, 2, 2048>(s, a, t);
     return cudaErrorNotSupported;
 #else
-    // Only the two shipped arithmetics are instantiated.  The scalar (v1) kernel and the studied, rejected relaxations ("gauss_fma" =
-    // oracle relax bit 0, "update_fma" = bit 6; DESIGN.md section 2) were removed from the library in round 2: the kernel templates
-    // still take FMA = 1 / UF = true, the oracle still restates the bits, but no binary code is carried for them.
-    if (a.scalar || a.ufma || a.fma == 1) return cudaErrorNotSupported;
-    if (a.fma == 2) return launch_gauss_fast2<MR, 2, false>(s, a, t);
-    return launch_gauss_fast2<MR, 0, false>(s, a, t);
+    if (a.fma == 2) return launch_gauss_fast2<MR, 2>(s, a, t);
+    return launch_gauss_fast2<MR, 0>(s, a, t);
 #endif
 }
 
 cudaError_t launch_gauss_iter(cudaStream_t s, const IterArgs &a, const WinTaps &t)
 {
-    if (a.ufma && a.fma != 2) return cudaErrorInvalidValue;
     if (t.m == 15) return launch_gauss_mr<15>(s, a, t);
     if (t.m == 7) return launch_gauss_mr<7>(s, a, t);
     dim3 grid((a.d.w + GI_TW - 1) / GI_TW, (a.d.h + GI_TH - 1) / GI_TH, a.batch);
@@ -2002,7 +1869,6 @@ __global__ void __launch_bounds__(SP_THREADS) gauss_last_sparse_kernel(IterArgs 
 #pragma unroll
             for (int c = 0; c < 5; c++) {
                 if (a.fma == 2) { v[c] = fmaf(up[c], k, v[c]); v[c] = fmaf(dn[c], k, v[c]); }
-                else if (a.fma == 1) v[c] = fmaf(__fadd_rn(dn[c], up[c]), k, v[c]);
                 else v[c] = __fadd_rn(v[c], __fmul_rn(__fadd_rn(dn[c], up[c]), k));
             }
         }
@@ -2020,7 +1886,6 @@ __global__ void __launch_bounds__(SP_THREADS) gauss_last_sparse_kernel(IterArgs 
         for (int i = 1; i <= m; i++) {
             const float k = t.k[i];
             if (a.fma == 2) { r = fmaf(k, p[-i], r); r = fmaf(k, p[i], r); }
-            else if (a.fma == 1) r = fmaf(k, __fadd_rn(p[-i], p[i]), r);
             else r = __fadd_rn(r, __fmul_rn(k, __fadd_rn(p[-i], p[i])));
         }
         sb[s][c] = r;
@@ -2056,7 +1921,6 @@ template <int FMA> __device__ __forceinline__ float sp3_taps(const float (&win)[
     for (int i = 1; i <= SP3_M; i++) {
         const float k = t.k[i], dn = win[c + i], up = win[c - i];
         if (FMA == 2) { v = fmaf(up, k, v); v = fmaf(dn, k, v); }
-        else if (FMA == 1) v = fmaf(__fadd_rn(dn, up), k, v);
         else v = __fadd_rn(v, __fmul_rn(__fadd_rn(dn, up), k));
     }
     return v;
@@ -2126,7 +1990,6 @@ template <int FMA> __global__ void __launch_bounds__(SP_THREADS, 2) gauss_last_s
         for (int i = 1; i <= m; i++) {
             const float k = t.k[i];
             if (FMA == 2) { r = fmaf(k, p[-i], r); r = fmaf(k, p[i], r); }
-            else if (FMA == 1) r = fmaf(k, __fadd_rn(p[-i], p[i]), r);
             else r = __fadd_rn(r, __fmul_rn(k, __fadd_rn(p[-i], p[i])));
         }
         sb[j][s][c] = r;
@@ -2167,7 +2030,6 @@ cudaError_t launch_gauss_last_sparse(cudaStream_t s, const IterArgs &a, const Wi
     if (t.m == SP3_M && a.span == SP3_SPAN && !one_row) {
         dim3 grid((a.d.w + cols - 1) / cols, (rows + SP3_R - 1) / SP3_R, a.batch);
         if (a.fma == 2) gauss_last_sparse3_kernel<2><<<grid, SP_THREADS, 0, s>>>(a, t);
-        else if (a.fma == 1) gauss_last_sparse3_kernel<1><<<grid, SP_THREADS, 0, s>>>(a, t);
         else gauss_last_sparse3_kernel<0><<<grid, SP_THREADS, 0, s>>>(a, t);
         return cudaGetLastError();
     }
@@ -2440,7 +2302,7 @@ __global__ void __launch_bounds__(BX_THREADS, 2) box_band_kernel(BoxBandArgs a)
                         if (ok[k]) {
                             const int y = y0 + ly + 8 * (jp + k);
                             float mm[5];
-                            upd_compute<false>(L[k], w, h, x, y, fx[k], fy[k], mm);
+                            upd_compute(L[k], w, h, x, y, fx[k], fy[k], mm);
                             store_M(a.Mout + (size_t)b * 5 * plane, pitch, y, x, mm);
                         }
                 }

@@ -87,7 +87,6 @@ struct FirstUpdateArgs {
     float *flow_out; // [B][2] planes (nullptr: skip; used when pyrIterations == 0)
     LevelDims d;
     int batch;
-    int ufma; // validated relaxation: fmaf chains in the update-matrices arithmetic (oracle relax bit 6)
 };
 cudaError_t launch_first_update(cudaStream_t s, const FirstUpdateArgs &a);
 
@@ -106,10 +105,8 @@ struct IterArgs {
     int span;
     double thr2;
     int *counts; // [B], zeroed by the host before the launch
-    int scalar; // 1: scalar FP32 tap sums (v1 kernel) instead of packed f32x2
-    int fma; // Gaussian tap sums: 0 = oracle order (add, mul, add); validated relaxations: 1 = fmaf(a + b, k, t) (oracle relax
-             // bit 0), 2 = direct form fmaf(a, k, t), fmaf(b, k, t) (bit 7).  Never set for the box window.
-    int ufma; // validated relaxation: fmaf chains in the update-matrices arithmetic (oracle relax bit 6)
+    int fma; // Gaussian tap sums: 0 = oracle order (add, mul, add); 2 = the validated relaxation, direct form fmaf(a, k, t),
+             // fmaf(b, k, t) (oracle relax bit 7).  Never set for the box window.
 };
 cudaError_t launch_gauss_iter(cudaStream_t s, const IterArgs &a, const WinTaps &t);
 // K4/K5 for window radius 15: the persistent, warp-specialised strip kernel (tw_window.cu).  Its operands arrive through

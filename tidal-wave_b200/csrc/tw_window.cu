@@ -671,7 +671,7 @@ gauss_strip_kernel(const __grid_constant__ CUtensorMap mapMp, const __grid_const
                                 }
                             }
                             float m[5];
-                            upd_core<false, true>(q, pt, pb, inside, fx1, fy1, w, h, x, y, dx, dy, m);
+                            upd_core<true>(q, pt, pb, inside, fx1, fy1, w, h, x, y, dx, dy, m);
                             store_M(Mo, pitch, y, x, m);
                         }
                     }
@@ -794,7 +794,7 @@ bool make_polyexp_map(const float *I, const LevelDims &d, int nimg, int polyN, T
 
 bool gauss_strip_ok(const IterArgs &a, const WinTaps &t)
 {
-    return t.m == WS_MR && !a.ufma && (a.fma == 0 || a.fma == 2) && !a.scalar && a.d.w >= 1 && a.d.h >= 1;
+    return t.m == WS_MR && a.d.w >= 1 && a.d.h >= 1;
 }
 
 cudaError_t launch_gauss_strip(cudaStream_t s, const IterArgs &a, const WinTaps &t, const StripMaps &m)
