@@ -131,8 +131,39 @@ int tw_pipe_pending(tw_ctx *ctx);
 /* 1 if the oldest pending batch has finished on the device (tw_pipe_collect would not block), else 0. */
 int tw_pipe_ready(tw_ctx *ctx);
 
+/* ---- ignore regions: leave chosen rectangles of a page out of a comparison (clocks, ads, carousels, avatars, build numbers) ----
+ * A region is a rectangle in EXPECTED-image pixels, [x, x + width) x [y, y + height); a pair has 0 .. TW_MAX_IGNORE of them.
+ * For a pair with regions:
+ *   1. before any flow work, every target pixel inside a region is replaced by the expected pixel at the same position (after the
+ *      +-5 px resize of the target); the flow is the ordinary flow of (expected, painted target), by the same kernels and arithmetic;
+ *   2. a sample point (x, y) of the span grid inside any region yields no vector and does not count toward n_vectors or the status.
+ * So the result equals the plain compare of (expected, painted target) minus the vectors inside the regions, bit for bit.
+ * Regions are clipped to the frame (one entirely outside changes nothing); width < 1, height < 1, more than TW_MAX_IGNORE regions or
+ * a NULL list with a count > 0 answer TW_BAD_PARAMETER with the reason "bad ignore region: ...".  With no regions on any pair the
+ * *_ignore entry points are exactly their plain counterparts (same kernels, same results).  The result shapes do not change. */
+#define TW_MAX_IGNORE 32
+typedef struct tw_rect {
+    int x, y, width, height; /* expected-image pixels */
+} tw_rect;
+
+/* tw_compare with ignore regions (ignore may be NULL when n_ignore == 0). */
+int tw_compare_ignore(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw, int th,
+                      const tw_flow_param *param, double threshold, int span, const tw_rect *ignore, int n_ignore,
+                      tw_vector *out, int cap, tw_result *res);
+/* tw_compare_batch with a region list per pair: pair i has n_ignore[i] regions at ignore[i].  n_ignore == NULL: no regions. */
+int tw_compare_batch_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h,
+                            int stride, const tw_flow_param *param, double threshold, int span,
+                            const tw_rect *const *ignore, const int *n_ignore, tw_vector *out, int cap, tw_result *res);
+/* tw_pipe_submit with a region list per pair (as tw_compare_batch_ignore).  The lists are copied before the call returns; they
+ * travel with the batch, so the next batch's lists do not disturb one in flight.  Collect with tw_pipe_collect. */
+int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h,
+                          int stride, const tw_flow_param *param, double threshold, int span,
+                          const tw_rect *const *ignore, const int *n_ignore);
+
 /* ---- split phases of tw_compare_batch (same stream; used by the dispatcher to overlap, and by the
- * benchmark to time the device-resident pass separately from the PCIe legs) ---- */
+ * benchmark to time the device-resident pass separately from the PCIe legs).  They take no ignore regions: painting changes the
+ * resident target, so only the whole-call entry points above apply them.  tw_batch_flow after a run with regions returns the flow of
+ * the painted pair. ---- */
 int tw_batch_upload(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w,
                     int h, int stride);                                     /* async H2D into the context */
 int tw_batch_run(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, double threshold,
@@ -222,6 +253,12 @@ long long tw_pool_submit(tw_pool *pool, const uint8_t *expect, int ew, int eh, c
  * the same request queue.  Empty path -> TW_BAD_PARAMETER, unreadable / undecodable file -> TW_BAD_IMAGE_FORMAT "Can't open <path>"
  * (src/opticalflow.cpp:20-49), sizes more than 5 px apart -> TW_DONT_MATCH_SIZE.  The pool owns the decoded images. */
 long long tw_pool_submit_files(tw_pool *pool, const char *expect_path, const char *target_path);
+/* The two submits with ignore regions (see tw_compare_ignore).  The list is copied at submit time.  A bad list answers that request
+ * alone with TW_BAD_PARAMETER "bad ignore region: ..."; requests with and without regions share batches. */
+long long tw_pool_submit_ignore(tw_pool *pool, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw, int th,
+                                const tw_rect *ignore, int n_ignore);
+long long tw_pool_submit_files_ignore(tw_pool *pool, const char *expect_path, const char *target_path,
+                                      const tw_rect *ignore, int n_ignore);
 int tw_pool_set_decoders(tw_pool *pool, int n);
 /* Blocks until request `id` is answered; copies up to cap vectors.  Returns res->code, or <0 if dropped. */
 int tw_pool_wait(tw_pool *pool, long long id, tw_vector *out, int cap, tw_result *res);

@@ -23,6 +23,7 @@ HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "tidalwave_b200.h"
 
 OK, BAD_PARAMETER, BAD_IMAGE_FORMAT, DONT_MATCH_SIZE, CUDA_ERROR, UNSUPPORTED = range(6)
 STATUS_NAMES = {0: "OK", 1: "SUSPICIOUS", 2: "ERROR"}
+MAX_IGNORE = 32  # TW_MAX_IGNORE: ignore regions per pair
 
 
 class tw_flow_param(C.Structure):
@@ -37,6 +38,38 @@ class tw_vector(C.Structure):
 class tw_result(C.Structure):
     _fields_ = [("code", C.c_int), ("status", C.c_int), ("n_vectors", C.c_int), ("width", C.c_int), ("height", C.c_int),
                 ("time", C.c_float), ("reason", C.c_char * 128)]
+
+
+class tw_rect(C.Structure):
+    """An ignore region in expected-image pixels: [x, x + width) x [y, y + height)."""
+    _fields_ = [("x", C.c_int), ("y", C.c_int), ("width", C.c_int), ("height", C.c_int)]
+
+
+def _int(v) -> int:
+    if isinstance(v, bool) or not isinstance(v, (int, np.integer)):
+        raise ValueError(f"bad ignore region: {v!r} is not an integer")
+    return int(v)
+
+
+def rect(region) -> tuple:
+    """An ignore region given as an ``(x, y, w, h)`` tuple or a ``{x, y, width, height}`` dict -> ``(x, y, w, h)`` ints.
+    Raises ValueError for anything else; sizes and counts are checked by the library (TW_BAD_PARAMETER)."""
+    if isinstance(region, dict):
+        try:
+            vals = [region[k] for k in ("x", "y", "width", "height")]
+        except KeyError as e:
+            raise ValueError(f"bad ignore region: {region!r} lacks {e.args[0]!r}") from None
+    elif isinstance(region, (tuple, list)) and len(region) == 4:
+        vals = list(region)
+    else:
+        raise ValueError(f"bad ignore region: {region!r} (an (x, y, w, h) tuple or an {{x, y, width, height}} dict)")
+    return tuple(_int(v) for v in vals)
+
+
+def _rects(regions):
+    """-> (tw_rect array or None, count) for a list of regions (None or empty: no regions)."""
+    rs = [rect(r) for r in (regions or [])]
+    return ((tw_rect * len(rs))(*[tw_rect(*r) for r in rs]) if rs else None), len(rs)
 
 
 @dataclass
@@ -80,7 +113,16 @@ def load() -> C.CDLL:
                              C.POINTER(tw_result)]
     L.tw_compare_batch.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
                                    C.c_double, C.c_int, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
+    rpp = C.POINTER(C.POINTER(tw_rect))
+    L.tw_compare_ignore.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                    C.POINTER(tw_flow_param), C.c_double, C.c_int, C.POINTER(tw_rect), C.c_int,
+                                    C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
+    L.tw_compare_batch_ignore.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
+                                          C.c_double, C.c_int, rpp, C.POINTER(C.c_int), C.POINTER(tw_vector), C.c_int,
+                                          C.POINTER(tw_result)]
     L.tw_pipe_submit.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param), C.c_double, C.c_int]
+    L.tw_pipe_submit_ignore.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
+                                        C.c_double, C.c_int, rpp, C.POINTER(C.c_int)]
     L.tw_pipe_collect.argtypes = [C.c_void_p, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
     L.tw_pipe_pending.argtypes = [C.c_void_p]
     L.tw_pipe_ready.argtypes = [C.c_void_p]
@@ -115,6 +157,11 @@ def load() -> C.CDLL:
     L.tw_pool_submit.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int]
     L.tw_pool_submit_files.restype = C.c_longlong
     L.tw_pool_submit_files.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p]
+    L.tw_pool_submit_ignore.restype = C.c_longlong
+    L.tw_pool_submit_ignore.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                        C.POINTER(tw_rect), C.c_int]
+    L.tw_pool_submit_files_ignore.restype = C.c_longlong
+    L.tw_pool_submit_files_ignore.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p, C.POINTER(tw_rect), C.c_int]
     L.tw_pool_set_decoders.argtypes = [C.c_void_p, C.c_int]
     L.tw_pool_peek.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_result)]
     L.tw_pool_wait.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
@@ -219,8 +266,10 @@ class OpticalFlow:
         return rc, fx, fy, sec.value
 
     def calculate(self, expectImg, targetImg, param: OpticalFlowParameter = OpticalFlowParameter(), threshold: float = 5.0,
-                  span: int = 10, cap: int | None = None, expect_image: str = "", target_image: str = "") -> dict:
-        """calculate + Consumer::run's sampling -> response dict (src/opticalflow.cpp:20-76, src/consumer.cpp:59-88)."""
+                  span: int = 10, cap: int | None = None, expect_image: str = "", target_image: str = "", ignore=None) -> dict:
+        """calculate + Consumer::run's sampling -> response dict (src/opticalflow.cpp:20-76, src/consumer.cpp:59-88).
+        ignore: regions of the expected image left out of the comparison (``(x, y, w, h)`` tuples or ``{x, y, width, height}``
+        dicts, at most MAX_IGNORE; include/tidalwave_b200.h, tw_compare_ignore)."""
         a = None if expectImg is None else _u8(expectImg)
         b = None if targetImg is None else _u8(targetImg)
         eh, ew = a.shape if a is not None else (0, 0)
@@ -230,13 +279,20 @@ class OpticalFlow:
         vec = (tw_vector * cap)()
         res = tw_result()
         p = param.c()
-        self.lib.tw_compare(self.ctx, a.ctypes.data if a is not None else None, ew, eh,
-                            b.ctypes.data if b is not None else None, tw, th, C.byref(p), threshold, span, vec, cap,
-                            C.byref(res))
+        if ignore is None:
+            self.lib.tw_compare(self.ctx, a.ctypes.data if a is not None else None, ew, eh,
+                                b.ctypes.data if b is not None else None, tw, th, C.byref(p), threshold, span, vec, cap,
+                                C.byref(res))
+        else:
+            rs, nr = _rects(ignore)
+            self.lib.tw_compare_ignore(self.ctx, a.ctypes.data if a is not None else None, ew, eh,
+                                       b.ctypes.data if b is not None else None, tw, th, C.byref(p), threshold, span, rs, nr,
+                                       vec, cap, C.byref(res))
         return _response(res, vec, min(res.n_vectors, cap), span, threshold, expect_image, target_image)
 
     def calculate_batch(self, pairs, param: OpticalFlowParameter = OpticalFlowParameter(), threshold: float = 5.0,
-                        span: int = 10, cap: int | None = None) -> list[dict]:
+                        span: int = 10, cap: int | None = None, ignore=None) -> list[dict]:
+        """ignore: one region list (or None) per pair, as in calculate()."""
         n = len(pairs)
         imgs = [(_u8(a), _u8(b)) for a, b in pairs]
         h, w = imgs[0][0].shape
@@ -247,7 +303,15 @@ class OpticalFlow:
         vec = (tw_vector * (cap * n))()
         res = (tw_result * n)()
         p = param.c()
-        self.lib.tw_compare_batch(self.ctx, n, ex, tg, w, h, w, C.byref(p), threshold, span, vec, cap, res)
+        if ignore is None:
+            self.lib.tw_compare_batch(self.ctx, n, ex, tg, w, h, w, C.byref(p), threshold, span, vec, cap, res)
+        else:
+            if len(ignore) != n:
+                raise ValueError("ignore: one region list per pair")
+            lists = [_rects(g) for g in ignore]
+            ig = (C.POINTER(tw_rect) * n)(*[C.cast(rs, C.POINTER(tw_rect)) if rs is not None else None for rs, _ in lists])
+            nig = (C.c_int * n)(*[k for _, k in lists])
+            self.lib.tw_compare_batch_ignore(self.ctx, n, ex, tg, w, h, w, C.byref(p), threshold, span, ig, nig, vec, cap, res)
         out = []
         for i in range(n):
             sub = (tw_vector * cap).from_buffer(vec, i * cap * C.sizeof(tw_vector))
@@ -303,21 +367,29 @@ class Pool:
             raise RuntimeError("tw_pool_create failed: " + err.value.decode())
         self._keep = {}
 
-    def request(self, expectImg, targetImg) -> int:
-        """Manager::request (src/manager.cpp:68-78)."""
+    def request(self, expectImg, targetImg, ignore=None) -> int:
+        """Manager::request (src/manager.cpp:68-78).  ignore: regions left out of the comparison, as in OpticalFlow.calculate."""
         a = None if expectImg is None else _u8(expectImg)
         b = None if targetImg is None else _u8(targetImg)
         eh, ew = a.shape if a is not None else (0, 0)
         th, tw = b.shape if b is not None else (0, 0)
-        rid = self.lib.tw_pool_submit(self.pool, a.ctypes.data if a is not None else None, ew, eh,
-                                      b.ctypes.data if b is not None else None, tw, th)
+        if ignore is None:
+            rid = self.lib.tw_pool_submit(self.pool, a.ctypes.data if a is not None else None, ew, eh,
+                                          b.ctypes.data if b is not None else None, tw, th)
+        else:
+            rs, nr = _rects(ignore)
+            rid = self.lib.tw_pool_submit_ignore(self.pool, a.ctypes.data if a is not None else None, ew, eh,
+                                                 b.ctypes.data if b is not None else None, tw, th, rs, nr)
         if rid >= 0:
             self._keep[rid] = (a, b)
         return rid
 
-    def request_files(self, expect_path: str, target_path: str) -> int:
+    def request_files(self, expect_path: str, target_path: str, ignore=None) -> int:
         """Manager::request with two image paths (src/manager.cpp:68-78): read + decoded on the pool's C++ decoder threads."""
-        return self.lib.tw_pool_submit_files(self.pool, (expect_path or "").encode(), (target_path or "").encode())
+        if ignore is None:
+            return self.lib.tw_pool_submit_files(self.pool, (expect_path or "").encode(), (target_path or "").encode())
+        rs, nr = _rects(ignore)
+        return self.lib.tw_pool_submit_files_ignore(self.pool, (expect_path or "").encode(), (target_path or "").encode(), rs, nr)
 
     def wait(self, rid: int) -> dict | None:
         cap = self.cap

@@ -19,9 +19,9 @@ using namespace tw;
 
 namespace {
 
-enum Family { F_LEVEL = 0, F_POLY, F_FIRST, F_GITER, F_GLAST, F_BVSUM, F_BITER, F_BLAST, F_BUPD, F_SAMPLE, F_COUNT };
+enum Family { F_LEVEL = 0, F_POLY, F_FIRST, F_GITER, F_GLAST, F_BVSUM, F_BITER, F_BLAST, F_BUPD, F_SAMPLE, F_PAINT, F_COUNT };
 const char *kFamilyNames[F_COUNT] = {"level_image", "polyexp", "first_update", "gauss_iter", "gauss_last",
-                                     "box_vsum", "box_hscan", "box_hscan_last", "box_update", "sample"};
+                                     "box_vsum", "box_hscan", "box_hscan_last", "box_update", "sample", "ignore_paint"};
 
 struct Scale {
     int k, ksize;
@@ -55,12 +55,15 @@ struct LaunchOptions {
     }
 };
 
-// A plan's CUDA graph of the launch sequence (enqueue) is captured for one (n, threshold, span, options, result buffer) key
+// A plan's CUDA graph of the launch sequence (enqueue) is captured for one (n, threshold, span, options, result buffer, ignore) key.
+// `ignore`: the batch has ignore regions (paint launch first, the ignore form of the sample kernel).  The graph reads the regions
+// from the context's region buffer at fixed addresses, so new lists replay the same graph.
 struct GraphKey {
-    int n = 0; double thr = 0; int span = 0; LaunchOptions opt; const void *vectors = nullptr; int dev_cap = 0;
+    int n = 0; double thr = 0; int span = 0; LaunchOptions opt; const void *vectors = nullptr; int dev_cap = 0; bool ignore = false;
     bool operator==(const GraphKey &o) const
     {
-        return n == o.n && thr == o.thr && span == o.span && opt == o.opt && vectors == o.vectors && dev_cap == o.dev_cap;
+        return n == o.n && thr == o.thr && span == o.span && opt == o.opt && vectors == o.vectors && dev_cap == o.dev_cap &&
+               ignore == o.ignore;
     }
 };
 
@@ -108,6 +111,9 @@ struct tw_ctx {
     // results
     int *d_counts = nullptr;
     int *h_counts = nullptr; // pinned
+    // ignore regions of the batch being run: [max_batch][kMaxIgnore] int4 clipped bounds, then [max_batch] counts (ignore_bytes);
+    // h_ignore is the page-locked mirror the synchronous entry points copy from
+    void *d_ignore = nullptr, *h_ignore = nullptr;
     void *d_vectors = nullptr;
     int dev_cap = 0;
     int last_n = 0, last_w = 0, last_h = 0;
@@ -127,6 +133,7 @@ struct tw_ctx {
         cudaEvent_t done = nullptr, r0 = nullptr, r1 = nullptr;
         int *d_counts = nullptr, *h_counts = nullptr;
         void *d_vec = nullptr;
+        void *h_ignore = nullptr; // page-locked: this batch's region lists, copied into the staging buffer behind its images
         size_t vec_bytes = 0;
         int n = 0, w = 0, h = 0, dev_cap = 0;
     };
@@ -581,6 +588,46 @@ bool ensure_results(tw_ctx *ctx, int cap)
     return true;
 }
 
+// Region buffer (tw_ctx::d_ignore, h_ignore, the pipe's staging tail): [max_batch][kMaxIgnore] int4, then [max_batch] int.
+size_t ignore_bytes(int max_batch) { return (size_t)max_batch * (kMaxIgnore * sizeof(int4) + sizeof(int)); }
+
+IgnoreRegions ignore_regions(const void *base, int max_batch)
+{
+    IgnoreRegions g;
+    g.rects = reinterpret_cast<const int4 *>(base);
+    g.n = reinterpret_cast<const int *>(g.rects + (size_t)max_batch * kMaxIgnore);
+    return g;
+}
+
+// Checks the region lists of n pairs (n_ignore == NULL: none) and writes them, clipped to the W x H frame, into `mirror` (layout of
+// ignore_bytes).  Returns 1 if some pair keeps a region, 0 if none does, -1 for a bad list (ctx->err says why).
+int pack_ignore(tw_ctx *ctx, int n, const tw_rect *const *ignore, const int *n_ignore, int W, int H, void *mirror)
+{
+    if (!n_ignore) return 0;
+    for (int i = 0; i < n; i++) {
+        const int k = n_ignore[i];
+        if (k < 0 || k > kMaxIgnore) { ctx->err = "bad ignore region: 0 to " + std::to_string(kMaxIgnore) + " regions per pair"; return -1; }
+        if (k > 0 && (!ignore || !ignore[i])) { ctx->err = "bad ignore region: NULL list with a count > 0"; return -1; }
+        for (int j = 0; j < k; j++)
+            if (ignore[i][j].width < 1 || ignore[i][j].height < 1) { ctx->err = "bad ignore region: width and height must be >= 1"; return -1; }
+    }
+    int4 *rects = reinterpret_cast<int4 *>(mirror);
+    int *cnt = reinterpret_cast<int *>(rects + (size_t)ctx->max_batch * kMaxIgnore);
+    int any = 0;
+    for (int i = 0; i < n; i++) {
+        int kept = 0;
+        for (int j = 0; j < n_ignore[i]; j++) {
+            const tw_rect &r = ignore[i][j];
+            const long long x0 = std::max<long long>(r.x, 0), y0 = std::max<long long>(r.y, 0);
+            const long long x1 = std::min<long long>((long long)r.x + r.width, W), y1 = std::min<long long>((long long)r.y + r.height, H);
+            if (x0 < x1 && y0 < y1) rects[(size_t)i * kMaxIgnore + kept++] = make_int4((int)x0, (int)y0, (int)x1, (int)y1);
+        }
+        cnt[i] = kept;
+        any |= kept > 0;
+    }
+    return any;
+}
+
 // Relaxed arithmetic (fmaf in the Gaussian window taps, mixed double / float horizontal pass of the polynomial
 // expansion) is used only for the option family it was validated on against the faithful oracle and cv2
 // (tools/relax_study.py, tests/test_gpu_parity.py): Gaussian window of the reference's default size or larger and
@@ -602,8 +649,9 @@ bool sparse_in_effect(const tw_ctx *ctx, int span)
     return gauss_last_sparse_ok(ia, pl.win);
 }
 
-// The launch sequence for n pairs already resident in plan.src.  SURVEY App. A.1 / A.7.
-bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
+// The launch sequence for n pairs already resident in plan.src.  SURVEY App. A.1 / A.7.  ignore: the batch has ignore regions
+// (in ctx->d_ignore): the target is painted first and the sample kernel leaves the points inside the regions out.
+bool enqueue(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
 {
     Plan &pl = ctx->plan;
     const tw_flow_param &p = pl.p;
@@ -613,6 +661,8 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
     const size_t ns = pl.scales.size();
     // sampling is fused into the last Gaussian iteration of the finest scale when that kernel runs (radius 15 / 7)
     const bool fused_count = span > 0 && (p.flags & 256) && p.pyrIterations > 0 && (pl.win.m == 15 || pl.win.m == 7);
+    if (ignore) // expected pixels over the target inside the regions, before anything reads the target
+        LAUNCH(F_PAINT, 0.0, launch_ignore_paint(ctx->stream, pl.src, H, pl.spitch, ignore_regions(ctx->d_ignore, ctx->max_batch), n));
     if (fused_count) {
         cudaError_t e = cudaMemsetAsync(ctx->d_counts, 0, sizeof(int) * n, ctx->stream);
         if (e != cudaSuccess) { set_err(ctx, "memset counts", e); return false; }
@@ -702,7 +752,8 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
         SampleArgs sa{};
         sa.flow = f.flow; sa.d = f.d; sa.batch = n; sa.span = span; sa.thr2 = threshold * threshold;
         sa.counts = ctx->d_counts; sa.vectors = ctx->d_vectors; sa.cap = ctx->dev_cap; sa.counted = fused_count ? 1 : 0;
-        LAUNCH(F_SAMPLE, 0.0, launch_sample(ctx->stream, sa));
+        if (ignore) LAUNCH(F_SAMPLE, 0.0, launch_sample_ignore(ctx->stream, sa, ignore_regions(ctx->d_ignore, ctx->max_batch)));
+        else LAUNCH(F_SAMPLE, 0.0, launch_sample(ctx->stream, sa));
     }
     return true;
 }
@@ -711,12 +762,12 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span)
 // cudaGraphLaunch of the captured sequence (the step is ~22 short launches; at the coarse scales the kernels are
 // shorter than their launch gaps).  The first run of a key is always eager: it configures the per-device kernel
 // attributes and sizes the result buffers outside any capture.  Profiling (per-family events) runs eagerly.
-bool run_sequence(tw_ctx *ctx, int n, double threshold, int span)
+bool run_sequence(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
 {
-    if (!ctx->opt_graph || ctx->profiling) return enqueue(ctx, n, threshold, span);
+    if (!ctx->opt_graph || ctx->profiling) return enqueue(ctx, n, threshold, span, ignore);
     Plan &pl = ctx->plan;
     GraphKey key;
-    key.n = n; key.thr = threshold; key.span = span; key.opt = ctx->opt;
+    key.n = n; key.thr = threshold; key.span = span; key.opt = ctx->opt; key.ignore = ignore;
     key.vectors = ctx->d_vectors; key.dev_cap = ctx->dev_cap; // the captured sample kernel bakes both in
     if (pl.graph_exec && key == pl.graph_key) {
         cudaError_t e = cudaGraphLaunch(pl.graph_exec, ctx->stream);
@@ -725,7 +776,7 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span)
         return true;
     }
     if (!(key == pl.seen_key)) { // first run of this key: eager
-        if (!enqueue(ctx, n, threshold, span)) return false;
+        if (!enqueue(ctx, n, threshold, span, ignore)) return false;
         pl.seen_key = key;
         pl.seen_key.vectors = ctx->d_vectors; pl.seen_key.dev_cap = ctx->dev_cap; // enqueue may have (re)allocated the result buffer
         return true;
@@ -738,9 +789,9 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span)
     if (e != cudaSuccess) { // capture unavailable: stay eager
         cudaGetLastError();
         ctx->opt_graph = 0;
-        return enqueue(ctx, n, threshold, span);
+        return enqueue(ctx, n, threshold, span, ignore);
     }
-    const bool ok = enqueue(ctx, n, threshold, span);
+    const bool ok = enqueue(ctx, n, threshold, span, ignore);
     e = cudaStreamEndCapture(ctx->stream, &graph);
     const long long captured = ctx->launches - before;
     ctx->launches = before;
@@ -749,7 +800,7 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span)
         cudaGetLastError();
         ctx->opt_graph = 0; // never retry on this context; the eager path is the same launch sequence
         if (!ok) return false;
-        return enqueue(ctx, n, threshold, span);
+        return enqueue(ctx, n, threshold, span, ignore);
     }
     e = cudaGraphInstantiate(&pl.graph_exec, graph, 0);
     cudaGraphDestroy(graph);
@@ -757,7 +808,7 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span)
         cudaGetLastError();
         pl.graph_exec = nullptr;
         ctx->opt_graph = 0;
-        return enqueue(ctx, n, threshold, span);
+        return enqueue(ctx, n, threshold, span, ignore);
     }
     pl.graph_key = key;
     pl.graph_launches = captured;
@@ -834,7 +885,9 @@ tw_ctx *tw_create(int device, int max_w, int max_h, int max_batch, char *err, in
     if ((e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess) { delete ctx; return fail(cudaGetErrorString(e)); }
     cudaEventCreate(&ctx->ev_t0); cudaEventCreate(&ctx->ev_t1); cudaEventCreate(&ctx->ev_r0); cudaEventCreate(&ctx->ev_r1);
     if ((e = cudaMalloc(&ctx->d_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
-        (e = cudaMallocHost(&ctx->h_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess) {
+        (e = cudaMallocHost(&ctx->h_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
+        (e = cudaMalloc(&ctx->d_ignore, ignore_bytes(ctx->max_batch))) != cudaSuccess ||
+        (e = cudaMallocHost(&ctx->h_ignore, ignore_bytes(ctx->max_batch))) != cudaSuccess) {
         std::string m = cudaGetErrorString(e);
         tw_destroy(ctx);
         return fail(m);
@@ -853,6 +906,8 @@ void tw_destroy(tw_ctx *ctx)
     for (auto e : ctx->ev_pool) cudaEventDestroy(e);
     if (ctx->d_counts) cudaFree(ctx->d_counts);
     if (ctx->h_counts) cudaFreeHost(ctx->h_counts);
+    if (ctx->d_ignore) cudaFree(ctx->d_ignore);
+    if (ctx->h_ignore) cudaFreeHost(ctx->h_ignore);
     if (ctx->d_vectors) cudaFree(ctx->d_vectors);
     if (ctx->flush_buf) cudaFree(ctx->flush_buf);
     if (ctx->rs_buf) cudaFree(ctx->rs_buf);
@@ -869,6 +924,7 @@ void tw_destroy(tw_ctx *ctx)
             if (s.r1) cudaEventDestroy(s.r1);
             if (s.d_counts) cudaFree(s.d_counts);
             if (s.h_counts) cudaFreeHost(s.h_counts);
+            if (s.h_ignore) cudaFreeHost(s.h_ignore);
             if (s.d_vec) cudaFree(s.d_vec);
         }
     }
@@ -960,12 +1016,27 @@ static bool upload_resized_target(tw_ctx *ctx, const uint8_t *target, int tw_, i
     return true;
 }
 
+// Checks and clips the region lists of n pairs of w x h frames and copies them into the region buffer on the context's stream (the
+// synchronous entry points: the page-locked mirror is free again once the call has fetched its results).  *any: some pair keeps a
+// region.  Returns a tw_error_code.
+static int upload_ignore(tw_ctx *ctx, int n, const tw_rect *const *ignore, const int *n_ignore, int w, int h, bool *any)
+{
+    const int r = pack_ignore(ctx, n, ignore, n_ignore, w, h, ctx->h_ignore);
+    if (r < 0) return TW_BAD_PARAMETER;
+    *any = r > 0;
+    if (!*any) return TW_OK;
+    cudaError_t e = cudaMemcpyAsync(ctx->d_ignore, ctx->h_ignore, ignore_bytes(ctx->max_batch), cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess) { set_err(ctx, "regions H2D", e); return TW_CUDA_ERROR; }
+    return TW_OK;
+}
+
 int tw_batch_upload(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride)
 {
     return upload_impl(ctx, n, expect, target, w, h, stride, nullptr);
 }
 
-int tw_batch_run(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, double threshold, int span)
+// tw_batch_run; ignore: run the ignore form with the regions already in the region buffer
+static int run_batch(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, double threshold, int span, bool ignore)
 {
     if (!ctx) return TW_BAD_PARAMETER;
     if (n < 1 || n > ctx->max_batch) { ctx->err = "bad batch"; return TW_BAD_PARAMETER; }
@@ -991,11 +1062,16 @@ int tw_batch_run(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, d
         if (!ok) return TW_CUDA_ERROR;
     }
     cudaEventRecord(ctx->ev_r0, ctx->stream);
-    if (!run_sequence(ctx, n, threshold, span)) return TW_CUDA_ERROR;
+    if (!run_sequence(ctx, n, threshold, span, ignore)) return TW_CUDA_ERROR;
     cudaEventRecord(ctx->ev_r1, ctx->stream);
     ctx->last_n = n; ctx->last_w = w; ctx->last_h = h; ctx->ran = true;
     ctx->last_sparse = sparse_in_effect(ctx, span);
     return TW_OK;
+}
+
+int tw_batch_run(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, double threshold, int span)
+{
+    return run_batch(ctx, n, w, h, param, threshold, span, false);
 }
 
 int tw_batch_fetch(tw_ctx *ctx, int n, tw_vector *out, int cap, tw_result *res)
@@ -1069,8 +1145,9 @@ int tw_flow(tw_ctx *ctx, const uint8_t *expect, const uint8_t *target, int w, in
     return TW_OK;
 }
 
-int tw_compare_batch(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
-                     const tw_flow_param *param, double threshold, int span, tw_vector *out, int cap, tw_result *res)
+int tw_compare_batch_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
+                            const tw_flow_param *param, double threshold, int span, const tw_rect *const *ignore, const int *n_ignore,
+                            tw_vector *out, int cap, tw_result *res)
 {
     if (!ctx || !res) return TW_BAD_PARAMETER;
     auto fail_all = [&](int code, const char *msg) {
@@ -1081,9 +1158,18 @@ int tw_compare_batch(tw_ctx *ctx, int n, const uint8_t *const *expect, const uin
     if (validate_param(param) != TW_OK) return fail_all(TW_BAD_PARAMETER, "bad optical-flow parameter");
     int rc = upload_impl(ctx, n, expect, target, w, h, stride, param);
     if (rc != TW_OK) return fail_all(rc, ctx->err.c_str());
-    rc = tw_batch_run(ctx, n, w, h, param, threshold, span);
+    bool any = false;
+    rc = upload_ignore(ctx, n, ignore, n_ignore, w, h, &any);
+    if (rc != TW_OK) return fail_all(rc, ctx->err.c_str());
+    rc = run_batch(ctx, n, w, h, param, threshold, span, any);
     if (rc != TW_OK) return fail_all(rc, ctx->err.c_str());
     return tw_batch_fetch(ctx, n, out, cap, res);
+}
+
+int tw_compare_batch(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
+                     const tw_flow_param *param, double threshold, int span, tw_vector *out, int cap, tw_result *res)
+{
+    return tw_compare_batch_ignore(ctx, n, expect, target, w, h, stride, param, threshold, span, nullptr, nullptr, out, cap, res);
 }
 
 // ---- pipelined form of tw_compare_batch: at most two batches in flight per context ----
@@ -1102,8 +1188,8 @@ int tw_pipe_ready(tw_ctx *ctx)
     return cudaEventQuery(ctx->pipe.slot[ctx->pipe.head].done) == cudaSuccess ? 1 : 0;
 }
 
-int tw_pipe_submit(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
-                   const tw_flow_param *param, double threshold, int span)
+int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
+                          const tw_flow_param *param, double threshold, int span, const tw_rect *const *ignore, const int *n_ignore)
 {
     if (!ctx) return TW_BAD_PARAMETER;
     tw_ctx::Pipe &pp = ctx->pipe;
@@ -1127,10 +1213,17 @@ int tw_pipe_submit(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8
         for (auto &s : pp.slot) {
             if ((e = cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming)) != cudaSuccess || (e = cudaEventCreate(&s.r0)) != cudaSuccess ||
                 (e = cudaEventCreate(&s.r1)) != cudaSuccess || (e = cudaMalloc(&s.d_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
-                (e = cudaMallocHost(&s.h_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess) { set_err(ctx, "pipe setup", e); return TW_CUDA_ERROR; }
+                (e = cudaMallocHost(&s.h_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
+                (e = cudaMallocHost(&s.h_ignore, ignore_bytes(ctx->max_batch))) != cudaSuccess) { set_err(ctx, "pipe setup", e); return TW_CUDA_ERROR; }
         }
     }
-    const size_t pair_bytes = (size_t)2 * h * pl.spitch, need = (size_t)ctx->max_batch * pair_bytes;
+    // this batch's slot: free (at most one other batch in flight), its page-locked region mirror with it
+    tw_ctx::PipeSlot &s = pp.slot[(pp.head + pp.count) & 1];
+    const int packed = pack_ignore(ctx, n, ignore, n_ignore, w, h, s.h_ignore);
+    if (packed < 0) return TW_BAD_PARAMETER;
+    const bool any = packed > 0;
+    // staging buffer: the images of max_batch pairs, then the region lists (ignore_bytes)
+    const size_t pair_bytes = (size_t)2 * h * pl.spitch, images = (size_t)ctx->max_batch * pair_bytes, need = images + ignore_bytes(ctx->max_batch);
     if (pp.stage_bytes < need) { // only with nothing in flight (same_plan is false for a new size)
         cudaStreamSynchronize(pp.copy);
         cudaStreamSynchronize(ctx->stream);
@@ -1147,16 +1240,20 @@ int tw_pipe_submit(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8
         if (e == cudaSuccess) e = cudaMemcpy2DAsync(d + (size_t)h * pl.spitch, pl.spitch, target[i], stride, w, h, cudaMemcpyHostToDevice, pp.copy);
         if (e != cudaSuccess) { set_err(ctx, "H2D", e); return TW_CUDA_ERROR; }
     }
+    if (any && (e = cudaMemcpyAsync(pp.stage + images, s.h_ignore, ignore_bytes(ctx->max_batch), cudaMemcpyHostToDevice, pp.copy)) != cudaSuccess) {
+        set_err(ctx, "regions H2D", e);
+        return TW_CUDA_ERROR;
+    }
     cudaEventRecord(pp.ev_up, pp.copy);
-    // compute stream
-    tw_ctx::PipeSlot &s = pp.slot[(pp.head + pp.count) & 1];
+    // compute stream: the take-over copies run behind the previous batch's kernels, so its region lists stay put while they read them
     cudaStreamWaitEvent(ctx->stream, pp.ev_up, 0);
     e = cudaMemcpyAsync(pl.src, pp.stage, (size_t)n * pair_bytes, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess && any) e = cudaMemcpyAsync(ctx->d_ignore, pp.stage + images, ignore_bytes(ctx->max_batch), cudaMemcpyDeviceToDevice, ctx->stream);
     if (e != cudaSuccess) { set_err(ctx, "stage -> src", e); return TW_CUDA_ERROR; }
     cudaEventRecord(pp.ev_stage_free, ctx->stream);
     pp.stage_used = true;
     cudaEventRecord(s.r0, ctx->stream);
-    if (!run_sequence(ctx, n, threshold, span)) return TW_CUDA_ERROR;
+    if (!run_sequence(ctx, n, threshold, span, any)) return TW_CUDA_ERROR;
     cudaEventRecord(s.r1, ctx->stream);
     ctx->last_n = n; ctx->last_w = w; ctx->last_h = h; ctx->ran = true;
     ctx->last_sparse = sparse_in_effect(ctx, span);
@@ -1176,6 +1273,12 @@ int tw_pipe_submit(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8
     s.n = n; s.w = w; s.h = h; s.dev_cap = ctx->dev_cap;
     pp.count++;
     return TW_OK;
+}
+
+int tw_pipe_submit(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
+                   const tw_flow_param *param, double threshold, int span)
+{
+    return tw_pipe_submit_ignore(ctx, n, expect, target, w, h, stride, param, threshold, span, nullptr, nullptr);
 }
 
 int tw_pipe_collect(tw_ctx *ctx, tw_vector *out, int cap, tw_result *res)
@@ -1216,8 +1319,9 @@ int tw_pipe_collect(tw_ctx *ctx, tw_vector *out, int cap, tw_result *res)
     return TW_OK;
 }
 
-int tw_compare(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
-               const tw_flow_param *param, double threshold, int span, tw_vector *out, int cap, tw_result *res)
+int tw_compare_ignore(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
+                      const tw_flow_param *param, double threshold, int span, const tw_rect *ignore, int n_ignore,
+                      tw_vector *out, int cap, tw_result *res)
 {
     if (!res) return TW_BAD_PARAMETER;
     if (!ctx) { fill_error(res, TW_BAD_PARAMETER, "null context"); return res->code; }
@@ -1232,13 +1336,21 @@ int tw_compare(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t
         if (validate_param(param) != TW_OK) { fill_error(res, TW_BAD_PARAMETER, "bad optical-flow parameter"); return res->code; }
         int rc = upload_impl(ctx, 1, &expect, &expect, ew, eh, ew, param); // builds the plan, fills the expected slot
         if (rc == TW_OK && !upload_resized_target(ctx, target, tw_, th_, ew, eh)) rc = TW_CUDA_ERROR;
-        if (rc == TW_OK) rc = tw_batch_run(ctx, 1, ew, eh, param, threshold, span);
+        bool any = false; // regions are painted over the resized target (the paint kernel runs first in the launch sequence)
+        if (rc == TW_OK) rc = upload_ignore(ctx, 1, &ignore, &n_ignore, ew, eh, &any);
+        if (rc == TW_OK) rc = run_batch(ctx, 1, ew, eh, param, threshold, span, any);
         if (rc != TW_OK) { fill_error(res, rc, ctx->err.c_str()); return res->code; }
         tw_batch_fetch(ctx, 1, out, cap, res);
         return res->code;
     }
-    tw_compare_batch(ctx, 1, &expect, &target, ew, eh, ew, param, threshold, span, out, cap, res);
+    tw_compare_batch_ignore(ctx, 1, &expect, &target, ew, eh, ew, param, threshold, span, &ignore, &n_ignore, out, cap, res);
     return res->code;
+}
+
+int tw_compare(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
+               const tw_flow_param *param, double threshold, int span, tw_vector *out, int cap, tw_result *res)
+{
+    return tw_compare_ignore(ctx, expect, ew, eh, target, tw_, th_, param, threshold, span, nullptr, 0, out, cap, res);
 }
 
 int tw_l2_flush(tw_ctx *ctx)

@@ -2376,15 +2376,34 @@ cudaError_t launch_resize_u8(cudaStream_t s, const ResizeU8Args &a)
 //   len = f32(f32(dx*dx) + f32(dy*dy));  keep iff double(len) > threshold*threshold (strict), row-major order.
 // One block per pair; each thread owns a contiguous run of sample points so a block-wide exclusive scan of
 // the per-thread counts yields row-major output positions.  Counts are reduced with warp shuffles.
+// `skip(x, y)`: sample points the caller leaves out (ignore regions); the same test in both passes.
 // ------------------------------------------------------------------------------------------------
 struct DevVector { int x, y; double dx, dy; };
 
-__global__ void __launch_bounds__(1024) sample_kernel(SampleArgs a)
+struct SkipNone {
+    __device__ __forceinline__ bool operator()(int, int) const { return false; }
+};
+
+// The regions of one pair, staged in shared memory by sample_ignore_kernel.
+struct SkipRegions {
+    const int4 *r;
+    int n;
+    __device__ __forceinline__ bool operator()(int x, int y) const
+    {
+        bool in = false;
+        for (int k = 0; k < n; k++) {
+            const int4 q = r[k];
+            in |= (x >= q.x) & (x < q.z) & (y >= q.y) & (y < q.w);
+        }
+        return in;
+    }
+};
+
+template <class Skip>
+__device__ __forceinline__ void sample_body(const SampleArgs &a, const int b, const Skip &skip)
 {
     __shared__ int warp_sums[32];
     __shared__ int total;
-    const int b = blockIdx.x;
-    if (a.counted && a.counts[b] == 0) return; // OK pair: nothing to compact (block-uniform)
     const float *fxp = a.flow + (size_t)b * 2 * a.d.plane, *fyp = fxp + a.d.plane;
     const int nsx = (a.d.w + a.span - 1) / a.span, nsy = (a.d.h + a.span - 1) / a.span, ns = nsx * nsy;
     const int per = (ns + blockDim.x - 1) / blockDim.x;
@@ -2392,6 +2411,7 @@ __global__ void __launch_bounds__(1024) sample_kernel(SampleArgs a)
     int cnt = 0;
     for (int i = i0; i < i1; i++) {
         int sy = i / nsx, sx = i - sy * nsx;
+        if (skip(sx * a.span, sy * a.span)) continue;
         size_t o = (size_t)(sy * a.span) * a.d.pitch + sx * a.span;
         float dx = fxp[o], dy = fyp[o];
         float len = (dx * dx) + (dy * dy);
@@ -2425,6 +2445,7 @@ __global__ void __launch_bounds__(1024) sample_kernel(SampleArgs a)
     DevVector *out = reinterpret_cast<DevVector *>(a.vectors) + (size_t)b * a.cap;
     for (int i = i0; i < i1; i++) {
         int sy = i / nsx, sx = i - sy * nsx;
+        if (skip(sx * a.span, sy * a.span)) continue;
         size_t o = (size_t)(sy * a.span) * a.d.pitch + sx * a.span;
         float dx = fxp[o], dy = fyp[o];
         float len = (dx * dx) + (dy * dy);
@@ -2439,9 +2460,70 @@ __global__ void __launch_bounds__(1024) sample_kernel(SampleArgs a)
     }
 }
 
+__global__ void __launch_bounds__(1024) sample_kernel(SampleArgs a)
+{
+    const int b = blockIdx.x;
+    if (a.counted && a.counts[b] == 0) return; // OK pair: nothing to compact (block-uniform)
+    sample_body(a, b, SkipNone{});
+}
+
+__global__ void __launch_bounds__(1024) sample_ignore_kernel(SampleArgs a, IgnoreRegions g)
+{
+    __shared__ int4 rects[kMaxIgnore];
+    const int b = blockIdx.x;
+    // counts[b] written by the fused last iteration (K5, K5s, the strip kernel's LAST form) is the count WITHOUT the regions, an
+    // upper bound of the count with them: a pair with 0 there has 0 here too and may exit with counts[b] == 0 as it stands.  Any
+    // other pair is counted again below, with the regions, and counts[b] rewritten -- so the hot kernels need no ignore form.
+    if (a.counted && a.counts[b] == 0) return; // block-uniform
+    const int n = min(g.n[b], kMaxIgnore);
+    if ((int)threadIdx.x < n) rects[threadIdx.x] = g.rects[(size_t)b * kMaxIgnore + threadIdx.x];
+    __syncthreads();
+    sample_body(a, b, SkipRegions{rects, n});
+}
+
 cudaError_t launch_sample(cudaStream_t s, const SampleArgs &a)
 {
     sample_kernel<<<a.batch, 1024, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_sample_ignore(cudaStream_t s, const SampleArgs &a, const IgnoreRegions &g)
+{
+    sample_ignore_kernel<<<a.batch, 1024, 0, s>>>(a, g);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------------
+// Ignore regions, step 1: the expected pixels inside each region replace the target's (after the +-5 px resize, before the level
+// images).  One CTA per (region, pair); warp = row, lane = 16-byte column where the row segment is aligned, bytes at its ends.
+// The expected and target slots of a pair share their alignment (spitch and H * spitch are multiples of 16).  Overlapping regions
+// write the same bytes, so the CTAs need no ordering.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) ignore_paint_kernel(uint8_t *src, int H, int spitch, IgnoreRegions g)
+{
+    const int b = blockIdx.y, r = blockIdx.x;
+    if (r >= g.n[b]) return;
+    const int4 q = g.rects[(size_t)b * kMaxIgnore + r];
+    const uint8_t *e = src + (size_t)b * 2 * H * spitch;
+    uint8_t *t = src + ((size_t)b * 2 + 1) * H * spitch;
+    const int a0 = (q.x + 15) & ~15, a1 = q.z & ~15; // the 16-byte aligned columns [a0, a1) of [x0, x1)
+    const int lane = threadIdx.x & 31;
+    for (int y = q.y + (int)(threadIdx.x >> 5); y < q.w; y += 8) {
+        const size_t row = (size_t)y * spitch;
+        if (a0 < a1) {
+            for (int x = a0 + 16 * lane; x < a1; x += 16 * 32)
+                *reinterpret_cast<uint4 *>(t + row + x) = *reinterpret_cast<const uint4 *>(e + row + x);
+            for (int x = q.x + lane; x < a0; x += 32) t[row + x] = e[row + x];
+            for (int x = a1 + lane; x < q.z; x += 32) t[row + x] = e[row + x];
+        } else {
+            for (int x = q.x + lane; x < q.z; x += 32) t[row + x] = e[row + x];
+        }
+    }
+}
+
+cudaError_t launch_ignore_paint(cudaStream_t s, uint8_t *src, int H, int spitch, const IgnoreRegions &g, int batch)
+{
+    ignore_paint_kernel<<<dim3(kMaxIgnore, batch), 256, 0, s>>>(src, H, spitch, g);
     return cudaGetLastError();
 }
 

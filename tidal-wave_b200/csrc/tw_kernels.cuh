@@ -159,4 +159,18 @@ struct SampleArgs {
 };
 cudaError_t launch_sample(cudaStream_t s, const SampleArgs &a);
 
+// Ignore regions (tw_compare_ignore and the other *_ignore entry points): up to kMaxIgnore rectangles per pair, clipped to the
+// frame on the host and stored as non-empty half-open bounds int4 (x0, y0, x1, y1).  Pairs without regions have n[b] = 0.
+constexpr int kMaxIgnore = 32; // TW_MAX_IGNORE
+struct IgnoreRegions {
+    const int4 *rects; // [B][kMaxIgnore]
+    const int *n;      // [B]
+};
+// Copies the expected pixels inside each region over the target slot of src ([B][2][H][spitch] u8): the flow is then the
+// ordinary flow of (expected, painted target).  Grid (kMaxIgnore, batch), one CTA per (region, pair).
+cudaError_t launch_ignore_paint(cudaStream_t s, uint8_t *src, int H, int spitch, const IgnoreRegions &g, int batch);
+// sample_kernel with the point test of the regions: a sample point inside any region of its pair yields no vector and is not
+// counted.  Same arguments as launch_sample (a.counted included: see the early exit of the kernel).
+cudaError_t launch_sample_ignore(cudaStream_t s, const SampleArgs &a, const IgnoreRegions &g);
+
 } // namespace tw

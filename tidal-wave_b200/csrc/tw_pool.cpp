@@ -33,11 +33,13 @@ struct Request { // Request, src/message_queue.h:13-18 (decoded images; `own` ho
     const uint8_t *expect, *target;
     int ew, eh, tw, th;
     std::shared_ptr<uint8_t> own_e, own_t; // pinned buffers of the pool's image store, returned to it when the request is done
+    std::vector<tw_rect> ignore;           // ignore regions, copied at submit time
 };
 
 struct FileJob { // Request as the reference has it: two paths (src/message_queue.h:13-18)
     long long id;
     std::string expect, target;
+    std::vector<tw_rect> ignore;
 };
 
 struct Slot {
@@ -97,6 +99,29 @@ void publish(tw_pool *p, long long id, const tw_result &res, const tw_vector *ve
     if (nvec > 0) s.vectors.assign(vec, vec + nvec);
     s.done = true;
     if (res.status == TW_STATUS_ERROR) p->error_count++; else p->data_count++; // Manager::notify, src/manager.cpp:109-114
+}
+
+// The frame-independent checks of an ignore-region list (tw_compare_ignore clips to the frame): "" if it is good, else the reason.
+std::string check_ignore(const tw_rect *r, int n)
+{
+    if (n < 0 || n > TW_MAX_IGNORE) return "bad ignore region: 0 to " + std::to_string(TW_MAX_IGNORE) + " regions per pair";
+    if (n > 0 && !r) return "bad ignore region: NULL list with a count > 0";
+    for (int i = 0; i < n; i++)
+        if (r[i].width < 1 || r[i].height < 1) return "bad ignore region: width and height must be >= 1";
+    return "";
+}
+
+// Registers a new request (p->mu held).  A bad ignore-region list answers it at once with TW_BAD_PARAMETER; returns false then.
+bool new_request(tw_pool *p, long long &id, const std::string &bad_ignore)
+{
+    id = p->next_id++;
+    Slot &s = p->slots[id];
+    p->request_count++; // Manager::request, src/manager.cpp:75-76
+    if (bad_ignore.empty()) return true;
+    fill_error(&s.res, TW_BAD_PARAMETER, bad_ignore.c_str());
+    s.done = true;
+    p->error_count++;
+    return false;
 }
 
 // imread of both paths (src/opticalflow.cpp:20-49) on a decoder thread, then the request joins the compute queue.
@@ -179,6 +204,7 @@ void decoder_main(tw_pool *p)
         }
         Request r{};
         r.id = job.id;
+        r.ignore = std::move(job.ignore);
         tw_result e;
         bool ok = true;
         // src/opticalflow.cpp:20-49: empty paths are BadParameter, unreadable / undecodable files BadImageFormat "Can't open <path>"
@@ -228,6 +254,8 @@ void consumer_main(tw_pool *p, int idx)
     std::vector<tw_result> res(p->batch);
     std::vector<Request> work;
     std::vector<const uint8_t *> ex(p->batch), tg(p->batch);
+    std::vector<const tw_rect *> ig(p->batch);
+    std::vector<int> nig(p->batch);
     // Up to two batches are in flight on the context (tw_pipe_*): while batch k runs, this thread pops and uploads batch k + 1
     // and then collects batch k - 1 -- one consumer thread per GPU keeps the device busy (src/consumer.cpp:18-24).
     struct InFlight { std::vector<Request> work; int cap = 0; };
@@ -291,17 +319,24 @@ void consumer_main(tw_pool *p, int idx)
             // error cases and the +-5 px resize path of OpticalFlow::calculate (src/opticalflow.cpp:37-68): synchronous, pipe drained
             while (!inflight.empty()) collect_oldest();
             if (vec.size() < (size_t)cap) vec.resize(cap);
-            tw_compare(ctx, r0.expect, r0.ew, r0.eh, r0.target, r0.tw, r0.th, &p->param, p->threshold, p->span, vec.data(), cap, &res[0]);
+            tw_compare_ignore(ctx, r0.expect, r0.ew, r0.eh, r0.target, r0.tw, r0.th, &p->param, p->threshold, p->span, r0.ignore.data(),
+                              (int)r0.ignore.size(), vec.data(), cap, &res[0]);
             publish(p, r0.id, res[0], vec.data(), std::min(res[0].n_vectors, cap));
             p->cv_res.notify_all();
             continue;
         }
         const int n = (int)work.size();
-        for (int i = 0; i < n; i++) { ex[i] = work[i].expect; tg[i] = work[i].target; }
+        bool any_ignore = false; // pairs with and without regions share a batch; one with regions runs the ignore form
+        for (int i = 0; i < n; i++) {
+            ex[i] = work[i].expect; tg[i] = work[i].target;
+            ig[i] = work[i].ignore.data(); nig[i] = (int)work[i].ignore.size();
+            any_ignore |= nig[i] > 0;
+        }
         if (!inflight.empty() && (inflight.back().work[0].ew != r0.ew || inflight.back().work[0].eh != r0.eh))
             while (!inflight.empty()) collect_oldest(); // a new size rebuilds the plan: nothing may be in flight
         if (tw_pipe_pending(ctx) >= 2) collect_oldest();
-        int rc = tw_pipe_submit(ctx, n, ex.data(), tg.data(), r0.ew, r0.eh, r0.ew, &p->param, p->threshold, p->span);
+        int rc = tw_pipe_submit_ignore(ctx, n, ex.data(), tg.data(), r0.ew, r0.eh, r0.ew, &p->param, p->threshold, p->span, ig.data(),
+                                       any_ignore ? nig.data() : nullptr);
         if (rc != TW_OK) {
             tw_result e;
             fill_error(&e, rc, tw_last_error(ctx));
@@ -362,27 +397,35 @@ tw_pool *tw_pool_create(const int *devices, int n_devices, int max_w, int max_h,
     return p;
 }
 
-long long tw_pool_submit(tw_pool *p, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_)
+long long tw_pool_submit_ignore(tw_pool *p, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
+                                const tw_rect *ignore, int n_ignore)
 {
     if (!p) return -1;
+    const std::string bad = check_ignore(ignore, n_ignore);
     long long id;
     {
         std::lock_guard<std::mutex> lk(p->mu);
         if (!p->running) return -1;
-        id = p->next_id++;
-        p->slots[id];
-        p->queue.push_back(Request{id, expect, target, ew, eh, tw_, th_});
-        p->request_count++; // Manager::request, src/manager.cpp:75-76
+        if (!new_request(p, id, bad)) { p->cv_res.notify_all(); return id; }
+        Request r{id, expect, target, ew, eh, tw_, th_};
+        if (n_ignore > 0) r.ignore.assign(ignore, ignore + n_ignore);
+        p->queue.push_back(std::move(r));
     }
     p->cv_req.notify_one();
     return id;
 }
 
+long long tw_pool_submit(tw_pool *p, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_)
+{
+    return tw_pool_submit_ignore(p, expect, ew, eh, target, tw_, th_, nullptr, 0);
+}
+
 // Manager::request as the reference has it (src/manager.cpp:68-78): two image PATHS.  The files are read and decoded on the pool's
 // decoder threads (cv::imread(IMREAD_GRAYSCALE), src/opticalflow.cpp:37,44 -> tw_decode_gray), started on first use.
-long long tw_pool_submit_files(tw_pool *p, const char *expect_path, const char *target_path)
+long long tw_pool_submit_files_ignore(tw_pool *p, const char *expect_path, const char *target_path, const tw_rect *ignore, int n_ignore)
 {
     if (!p) return -1;
+    const std::string bad = check_ignore(ignore, n_ignore);
     long long id;
     {
         std::lock_guard<std::mutex> lk(p->mu);
@@ -391,13 +434,18 @@ long long tw_pool_submit_files(tw_pool *p, const char *expect_path, const char *
             int n = p->n_decoders > 0 ? p->n_decoders : (int)std::min(32u, std::max(1u, std::thread::hardware_concurrency()));
             for (int i = 0; i < n; i++) p->decoders.emplace_back(decoder_main, p);
         }
-        id = p->next_id++;
-        p->slots[id];
-        p->files.push_back(FileJob{id, expect_path ? expect_path : "", target_path ? target_path : ""});
-        p->request_count++;
+        if (!new_request(p, id, bad)) { p->cv_res.notify_all(); return id; }
+        FileJob job{id, expect_path ? expect_path : "", target_path ? target_path : "", {}};
+        if (n_ignore > 0) job.ignore.assign(ignore, ignore + n_ignore);
+        p->files.push_back(std::move(job));
     }
     p->cv_file.notify_one();
     return id;
+}
+
+long long tw_pool_submit_files(tw_pool *p, const char *expect_path, const char *target_path)
+{
+    return tw_pool_submit_files_ignore(p, expect_path, target_path, nullptr, 0);
 }
 
 int tw_pool_set_decoders(tw_pool *p, int n)

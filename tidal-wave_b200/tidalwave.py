@@ -2,7 +2,11 @@
 
 Mirrors /root/reference/index.js:14-73 (directory pairing + lifecycle) and the option parsing of
 Broker::createInstance (/root/reference/src/broker.cpp:101-123, typed defaults :106-117, wrong-typed keys silently fall back
-to the default :190-209) on top of the dispatcher (tw_pool_*).  Files are decoded with ``imread_gray`` (PNG / JPEG / PGM,
+to the default :190-209) on top of the dispatcher (tw_pool_*).  Two options of this port have no reference counterpart:
+``ignoreRegions`` (a list of ``{x, y, width, height}`` in expected-image pixels, for every pair) and ``getIgnoreRegions(shortPath)``
+(a callable like ``getExpectedPath`` returning a pair's own list, or something falsy): parts of the page that are expected to change
+and are left out of the comparison (include/tidalwave_b200.h, tw_compare_ignore).  A pair's regions are the union of the two; a
+malformed region makes that pair an 'error' event rather than a comparison of the region it asked to ignore.  Files are decoded with ``imread_gray`` (PNG / JPEG / PGM,
 bit-exact to cv::imread IMREAD_GRAYSCALE); a file that cannot be decoded becomes the reference's "Can't open <path>" error.
 """
 from __future__ import annotations
@@ -10,7 +14,7 @@ from __future__ import annotations
 import glob
 import os
 
-from .api import OpticalFlowParameter, Pool, imread_gray
+from .api import OpticalFlowParameter, Pool, imread_gray, rect
 
 
 def _number(opts, key, default):
@@ -35,6 +39,8 @@ class TidalWave:
             pyrScale=_number(o, "pyrScale", 0.5), pyrLevels=_int32(o, "pyrLevels", 3), winSize=_int32(o, "winSize", 30),
             pyrIterations=_int32(o, "pyrIterations", 3), polyN=_int32(o, "polyN", 7), polySigma=_number(o, "polySigma", 1.5),
             flags=_int32(o, "flags", 256))
+        self.ignoreRegions = o.get("ignoreRegions")
+        self.getIgnoreRegions = o.get("getIgnoreRegions") if callable(o.get("getIgnoreRegions")) else None
         self._handlers = {"data": [], "error": [], "finish": []}
         self._pending = []   # (request id | None, expect path, target path, immediate error | None)
         self._report = {"request": 0, "data": 0, "error": 0}
@@ -63,8 +69,28 @@ class TidalWave:
             load().tw_pool_set_decoders(self._pool.pool, max(1, self.numThreads))
         return self._pool
 
-    def calc(self, expected: str, target: str):
-        """Broker::requestCalc -> Manager::request (src/broker.cpp:125-150, src/manager.cpp:68-78)."""
+    def ignore_regions(self, shortPath) -> list:
+        """The ignore regions of the pair whose target is ``shortPath`` (relative to targetDir): ``ignoreRegions`` followed by
+        ``getIgnoreRegions(shortPath)``, as ``(x, y, w, h)`` tuples.  Raises ValueError for a malformed list or region."""
+        regions = []
+        for src in (self.ignoreRegions, self.getIgnoreRegions(shortPath) if self.getIgnoreRegions else None):
+            if not src:
+                continue
+            if not isinstance(src, (list, tuple)):
+                raise ValueError(f"bad ignore region: {src!r} is not a list of regions")
+            regions += [rect(r) for r in src]
+        return regions
+
+    def reject(self, expected: str, target: str, reason: str):
+        """Counts a request that is answered with an 'error' event without being computed."""
+        if self._disposed:
+            return
+        self._report["request"] += 1
+        self._pending.append((None, expected, target, reason))
+
+    def calc(self, expected: str, target: str, ignore=None):
+        """Broker::requestCalc -> Manager::request (src/broker.cpp:125-150, src/manager.cpp:68-78).  ignore: regions of the
+        expected image left out of the comparison (see ignore_regions)."""
         if self._disposed:
             return
         self._report["request"] += 1
@@ -76,7 +102,8 @@ class TidalWave:
         # Manager::request with the two paths: the imreads run on the dispatcher's C++ decoder threads (numThreads of them, as the
         # reference decodes inside its numThreads consumers, src/consumer.cpp:54), the pair joins the compute queue when both are in
         pool = self._ensure_pool(0, 0)
-        self._pending.append((pool.request_files(expected, target), expected, target, None))
+        rid = pool.request_files(expected, target, ignore=ignore) if ignore else pool.request_files(expected, target)
+        self._pending.append((rid, expected, target, None))
 
     def flush(self):
         """Delivers every outstanding answer as 'data' / 'error' events (the uv_async hop of src/manager.cpp:102-125)."""
@@ -133,10 +160,16 @@ def _calc_all(t: TidalWave, targetDir, getExpectedPath):
     for target in sorted(glob.glob(os.path.join(base, "**", "*.*"), recursive=True)):
         if not os.path.isfile(target):
             continue
-        expected = getExpectedPath(os.path.relpath(target, base))
+        short = os.path.relpath(target, base)
+        expected = getExpectedPath(short)
         if not expected:
             continue  # index.js:50-51
-        t.calc(expected, target)  # FS.exists' answer is ignored by the reference too (index.js:57-58)
+        try:
+            regions = t.ignore_regions(short)
+        except ValueError as e:
+            t.reject(expected, target, str(e))
+            continue
+        t.calc(expected, target, regions)  # FS.exists' answer is ignored by the reference too (index.js:57-58)
     t.dispose()
     return t
 
