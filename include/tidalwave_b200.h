@@ -160,10 +160,44 @@ int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, cons
                           int stride, const tw_flow_param *param, double threshold, int span,
                           const tw_rect *const *ignore, const int *n_ignore);
 
+/* ---- ignore masks: leave chosen pixels of a page out of a comparison (a timestamp on every row of a feed, round avatars, shapes
+ * that are not rectangles, "dynamic element" masks rendered by the capture tool) ----
+ * A mask is an 8-bit plane the size of the EXPECTED image, in expected-image pixels like a region; nonzero means ignore.
+ * For a pair with a mask:
+ *   1. after the +-5 px resize of the target and before any flow work, every target pixel whose mask byte is nonzero is replaced by
+ *      the expected pixel at the same position;
+ *   2. a sample point (x, y) of the span grid whose mask byte is nonzero yields no vector and does not count toward n_vectors or the
+ *      status.
+ * A pair can have a mask, regions, both or neither; with both, the ignored set is their union.  So the result equals the plain
+ * compare of (expected, painted target) minus the vectors at ignored points, bit for bit.  A mask that is the rasterisation of a
+ * region list gives exactly the result of that list; an all-zero mask gives exactly the plain result.  A mask whose size differs
+ * from the expected image's (also when the target is resized: the mask follows the expected size) answers TW_BAD_PARAMETER with
+ * the reason "bad ignore mask: <mw>x<mh> mask for a <ew>x<eh> expected image" where the size is known (the pool's mask files, the
+ * Python binding); here the size is implied.  A NULL mask means "no mask".  With no mask on any pair the *_mask entry points are
+ * exactly their *_ignore counterparts (same kernels, same results). */
+
+/* tw_compare_ignore with an ignore mask: ew x eh bytes, tightly packed like expect; may be NULL. */
+int tw_compare_mask(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw, int th,
+                    const tw_flow_param *param, double threshold, int span, const tw_rect *ignore, int n_ignore,
+                    const uint8_t *mask, tw_vector *out, int cap, tw_result *res);
+/* tw_compare_batch_ignore with a mask per pair: pair i's mask is mask[i] (w x h bytes, rows `stride` apart like the images).
+ * mask == NULL: no masks; mask[i] == NULL: pair i has none. */
+int tw_compare_batch_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h,
+                          int stride, const tw_flow_param *param, double threshold, int span,
+                          const tw_rect *const *ignore, const int *n_ignore, const uint8_t *const *mask, tw_vector *out,
+                          int cap, tw_result *res);
+/* tw_pipe_submit_ignore with a mask per pair (as tw_compare_batch_mask).  The masks must stay valid until the batch has been
+ * collected, like its images; they travel with the batch, so the next batch's masks do not disturb one in flight.  The staging
+ * buffer grows to hold mask planes on the first masked batch (waiting for the batch in flight to take its images over); batches
+ * with and without masks alternate freely. */
+int tw_pipe_submit_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h,
+                        int stride, const tw_flow_param *param, double threshold, int span,
+                        const tw_rect *const *ignore, const int *n_ignore, const uint8_t *const *mask);
+
 /* ---- split phases of tw_compare_batch (same stream; used by the dispatcher to overlap, and by the
- * benchmark to time the device-resident pass separately from the PCIe legs).  They take no ignore regions: painting changes the
- * resident target, so only the whole-call entry points above apply them.  tw_batch_flow after a run with regions returns the flow of
- * the painted pair. ---- */
+ * benchmark to time the device-resident pass separately from the PCIe legs).  They take no ignore regions and no ignore masks:
+ * painting changes the resident target, so only the whole-call entry points above apply them.  tw_batch_flow after a run with
+ * regions or masks returns the flow of the painted pair. ---- */
 int tw_batch_upload(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w,
                     int h, int stride);                                     /* async H2D into the context */
 int tw_batch_run(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, double threshold,
@@ -259,6 +293,16 @@ long long tw_pool_submit_ignore(tw_pool *pool, const uint8_t *expect, int ew, in
                                 const tw_rect *ignore, int n_ignore);
 long long tw_pool_submit_files_ignore(tw_pool *pool, const char *expect_path, const char *target_path,
                                       const tw_rect *ignore, int n_ignore);
+/* The two submits with ignore regions and an ignore mask (see tw_compare_mask).  tw_pool_submit_mask: the mask (ew x eh bytes,
+ * or NULL) is caller-owned and must stay valid until the result has been taken, like the images.  tw_pool_submit_files_mask: the
+ * mask file (NULL or "": none) is read and decoded on the decoder threads with the two images, by tw_decode_gray, so it is a gray
+ * value: colour is converted as for the images and alpha is dropped.  A mask file that cannot be read or decoded answers that
+ * request alone with TW_BAD_IMAGE_FORMAT "Can't open <mask path>", one of another size than the expected image with
+ * TW_BAD_PARAMETER "bad ignore mask: ...".  Requests with masks, regions, both or neither share batches. */
+long long tw_pool_submit_mask(tw_pool *pool, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw, int th,
+                              const tw_rect *ignore, int n_ignore, const uint8_t *mask);
+long long tw_pool_submit_files_mask(tw_pool *pool, const char *expect_path, const char *target_path, const char *mask_path,
+                                    const tw_rect *ignore, int n_ignore);
 int tw_pool_set_decoders(tw_pool *pool, int n);
 /* Blocks until request `id` is answered; copies up to cap vectors.  Returns res->code, or <0 if dropped. */
 int tw_pool_wait(tw_pool *pool, long long id, tw_vector *out, int cap, tw_result *res);

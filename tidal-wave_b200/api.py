@@ -72,6 +72,24 @@ def _rects(regions):
     return ((tw_rect * len(rs))(*[tw_rect(*r) for r in rs]) if rs else None), len(rs)
 
 
+def mask_size_error(mask_shape, expect_shape) -> str:
+    """The library's reason for a mask of the wrong size (include/tidalwave_b200.h, tw_compare_mask)."""
+    (mh, mw), (eh, ew) = mask_shape, expect_shape
+    return f"bad ignore mask: {mw}x{mh} mask for a {ew}x{eh} expected image"
+
+
+def mask_array(mask):
+    """An ignore mask (2-D ``uint8`` or ``bool`` array in expected-image pixels, nonzero / True = ignore) -> a C-contiguous
+    ``uint8`` array, or None for None.  Raises ValueError for anything else; the size is checked against the expected image by the
+    callers (``mask_size_error``)."""
+    if mask is None:
+        return None
+    if not isinstance(mask, np.ndarray) or mask.ndim != 2 or mask.dtype not in (np.uint8, np.bool_):
+        raise ValueError(f"bad ignore mask: a 2-D uint8 or bool array expected, not {type(mask).__name__}"
+                         + (f" {mask.dtype} {mask.shape}" if isinstance(mask, np.ndarray) else ""))
+    return np.ascontiguousarray(mask.view(np.uint8) if mask.dtype == np.bool_ else mask)
+
+
 @dataclass
 class OpticalFlowParameter:
     pyrScale: float = 0.5
@@ -120,9 +138,17 @@ def load() -> C.CDLL:
     L.tw_compare_batch_ignore.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
                                           C.c_double, C.c_int, rpp, C.POINTER(C.c_int), C.POINTER(tw_vector), C.c_int,
                                           C.POINTER(tw_result)]
+    L.tw_compare_mask.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                  C.POINTER(tw_flow_param), C.c_double, C.c_int, C.POINTER(tw_rect), C.c_int, C.c_void_p,
+                                  C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
+    L.tw_compare_batch_mask.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
+                                        C.c_double, C.c_int, rpp, C.POINTER(C.c_int), u8pp, C.POINTER(tw_vector), C.c_int,
+                                        C.POINTER(tw_result)]
     L.tw_pipe_submit.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param), C.c_double, C.c_int]
     L.tw_pipe_submit_ignore.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
                                         C.c_double, C.c_int, rpp, C.POINTER(C.c_int)]
+    L.tw_pipe_submit_mask.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
+                                      C.c_double, C.c_int, rpp, C.POINTER(C.c_int), u8pp]
     L.tw_pipe_collect.argtypes = [C.c_void_p, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
     L.tw_pipe_pending.argtypes = [C.c_void_p]
     L.tw_pipe_ready.argtypes = [C.c_void_p]
@@ -162,6 +188,11 @@ def load() -> C.CDLL:
                                         C.POINTER(tw_rect), C.c_int]
     L.tw_pool_submit_files_ignore.restype = C.c_longlong
     L.tw_pool_submit_files_ignore.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p, C.POINTER(tw_rect), C.c_int]
+    L.tw_pool_submit_mask.restype = C.c_longlong
+    L.tw_pool_submit_mask.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
+                                      C.POINTER(tw_rect), C.c_int, C.c_void_p]
+    L.tw_pool_submit_files_mask.restype = C.c_longlong
+    L.tw_pool_submit_files_mask.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p, C.c_char_p, C.POINTER(tw_rect), C.c_int]
     L.tw_pool_set_decoders.argtypes = [C.c_void_p, C.c_int]
     L.tw_pool_peek.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_result)]
     L.tw_pool_wait.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
@@ -266,10 +297,13 @@ class OpticalFlow:
         return rc, fx, fy, sec.value
 
     def calculate(self, expectImg, targetImg, param: OpticalFlowParameter = OpticalFlowParameter(), threshold: float = 5.0,
-                  span: int = 10, cap: int | None = None, expect_image: str = "", target_image: str = "", ignore=None) -> dict:
+                  span: int = 10, cap: int | None = None, expect_image: str = "", target_image: str = "", ignore=None,
+                  ignore_mask=None) -> dict:
         """calculate + Consumer::run's sampling -> response dict (src/opticalflow.cpp:20-76, src/consumer.cpp:59-88).
         ignore: regions of the expected image left out of the comparison (``(x, y, w, h)`` tuples or ``{x, y, width, height}``
-        dicts, at most MAX_IGNORE; include/tidalwave_b200.h, tw_compare_ignore)."""
+        dicts, at most MAX_IGNORE; include/tidalwave_b200.h, tw_compare_ignore).  ignore_mask: pixels of the expected image left
+        out of the comparison, a 2-D ``uint8`` or ``bool`` array of the expected image's shape, nonzero = ignore (tw_compare_mask);
+        a mask of another shape answers an ERROR response "bad ignore mask: ..."."""
         a = None if expectImg is None else _u8(expectImg)
         b = None if targetImg is None else _u8(targetImg)
         eh, ew = a.shape if a is not None else (0, 0)
@@ -279,7 +313,15 @@ class OpticalFlow:
         vec = (tw_vector * cap)()
         res = tw_result()
         p = param.c()
-        if ignore is None:
+        m = mask_array(ignore_mask)
+        if m is not None and a is not None and m.shape != a.shape:
+            return {"status": "ERROR", "reason": mask_size_error(m.shape, a.shape), "code": BAD_PARAMETER}
+        if m is not None:
+            rs, nr = _rects(ignore)
+            self.lib.tw_compare_mask(self.ctx, a.ctypes.data if a is not None else None, ew, eh,
+                                     b.ctypes.data if b is not None else None, tw, th, C.byref(p), threshold, span, rs, nr,
+                                     m.ctypes.data, vec, cap, C.byref(res))
+        elif ignore is None:
             self.lib.tw_compare(self.ctx, a.ctypes.data if a is not None else None, ew, eh,
                                 b.ctypes.data if b is not None else None, tw, th, C.byref(p), threshold, span, vec, cap,
                                 C.byref(res))
@@ -291,8 +333,10 @@ class OpticalFlow:
         return _response(res, vec, min(res.n_vectors, cap), span, threshold, expect_image, target_image)
 
     def calculate_batch(self, pairs, param: OpticalFlowParameter = OpticalFlowParameter(), threshold: float = 5.0,
-                        span: int = 10, cap: int | None = None, ignore=None) -> list[dict]:
-        """ignore: one region list (or None) per pair, as in calculate()."""
+                        span: int = 10, cap: int | None = None, ignore=None, ignore_mask=None) -> list[dict]:
+        """ignore: one region list (or None) per pair, as in calculate().  ignore_mask: one mask (or None) per pair, as in
+        calculate(); a mask of another shape than the pairs' answers every pair with ERROR "bad ignore mask: ..." (as a bad region
+        list does)."""
         n = len(pairs)
         imgs = [(_u8(a), _u8(b)) for a, b in pairs]
         h, w = imgs[0][0].shape
@@ -303,15 +347,25 @@ class OpticalFlow:
         vec = (tw_vector * (cap * n))()
         res = (tw_result * n)()
         p = param.c()
-        if ignore is None:
+        if ignore is not None and len(ignore) != n:
+            raise ValueError("ignore: one region list per pair")
+        if ignore_mask is not None and len(ignore_mask) != n:
+            raise ValueError("ignore_mask: one mask (or None) per pair")
+        masks = [mask_array(m) for m in ignore_mask] if ignore_mask is not None else None
+        for m in masks or []:
+            if m is not None and m.shape != (h, w):
+                return [{"status": "ERROR", "reason": mask_size_error(m.shape, (h, w)), "code": BAD_PARAMETER} for _ in range(n)]
+        if ignore is None and masks is None:
             self.lib.tw_compare_batch(self.ctx, n, ex, tg, w, h, w, C.byref(p), threshold, span, vec, cap, res)
         else:
-            if len(ignore) != n:
-                raise ValueError("ignore: one region list per pair")
-            lists = [_rects(g) for g in ignore]
-            ig = (C.POINTER(tw_rect) * n)(*[C.cast(rs, C.POINTER(tw_rect)) if rs is not None else None for rs, _ in lists])
-            nig = (C.c_int * n)(*[k for _, k in lists])
-            self.lib.tw_compare_batch_ignore(self.ctx, n, ex, tg, w, h, w, C.byref(p), threshold, span, ig, nig, vec, cap, res)
+            lists = [_rects(g) for g in ignore] if ignore is not None else None
+            ig = (C.POINTER(tw_rect) * n)(*[C.cast(rs, C.POINTER(tw_rect)) if rs is not None else None for rs, _ in lists]) if lists else None
+            nig = (C.c_int * n)(*[k for _, k in lists]) if lists else None
+            if masks is None:
+                self.lib.tw_compare_batch_ignore(self.ctx, n, ex, tg, w, h, w, C.byref(p), threshold, span, ig, nig, vec, cap, res)
+            else:
+                mk = (C.c_void_p * n)(*[m.ctypes.data if m is not None else None for m in masks])
+                self.lib.tw_compare_batch_mask(self.ctx, n, ex, tg, w, h, w, C.byref(p), threshold, span, ig, nig, mk, vec, cap, res)
         out = []
         for i in range(n):
             sub = (tw_vector * cap).from_buffer(vec, i * cap * C.sizeof(tw_vector))
@@ -367,13 +421,22 @@ class Pool:
             raise RuntimeError("tw_pool_create failed: " + err.value.decode())
         self._keep = {}
 
-    def request(self, expectImg, targetImg, ignore=None) -> int:
-        """Manager::request (src/manager.cpp:68-78).  ignore: regions left out of the comparison, as in OpticalFlow.calculate."""
+    def request(self, expectImg, targetImg, ignore=None, ignore_mask=None) -> int:
+        """Manager::request (src/manager.cpp:68-78).  ignore / ignore_mask: regions and pixels left out of the comparison, as in
+        OpticalFlow.calculate; a mask of another shape than the expected image raises ValueError "bad ignore mask: ..." (no
+        request is made)."""
         a = None if expectImg is None else _u8(expectImg)
         b = None if targetImg is None else _u8(targetImg)
         eh, ew = a.shape if a is not None else (0, 0)
         th, tw = b.shape if b is not None else (0, 0)
-        if ignore is None:
+        m = mask_array(ignore_mask)
+        if m is not None and m.shape != (eh, ew):
+            raise ValueError(mask_size_error(m.shape, (eh, ew)))
+        if m is not None:
+            rs, nr = _rects(ignore)
+            rid = self.lib.tw_pool_submit_mask(self.pool, a.ctypes.data if a is not None else None, ew, eh,
+                                               b.ctypes.data if b is not None else None, tw, th, rs, nr, m.ctypes.data)
+        elif ignore is None:
             rid = self.lib.tw_pool_submit(self.pool, a.ctypes.data if a is not None else None, ew, eh,
                                           b.ctypes.data if b is not None else None, tw, th)
         else:
@@ -381,11 +444,17 @@ class Pool:
             rid = self.lib.tw_pool_submit_ignore(self.pool, a.ctypes.data if a is not None else None, ew, eh,
                                                  b.ctypes.data if b is not None else None, tw, th, rs, nr)
         if rid >= 0:
-            self._keep[rid] = (a, b)
+            self._keep[rid] = (a, b, m)
         return rid
 
-    def request_files(self, expect_path: str, target_path: str, ignore=None) -> int:
-        """Manager::request with two image paths (src/manager.cpp:68-78): read + decoded on the pool's C++ decoder threads."""
+    def request_files(self, expect_path: str, target_path: str, ignore=None, ignore_mask=None) -> int:
+        """Manager::request with two image paths (src/manager.cpp:68-78): read + decoded on the pool's C++ decoder threads.
+        ignore_mask: the path of a mask image (decoded to gray like the images, nonzero = ignore; include/tidalwave_b200.h,
+        tw_pool_submit_files_mask) or None."""
+        if ignore_mask is not None:
+            rs, nr = _rects(ignore)
+            return self.lib.tw_pool_submit_files_mask(self.pool, (expect_path or "").encode(), (target_path or "").encode(),
+                                                      os.fsencode(ignore_mask), rs, nr)
         if ignore is None:
             return self.lib.tw_pool_submit_files(self.pool, (expect_path or "").encode(), (target_path or "").encode())
         rs, nr = _rects(ignore)
@@ -394,7 +463,7 @@ class Pool:
     def wait(self, rid: int) -> dict | None:
         cap = self.cap
         if cap <= 0:  # all vectors: the request's own sampling grid (src/consumer.cpp:60-76)
-            a = self._keep.get(rid, (None, None))[0]
+            a = self._keep.get(rid, (None,))[0]
             if a is not None:
                 eh, ew = a.shape
                 cap = max(1, ((ew + self.span - 1) // self.span) * ((eh + self.span - 1) // self.span))

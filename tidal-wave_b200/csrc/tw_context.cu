@@ -19,9 +19,10 @@ using namespace tw;
 
 namespace {
 
-enum Family { F_LEVEL = 0, F_POLY, F_FIRST, F_GITER, F_GLAST, F_BVSUM, F_BITER, F_BLAST, F_BUPD, F_SAMPLE, F_PAINT, F_COUNT };
+enum Family { F_LEVEL = 0, F_POLY, F_FIRST, F_GITER, F_GLAST, F_BVSUM, F_BITER, F_BLAST, F_BUPD, F_SAMPLE, F_PAINT, F_MASK, F_COUNT };
 const char *kFamilyNames[F_COUNT] = {"level_image", "polyexp", "first_update", "gauss_iter", "gauss_last",
-                                     "box_vsum", "box_hscan", "box_hscan_last", "box_update", "sample", "ignore_paint"};
+                                     "box_vsum", "box_hscan", "box_hscan_last", "box_update", "sample", "ignore_paint",
+                                     "mask_paint"};
 
 struct Scale {
     int k, ksize;
@@ -55,15 +56,18 @@ struct LaunchOptions {
     }
 };
 
-// A plan's CUDA graph of the launch sequence (enqueue) is captured for one (n, threshold, span, options, result buffer, ignore) key.
-// `ignore`: the batch has ignore regions (paint launch first, the ignore form of the sample kernel).  The graph reads the regions
-// from the context's region buffer at fixed addresses, so new lists replay the same graph.
+// A plan's CUDA graph of the launch sequence (enqueue) is captured for one (n, threshold, span, options, result buffer, ignore,
+// mask) key.  `ignore`: the batch has ignore regions (paint launch first, the ignore form of the sample kernel).  `mask`: the batch
+// has ignore masks (mask paint launch first, the mask form of the sample kernel, which also tests the regions if `ignore`).  The
+// graph reads the regions from the context's region buffer and the masks from the plan's mask plane at fixed addresses, so new
+// lists and new masks replay the same graph.
 struct GraphKey {
     int n = 0; double thr = 0; int span = 0; LaunchOptions opt; const void *vectors = nullptr; int dev_cap = 0; bool ignore = false;
+    bool mask = false;
     bool operator==(const GraphKey &o) const
     {
         return n == o.n && thr == o.thr && span == o.span && opt == o.opt && vectors == o.vectors && dev_cap == o.dev_cap &&
-               ignore == o.ignore;
+               ignore == o.ignore && mask == o.mask;
     }
 };
 
@@ -80,6 +84,9 @@ struct Plan {
     double *V = nullptr; // box only
     float *T = nullptr;  // long pre-blur levels only: row-pass intermediate of launch_level_image_big
     bool fused_levels = false;
+    // ignore masks ([B][H][spitch] u8, nonzero = ignore) and their per-pair flags ([B] int): allocated on the plan's first masked batch
+    uint8_t *mask = nullptr;
+    int *mask_has = nullptr;
     // captured launch sequence (run_sequence): graph_exec replays graph_key; seen_key is the key of the last eager run
     GraphKey graph_key, seen_key;
     cudaGraphExec_t graph_exec = nullptr;
@@ -114,6 +121,7 @@ struct tw_ctx {
     // ignore regions of the batch being run: [max_batch][kMaxIgnore] int4 clipped bounds, then [max_batch] counts (ignore_bytes);
     // h_ignore is the page-locked mirror the synchronous entry points copy from
     void *d_ignore = nullptr, *h_ignore = nullptr;
+    int *h_mask_has = nullptr; // page-locked [max_batch]: which pairs of the batch have a mask (the plan holds the planes)
     void *d_vectors = nullptr;
     int dev_cap = 0;
     int last_n = 0, last_w = 0, last_h = 0;
@@ -134,6 +142,7 @@ struct tw_ctx {
         int *d_counts = nullptr, *h_counts = nullptr;
         void *d_vec = nullptr;
         void *h_ignore = nullptr; // page-locked: this batch's region lists, copied into the staging buffer behind its images
+        int *h_mask_has = nullptr; // page-locked [max_batch]: which pairs of this batch have a mask
         size_t vec_bytes = 0;
         int n = 0, w = 0, h = 0, dev_cap = 0;
     };
@@ -628,6 +637,19 @@ int pack_ignore(tw_ctx *ctx, int n, const tw_rect *const *ignore, const int *n_i
     return any;
 }
 
+// The plan's ignore-mask plane and flags (Plan::mask, mask_has), allocated on its first masked batch and freed with it.
+bool ensure_mask_plane(tw_ctx *ctx)
+{
+    Plan &pl = ctx->plan;
+    if (pl.mask) return true;
+    return dev_alloc(ctx, &pl.mask, (size_t)pl.batch * pl.H * pl.spitch) && dev_alloc(ctx, &pl.mask_has, (size_t)pl.batch);
+}
+
+IgnoreMasks ignore_masks(const Plan &pl) { return IgnoreMasks{pl.mask, pl.mask_has, pl.W, pl.H, pl.spitch}; }
+
+// Pipe staging buffer behind the images and the region lists (tw_pipe_submit_mask): [max_batch] int flags, then the planes.
+size_t mask_flag_bytes(int max_batch) { return ((size_t)max_batch * sizeof(int) + 255) & ~(size_t)255; }
+
 // Relaxed arithmetic (fmaf in the Gaussian window taps, mixed double / float horizontal pass of the polynomial
 // expansion) is used only for the option family it was validated on against the faithful oracle and cv2
 // (tools/relax_study.py, tests/test_gpu_parity.py): Gaussian window of the reference's default size or larger and
@@ -650,8 +672,9 @@ bool sparse_in_effect(const tw_ctx *ctx, int span)
 }
 
 // The launch sequence for n pairs already resident in plan.src.  SURVEY App. A.1 / A.7.  ignore: the batch has ignore regions
-// (in ctx->d_ignore): the target is painted first and the sample kernel leaves the points inside the regions out.
-bool enqueue(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
+// (in ctx->d_ignore): the target is painted first and the sample kernel leaves the points inside the regions out.  mask: the batch
+// has ignore masks (in plan.mask / mask_has): the same for the pixels and points under the masks.
+bool enqueue(tw_ctx *ctx, int n, double threshold, int span, bool ignore, bool mask)
 {
     Plan &pl = ctx->plan;
     const tw_flow_param &p = pl.p;
@@ -661,6 +684,8 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
     const size_t ns = pl.scales.size();
     // sampling is fused into the last Gaussian iteration of the finest scale when that kernel runs (radius 15 / 7)
     const bool fused_count = span > 0 && (p.flags & 256) && p.pyrIterations > 0 && (pl.win.m == 15 || pl.win.m == 7);
+    if (mask) // expected pixels over the target under the masks, before anything reads the target
+        LAUNCH(F_MASK, 0.0, launch_mask_paint(ctx->stream, pl.src, ignore_masks(pl), n));
     if (ignore) // expected pixels over the target inside the regions, before anything reads the target
         LAUNCH(F_PAINT, 0.0, launch_ignore_paint(ctx->stream, pl.src, H, pl.spitch, ignore_regions(ctx->d_ignore, ctx->max_batch), n));
     if (fused_count) {
@@ -752,7 +777,10 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
         SampleArgs sa{};
         sa.flow = f.flow; sa.d = f.d; sa.batch = n; sa.span = span; sa.thr2 = threshold * threshold;
         sa.counts = ctx->d_counts; sa.vectors = ctx->d_vectors; sa.cap = ctx->dev_cap; sa.counted = fused_count ? 1 : 0;
-        if (ignore) LAUNCH(F_SAMPLE, 0.0, launch_sample_ignore(ctx->stream, sa, ignore_regions(ctx->d_ignore, ctx->max_batch)));
+        if (mask)
+            LAUNCH(F_SAMPLE, 0.0, launch_sample_mask(ctx->stream, sa, ignore ? ignore_regions(ctx->d_ignore, ctx->max_batch) : IgnoreRegions{},
+                                                     ignore_masks(pl)));
+        else if (ignore) LAUNCH(F_SAMPLE, 0.0, launch_sample_ignore(ctx->stream, sa, ignore_regions(ctx->d_ignore, ctx->max_batch)));
         else LAUNCH(F_SAMPLE, 0.0, launch_sample(ctx->stream, sa));
     }
     return true;
@@ -762,12 +790,12 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
 // cudaGraphLaunch of the captured sequence (the step is ~22 short launches; at the coarse scales the kernels are
 // shorter than their launch gaps).  The first run of a key is always eager: it configures the per-device kernel
 // attributes and sizes the result buffers outside any capture.  Profiling (per-family events) runs eagerly.
-bool run_sequence(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
+bool run_sequence(tw_ctx *ctx, int n, double threshold, int span, bool ignore, bool mask)
 {
-    if (!ctx->opt_graph || ctx->profiling) return enqueue(ctx, n, threshold, span, ignore);
+    if (!ctx->opt_graph || ctx->profiling) return enqueue(ctx, n, threshold, span, ignore, mask);
     Plan &pl = ctx->plan;
     GraphKey key;
-    key.n = n; key.thr = threshold; key.span = span; key.opt = ctx->opt; key.ignore = ignore;
+    key.n = n; key.thr = threshold; key.span = span; key.opt = ctx->opt; key.ignore = ignore; key.mask = mask;
     key.vectors = ctx->d_vectors; key.dev_cap = ctx->dev_cap; // the captured sample kernel bakes both in
     if (pl.graph_exec && key == pl.graph_key) {
         cudaError_t e = cudaGraphLaunch(pl.graph_exec, ctx->stream);
@@ -776,7 +804,7 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
         return true;
     }
     if (!(key == pl.seen_key)) { // first run of this key: eager
-        if (!enqueue(ctx, n, threshold, span, ignore)) return false;
+        if (!enqueue(ctx, n, threshold, span, ignore, mask)) return false;
         pl.seen_key = key;
         pl.seen_key.vectors = ctx->d_vectors; pl.seen_key.dev_cap = ctx->dev_cap; // enqueue may have (re)allocated the result buffer
         return true;
@@ -789,9 +817,9 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
     if (e != cudaSuccess) { // capture unavailable: stay eager
         cudaGetLastError();
         ctx->opt_graph = 0;
-        return enqueue(ctx, n, threshold, span, ignore);
+        return enqueue(ctx, n, threshold, span, ignore, mask);
     }
-    const bool ok = enqueue(ctx, n, threshold, span, ignore);
+    const bool ok = enqueue(ctx, n, threshold, span, ignore, mask);
     e = cudaStreamEndCapture(ctx->stream, &graph);
     const long long captured = ctx->launches - before;
     ctx->launches = before;
@@ -800,7 +828,7 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
         cudaGetLastError();
         ctx->opt_graph = 0; // never retry on this context; the eager path is the same launch sequence
         if (!ok) return false;
-        return enqueue(ctx, n, threshold, span, ignore);
+        return enqueue(ctx, n, threshold, span, ignore, mask);
     }
     e = cudaGraphInstantiate(&pl.graph_exec, graph, 0);
     cudaGraphDestroy(graph);
@@ -808,7 +836,7 @@ bool run_sequence(tw_ctx *ctx, int n, double threshold, int span, bool ignore)
         cudaGetLastError();
         pl.graph_exec = nullptr;
         ctx->opt_graph = 0;
-        return enqueue(ctx, n, threshold, span, ignore);
+        return enqueue(ctx, n, threshold, span, ignore, mask);
     }
     pl.graph_key = key;
     pl.graph_launches = captured;
@@ -887,7 +915,8 @@ tw_ctx *tw_create(int device, int max_w, int max_h, int max_batch, char *err, in
     if ((e = cudaMalloc(&ctx->d_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
         (e = cudaMallocHost(&ctx->h_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
         (e = cudaMalloc(&ctx->d_ignore, ignore_bytes(ctx->max_batch))) != cudaSuccess ||
-        (e = cudaMallocHost(&ctx->h_ignore, ignore_bytes(ctx->max_batch))) != cudaSuccess) {
+        (e = cudaMallocHost(&ctx->h_ignore, ignore_bytes(ctx->max_batch))) != cudaSuccess ||
+        (e = cudaMallocHost(&ctx->h_mask_has, sizeof(int) * ctx->max_batch)) != cudaSuccess) {
         std::string m = cudaGetErrorString(e);
         tw_destroy(ctx);
         return fail(m);
@@ -908,6 +937,7 @@ void tw_destroy(tw_ctx *ctx)
     if (ctx->h_counts) cudaFreeHost(ctx->h_counts);
     if (ctx->d_ignore) cudaFree(ctx->d_ignore);
     if (ctx->h_ignore) cudaFreeHost(ctx->h_ignore);
+    if (ctx->h_mask_has) cudaFreeHost(ctx->h_mask_has);
     if (ctx->d_vectors) cudaFree(ctx->d_vectors);
     if (ctx->flush_buf) cudaFree(ctx->flush_buf);
     if (ctx->rs_buf) cudaFree(ctx->rs_buf);
@@ -925,6 +955,7 @@ void tw_destroy(tw_ctx *ctx)
             if (s.d_counts) cudaFree(s.d_counts);
             if (s.h_counts) cudaFreeHost(s.h_counts);
             if (s.h_ignore) cudaFreeHost(s.h_ignore);
+            if (s.h_mask_has) cudaFreeHost(s.h_mask_has);
             if (s.d_vec) cudaFree(s.d_vec);
         }
     }
@@ -1030,13 +1061,31 @@ static int upload_ignore(tw_ctx *ctx, int n, const tw_rect *const *ignore, const
     return TW_OK;
 }
 
+// Copies the ignore masks of n pairs of w x h frames (mask == NULL: none; mask[i] == NULL: pair i has none) into the plan's mask
+// plane and flags on the context's stream (the synchronous entry points; plan already built).  *any: some pair has a mask.
+static int upload_mask(tw_ctx *ctx, int n, const uint8_t *const *mask, int w, int h, int stride, bool *any)
+{
+    *any = false;
+    if (!mask) return TW_OK;
+    for (int i = 0; i < n; i++) *any |= (ctx->h_mask_has[i] = mask[i] ? 1 : 0) != 0;
+    if (!*any) return TW_OK;
+    if (!ensure_mask_plane(ctx)) return TW_CUDA_ERROR;
+    Plan &pl = ctx->plan;
+    cudaError_t e = cudaMemcpyAsync(pl.mask_has, ctx->h_mask_has, sizeof(int) * n, cudaMemcpyHostToDevice, ctx->stream);
+    for (int i = 0; i < n && e == cudaSuccess; i++)
+        if (mask[i])
+            e = cudaMemcpy2DAsync(pl.mask + (size_t)i * h * pl.spitch, pl.spitch, mask[i], stride, w, h, cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess) { set_err(ctx, "mask H2D", e); return TW_CUDA_ERROR; }
+    return TW_OK;
+}
+
 int tw_batch_upload(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride)
 {
     return upload_impl(ctx, n, expect, target, w, h, stride, nullptr);
 }
 
-// tw_batch_run; ignore: run the ignore form with the regions already in the region buffer
-static int run_batch(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, double threshold, int span, bool ignore)
+// tw_batch_run; ignore / mask: run the ignore / mask form with the regions / masks already in place
+static int run_batch(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, double threshold, int span, bool ignore, bool mask)
 {
     if (!ctx) return TW_BAD_PARAMETER;
     if (n < 1 || n > ctx->max_batch) { ctx->err = "bad batch"; return TW_BAD_PARAMETER; }
@@ -1062,7 +1111,7 @@ static int run_batch(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *para
         if (!ok) return TW_CUDA_ERROR;
     }
     cudaEventRecord(ctx->ev_r0, ctx->stream);
-    if (!run_sequence(ctx, n, threshold, span, ignore)) return TW_CUDA_ERROR;
+    if (!run_sequence(ctx, n, threshold, span, ignore, mask)) return TW_CUDA_ERROR;
     cudaEventRecord(ctx->ev_r1, ctx->stream);
     ctx->last_n = n; ctx->last_w = w; ctx->last_h = h; ctx->ran = true;
     ctx->last_sparse = sparse_in_effect(ctx, span);
@@ -1071,7 +1120,7 @@ static int run_batch(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *para
 
 int tw_batch_run(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *param, double threshold, int span)
 {
-    return run_batch(ctx, n, w, h, param, threshold, span, false);
+    return run_batch(ctx, n, w, h, param, threshold, span, false, false);
 }
 
 int tw_batch_fetch(tw_ctx *ctx, int n, tw_vector *out, int cap, tw_result *res)
@@ -1145,9 +1194,9 @@ int tw_flow(tw_ctx *ctx, const uint8_t *expect, const uint8_t *target, int w, in
     return TW_OK;
 }
 
-int tw_compare_batch_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
-                            const tw_flow_param *param, double threshold, int span, const tw_rect *const *ignore, const int *n_ignore,
-                            tw_vector *out, int cap, tw_result *res)
+int tw_compare_batch_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
+                          const tw_flow_param *param, double threshold, int span, const tw_rect *const *ignore, const int *n_ignore,
+                          const uint8_t *const *mask, tw_vector *out, int cap, tw_result *res)
 {
     if (!ctx || !res) return TW_BAD_PARAMETER;
     auto fail_all = [&](int code, const char *msg) {
@@ -1158,12 +1207,20 @@ int tw_compare_batch_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, co
     if (validate_param(param) != TW_OK) return fail_all(TW_BAD_PARAMETER, "bad optical-flow parameter");
     int rc = upload_impl(ctx, n, expect, target, w, h, stride, param);
     if (rc != TW_OK) return fail_all(rc, ctx->err.c_str());
-    bool any = false;
+    bool any = false, any_mask = false;
     rc = upload_ignore(ctx, n, ignore, n_ignore, w, h, &any);
+    if (rc == TW_OK) rc = upload_mask(ctx, n, mask, w, h, stride, &any_mask);
     if (rc != TW_OK) return fail_all(rc, ctx->err.c_str());
-    rc = run_batch(ctx, n, w, h, param, threshold, span, any);
+    rc = run_batch(ctx, n, w, h, param, threshold, span, any, any_mask);
     if (rc != TW_OK) return fail_all(rc, ctx->err.c_str());
     return tw_batch_fetch(ctx, n, out, cap, res);
+}
+
+int tw_compare_batch_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
+                            const tw_flow_param *param, double threshold, int span, const tw_rect *const *ignore, const int *n_ignore,
+                            tw_vector *out, int cap, tw_result *res)
+{
+    return tw_compare_batch_mask(ctx, n, expect, target, w, h, stride, param, threshold, span, ignore, n_ignore, nullptr, out, cap, res);
 }
 
 int tw_compare_batch(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
@@ -1188,8 +1245,9 @@ int tw_pipe_ready(tw_ctx *ctx)
     return cudaEventQuery(ctx->pipe.slot[ctx->pipe.head].done) == cudaSuccess ? 1 : 0;
 }
 
-int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
-                          const tw_flow_param *param, double threshold, int span, const tw_rect *const *ignore, const int *n_ignore)
+int tw_pipe_submit_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
+                        const tw_flow_param *param, double threshold, int span, const tw_rect *const *ignore, const int *n_ignore,
+                        const uint8_t *const *mask)
 {
     if (!ctx) return TW_BAD_PARAMETER;
     tw_ctx::Pipe &pp = ctx->pipe;
@@ -1214,7 +1272,8 @@ int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, cons
             if ((e = cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming)) != cudaSuccess || (e = cudaEventCreate(&s.r0)) != cudaSuccess ||
                 (e = cudaEventCreate(&s.r1)) != cudaSuccess || (e = cudaMalloc(&s.d_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
                 (e = cudaMallocHost(&s.h_counts, sizeof(int) * ctx->max_batch)) != cudaSuccess ||
-                (e = cudaMallocHost(&s.h_ignore, ignore_bytes(ctx->max_batch))) != cudaSuccess) { set_err(ctx, "pipe setup", e); return TW_CUDA_ERROR; }
+                (e = cudaMallocHost(&s.h_ignore, ignore_bytes(ctx->max_batch))) != cudaSuccess ||
+                (e = cudaMallocHost(&s.h_mask_has, sizeof(int) * ctx->max_batch)) != cudaSuccess) { set_err(ctx, "pipe setup", e); return TW_CUDA_ERROR; }
         }
     }
     // this batch's slot: free (at most one other batch in flight), its page-locked region mirror with it
@@ -1222,11 +1281,19 @@ int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, cons
     const int packed = pack_ignore(ctx, n, ignore, n_ignore, w, h, s.h_ignore);
     if (packed < 0) return TW_BAD_PARAMETER;
     const bool any = packed > 0;
-    // staging buffer: the images of max_batch pairs, then the region lists (ignore_bytes)
-    const size_t pair_bytes = (size_t)2 * h * pl.spitch, images = (size_t)ctx->max_batch * pair_bytes, need = images + ignore_bytes(ctx->max_batch);
-    if (pp.stage_bytes < need) { // only with nothing in flight (same_plan is false for a new size)
+    bool any_mask = false;
+    for (int i = 0; mask && i < n; i++) any_mask |= (s.h_mask_has[i] = mask[i] ? 1 : 0) != 0;
+    if (any_mask && !ensure_mask_plane(ctx)) return TW_CUDA_ERROR;
+    // staging buffer: the images of max_batch pairs, then the region lists (ignore_bytes); from the first masked batch on, then the
+    // mask flags and the mask planes (at mask_at, 256-byte aligned)
+    const size_t pair_bytes = (size_t)2 * h * pl.spitch, images = (size_t)ctx->max_batch * pair_bytes, plane = (size_t)h * pl.spitch;
+    const size_t mask_at = (images + ignore_bytes(ctx->max_batch) + 255) & ~(size_t)255, mask_planes = mask_at + mask_flag_bytes(ctx->max_batch);
+    const size_t need = any_mask ? mask_planes + ctx->max_batch * plane : images + ignore_bytes(ctx->max_batch);
+    if (pp.stage_bytes < need) { // a new plan: nothing in flight (same_plan is false for a new size); the first masked batch: the batch
+                                 // in flight, if any, must have taken its images over first
         cudaStreamSynchronize(pp.copy);
-        cudaStreamSynchronize(ctx->stream);
+        if (pp.count > 0) cudaEventSynchronize(pp.ev_stage_free);
+        else cudaStreamSynchronize(ctx->stream);
         if (pp.stage) cudaFree(pp.stage);
         pp.stage = nullptr; pp.stage_bytes = 0; pp.stage_used = false;
         if ((e = cudaMalloc(&pp.stage, need)) != cudaSuccess) { set_err(ctx, "cudaMalloc stage", e); return TW_CUDA_ERROR; }
@@ -1244,16 +1311,25 @@ int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, cons
         set_err(ctx, "regions H2D", e);
         return TW_CUDA_ERROR;
     }
+    if (any_mask) {
+        e = cudaMemcpyAsync(pp.stage + mask_at, s.h_mask_has, sizeof(int) * n, cudaMemcpyHostToDevice, pp.copy);
+        for (int i = 0; i < n && e == cudaSuccess; i++)
+            if (mask[i]) e = cudaMemcpy2DAsync(pp.stage + mask_planes + i * plane, pl.spitch, mask[i], stride, w, h, cudaMemcpyHostToDevice, pp.copy);
+        if (e != cudaSuccess) { set_err(ctx, "mask H2D", e); return TW_CUDA_ERROR; }
+    }
     cudaEventRecord(pp.ev_up, pp.copy);
-    // compute stream: the take-over copies run behind the previous batch's kernels, so its region lists stay put while they read them
+    // compute stream: the take-over copies run behind the previous batch's kernels, so its region lists and masks stay put while
+    // they read them
     cudaStreamWaitEvent(ctx->stream, pp.ev_up, 0);
     e = cudaMemcpyAsync(pl.src, pp.stage, (size_t)n * pair_bytes, cudaMemcpyDeviceToDevice, ctx->stream);
     if (e == cudaSuccess && any) e = cudaMemcpyAsync(ctx->d_ignore, pp.stage + images, ignore_bytes(ctx->max_batch), cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess && any_mask) e = cudaMemcpyAsync(pl.mask_has, pp.stage + mask_at, sizeof(int) * n, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess && any_mask) e = cudaMemcpyAsync(pl.mask, pp.stage + mask_planes, n * plane, cudaMemcpyDeviceToDevice, ctx->stream);
     if (e != cudaSuccess) { set_err(ctx, "stage -> src", e); return TW_CUDA_ERROR; }
     cudaEventRecord(pp.ev_stage_free, ctx->stream);
     pp.stage_used = true;
     cudaEventRecord(s.r0, ctx->stream);
-    if (!run_sequence(ctx, n, threshold, span, any)) return TW_CUDA_ERROR;
+    if (!run_sequence(ctx, n, threshold, span, any, any_mask)) return TW_CUDA_ERROR;
     cudaEventRecord(s.r1, ctx->stream);
     ctx->last_n = n; ctx->last_w = w; ctx->last_h = h; ctx->ran = true;
     ctx->last_sparse = sparse_in_effect(ctx, span);
@@ -1273,6 +1349,12 @@ int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, cons
     s.n = n; s.w = w; s.h = h; s.dev_cap = ctx->dev_cap;
     pp.count++;
     return TW_OK;
+}
+
+int tw_pipe_submit_ignore(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
+                          const tw_flow_param *param, double threshold, int span, const tw_rect *const *ignore, const int *n_ignore)
+{
+    return tw_pipe_submit_mask(ctx, n, expect, target, w, h, stride, param, threshold, span, ignore, n_ignore, nullptr);
 }
 
 int tw_pipe_submit(tw_ctx *ctx, int n, const uint8_t *const *expect, const uint8_t *const *target, int w, int h, int stride,
@@ -1319,9 +1401,9 @@ int tw_pipe_collect(tw_ctx *ctx, tw_vector *out, int cap, tw_result *res)
     return TW_OK;
 }
 
-int tw_compare_ignore(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
-                      const tw_flow_param *param, double threshold, int span, const tw_rect *ignore, int n_ignore,
-                      tw_vector *out, int cap, tw_result *res)
+int tw_compare_mask(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
+                    const tw_flow_param *param, double threshold, int span, const tw_rect *ignore, int n_ignore, const uint8_t *mask,
+                    tw_vector *out, int cap, tw_result *res)
 {
     if (!res) return TW_BAD_PARAMETER;
     if (!ctx) { fill_error(res, TW_BAD_PARAMETER, "null context"); return res->code; }
@@ -1336,15 +1418,24 @@ int tw_compare_ignore(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const 
         if (validate_param(param) != TW_OK) { fill_error(res, TW_BAD_PARAMETER, "bad optical-flow parameter"); return res->code; }
         int rc = upload_impl(ctx, 1, &expect, &expect, ew, eh, ew, param); // builds the plan, fills the expected slot
         if (rc == TW_OK && !upload_resized_target(ctx, target, tw_, th_, ew, eh)) rc = TW_CUDA_ERROR;
-        bool any = false; // regions are painted over the resized target (the paint kernel runs first in the launch sequence)
+        // regions and masks are painted over the resized target (the paint kernels run first in the launch sequence)
+        bool any = false, any_mask = false;
         if (rc == TW_OK) rc = upload_ignore(ctx, 1, &ignore, &n_ignore, ew, eh, &any);
-        if (rc == TW_OK) rc = run_batch(ctx, 1, ew, eh, param, threshold, span, any);
+        if (rc == TW_OK) rc = upload_mask(ctx, 1, &mask, ew, eh, ew, &any_mask);
+        if (rc == TW_OK) rc = run_batch(ctx, 1, ew, eh, param, threshold, span, any, any_mask);
         if (rc != TW_OK) { fill_error(res, rc, ctx->err.c_str()); return res->code; }
         tw_batch_fetch(ctx, 1, out, cap, res);
         return res->code;
     }
-    tw_compare_batch_ignore(ctx, 1, &expect, &target, ew, eh, ew, param, threshold, span, &ignore, &n_ignore, out, cap, res);
+    tw_compare_batch_mask(ctx, 1, &expect, &target, ew, eh, ew, param, threshold, span, &ignore, &n_ignore, &mask, out, cap, res);
     return res->code;
+}
+
+int tw_compare_ignore(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
+                      const tw_flow_param *param, double threshold, int span, const tw_rect *ignore, int n_ignore,
+                      tw_vector *out, int cap, tw_result *res)
+{
+    return tw_compare_mask(ctx, expect, ew, eh, target, tw_, th_, param, threshold, span, ignore, n_ignore, nullptr, out, cap, res);
 }
 
 int tw_compare(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,

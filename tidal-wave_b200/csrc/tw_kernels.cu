@@ -2481,6 +2481,32 @@ __global__ void __launch_bounds__(1024) sample_ignore_kernel(SampleArgs a, Ignor
     sample_body(a, b, SkipRegions{rects, n});
 }
 
+// The mask of one pair (NULL: the pair has none), then its regions as SkipRegions tests them.
+struct SkipMask {
+    const uint8_t *m;
+    int spitch;
+    SkipRegions r;
+    __device__ __forceinline__ bool operator()(int x, int y) const
+    {
+        if (m && m[(size_t)y * spitch + x]) return true;
+        return r(x, y);
+    }
+};
+
+__global__ void __launch_bounds__(1024) sample_mask_kernel(SampleArgs a, IgnoreRegions g, IgnoreMasks k)
+{
+    __shared__ int4 rects[kMaxIgnore];
+    const int b = blockIdx.x;
+    // A mask, like the regions, only removes sample points: the fused count is an upper bound here too, and the early exit of
+    // sample_ignore_kernel (see its comment) holds as it stands.
+    if (a.counted && a.counts[b] == 0) return; // block-uniform
+    const int n = g.n ? min(g.n[b], kMaxIgnore) : 0;
+    if ((int)threadIdx.x < n) rects[threadIdx.x] = g.rects[(size_t)b * kMaxIgnore + threadIdx.x];
+    __syncthreads();
+    const uint8_t *m = k.has[b] ? k.m + (size_t)b * k.H * k.spitch : nullptr;
+    sample_body(a, b, SkipMask{m, k.spitch, SkipRegions{rects, n}});
+}
+
 cudaError_t launch_sample(cudaStream_t s, const SampleArgs &a)
 {
     sample_kernel<<<a.batch, 1024, 0, s>>>(a);
@@ -2490,6 +2516,12 @@ cudaError_t launch_sample(cudaStream_t s, const SampleArgs &a)
 cudaError_t launch_sample_ignore(cudaStream_t s, const SampleArgs &a, const IgnoreRegions &g)
 {
     sample_ignore_kernel<<<a.batch, 1024, 0, s>>>(a, g);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_sample_mask(cudaStream_t s, const SampleArgs &a, const IgnoreRegions &g, const IgnoreMasks &k)
+{
+    sample_mask_kernel<<<a.batch, 1024, 0, s>>>(a, g, k);
     return cudaGetLastError();
 }
 
@@ -2524,6 +2556,48 @@ __global__ void __launch_bounds__(256) ignore_paint_kernel(uint8_t *src, int H, 
 cudaError_t launch_ignore_paint(cudaStream_t s, uint8_t *src, int H, int spitch, const IgnoreRegions &g, int batch)
 {
     ignore_paint_kernel<<<dim3(kMaxIgnore, batch), 256, 0, s>>>(src, H, spitch, g);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------------
+// Ignore masks, step 1: the expected pixels where the pair's mask is nonzero replace the target's (after the +-5 px resize, before
+// the level images).  Thread = 16 bytes of a row: expected, target and mask vectors in, t = m ? e : t per byte (__vcmpne4 gives
+// 0xff for every nonzero mask byte), the target vector out.  When W is not a multiple of 16 the last vector of a row reaches past
+// column W into the row's padding: that one goes byte by byte up to W, so the padding of the mask plane is never read.  The mask
+// plane shares the slots' pitch and alignment.  With ignore regions as well, both kernels write expected bytes, so their order
+// does not matter.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) mask_paint_kernel(uint8_t *src, IgnoreMasks k)
+{
+    const int b = blockIdx.y;
+    if (!k.has[b]) return; // block-uniform: pairs without a mask
+    const int nc = (k.W + 15) >> 4;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= k.H * nc) return;
+    const int y = i / nc, x = (i - y * nc) << 4;
+    const size_t plane = (size_t)k.H * k.spitch, row = (size_t)y * k.spitch + x;
+    const uint8_t *e = src + (size_t)b * 2 * plane + row;
+    uint8_t *t = src + ((size_t)b * 2 + 1) * plane + row;
+    const uint8_t *m = k.m + (size_t)b * plane + row;
+    if (x + 16 <= k.W) {
+        const uint4 ev = *reinterpret_cast<const uint4 *>(e), mv = *reinterpret_cast<const uint4 *>(m);
+        uint4 tv = *reinterpret_cast<const uint4 *>(t);
+        unsigned s;
+        s = __vcmpne4(mv.x, 0u); tv.x = (ev.x & s) | (tv.x & ~s);
+        s = __vcmpne4(mv.y, 0u); tv.y = (ev.y & s) | (tv.y & ~s);
+        s = __vcmpne4(mv.z, 0u); tv.z = (ev.z & s) | (tv.z & ~s);
+        s = __vcmpne4(mv.w, 0u); tv.w = (ev.w & s) | (tv.w & ~s);
+        *reinterpret_cast<uint4 *>(t) = tv;
+    } else {
+        for (int j = 0; j < k.W - x; j++)
+            if (m[j]) t[j] = e[j];
+    }
+}
+
+cudaError_t launch_mask_paint(cudaStream_t s, uint8_t *src, const IgnoreMasks &k, int batch)
+{
+    const long long threads = (long long)k.H * ((k.W + 15) >> 4);
+    mask_paint_kernel<<<dim3((unsigned)((threads + 255) / 256), batch), 256, 0, s>>>(src, k);
     return cudaGetLastError();
 }
 

@@ -173,4 +173,19 @@ cudaError_t launch_ignore_paint(cudaStream_t s, uint8_t *src, int H, int spitch,
 // counted.  Same arguments as launch_sample (a.counted included: see the early exit of the kernel).
 cudaError_t launch_sample_ignore(cudaStream_t s, const SampleArgs &a, const IgnoreRegions &g);
 
+// Ignore masks (tw_compare_mask and the other *_mask entry points): one u8 plane per pair in expected-image pixels, nonzero =
+// ignore, laid out like a slot of src ([B][H][spitch], 16-byte aligned rows; the bytes past column W are never read).  Pairs
+// without a mask have has[b] = 0 and their plane is not read.
+struct IgnoreMasks {
+    const uint8_t *m; // [B][H][spitch]
+    const int *has;   // [B]
+    int W, H, spitch;
+};
+// Copies the expected pixels where the pair's mask is nonzero over the target slot of src (as launch_ignore_paint does inside
+// regions).  One thread per 16 bytes of a row; grid (ceil(H * ceil(W / 16) / 256), batch).
+cudaError_t launch_mask_paint(cudaStream_t s, uint8_t *src, const IgnoreMasks &k, int batch);
+// sample_kernel with the point test of the pair's mask and then of its regions (g.n == NULL: no pair has regions).  Same
+// arguments as launch_sample_ignore.
+cudaError_t launch_sample_mask(cudaStream_t s, const SampleArgs &a, const IgnoreRegions &g, const IgnoreMasks &k);
+
 } // namespace tw

@@ -34,12 +34,15 @@ struct Request { // Request, src/message_queue.h:13-18 (decoded images; `own` ho
     int ew, eh, tw, th;
     std::shared_ptr<uint8_t> own_e, own_t; // pinned buffers of the pool's image store, returned to it when the request is done
     std::vector<tw_rect> ignore;           // ignore regions, copied at submit time
+    const uint8_t *mask = nullptr;         // ignore mask (ew x eh) or NULL; caller-owned, or held by own_m for path-based requests
+    std::shared_ptr<uint8_t> own_m;
 };
 
 struct FileJob { // Request as the reference has it: two paths (src/message_queue.h:13-18)
     long long id;
     std::string expect, target;
     std::vector<tw_rect> ignore;
+    std::string mask; // "" = no mask
 };
 
 struct Slot {
@@ -109,6 +112,12 @@ std::string check_ignore(const tw_rect *r, int n)
     for (int i = 0; i < n; i++)
         if (r[i].width < 1 || r[i].height < 1) return "bad ignore region: width and height must be >= 1";
     return "";
+}
+
+std::string bad_mask_size(int mw, int mh, int ew, int eh)
+{
+    return "bad ignore mask: " + std::to_string(mw) + "x" + std::to_string(mh) + " mask for a " + std::to_string(ew) + "x" +
+           std::to_string(eh) + " expected image";
 }
 
 // Registers a new request (p->mu held).  A bad ignore-region list answers it at once with TW_BAD_PARAMETER; returns false then.
@@ -212,6 +221,12 @@ void decoder_main(tw_pool *p)
         else if (job.target.empty()) { fill_error(&e, TW_BAD_PARAMETER, "TargetImagePath is empty."); ok = false; }
         else if (!imread_gray(p, job.expect, raw, r.own_e, r.ew, r.eh)) { fill_error(&e, TW_BAD_IMAGE_FORMAT, ("Can't open " + job.expect).c_str()); ok = false; }
         else if (!imread_gray(p, job.target, raw, r.own_t, r.tw, r.th)) { fill_error(&e, TW_BAD_IMAGE_FORMAT, ("Can't open " + job.target).c_str()); ok = false; }
+        else if (!job.mask.empty()) { // the ignore mask: a gray image of the expected image's size, into the same image store
+            int mw = 0, mh = 0;
+            if (!imread_gray(p, job.mask, raw, r.own_m, mw, mh)) { fill_error(&e, TW_BAD_IMAGE_FORMAT, ("Can't open " + job.mask).c_str()); ok = false; }
+            else if (mw != r.ew || mh != r.eh) { fill_error(&e, TW_BAD_PARAMETER, bad_mask_size(mw, mh, r.ew, r.eh).c_str()); ok = false; }
+            else r.mask = r.own_m.get();
+        }
         if (!ok) {
             publish(p, job.id, e, nullptr, 0);
             std::lock_guard<std::mutex> lk(p->mu);
@@ -256,6 +271,7 @@ void consumer_main(tw_pool *p, int idx)
     std::vector<const uint8_t *> ex(p->batch), tg(p->batch);
     std::vector<const tw_rect *> ig(p->batch);
     std::vector<int> nig(p->batch);
+    std::vector<const uint8_t *> mk(p->batch);
     // Up to two batches are in flight on the context (tw_pipe_*): while batch k runs, this thread pops and uploads batch k + 1
     // and then collects batch k - 1 -- one consumer thread per GPU keeps the device busy (src/consumer.cpp:18-24).
     struct InFlight { std::vector<Request> work; int cap = 0; };
@@ -319,24 +335,27 @@ void consumer_main(tw_pool *p, int idx)
             // error cases and the +-5 px resize path of OpticalFlow::calculate (src/opticalflow.cpp:37-68): synchronous, pipe drained
             while (!inflight.empty()) collect_oldest();
             if (vec.size() < (size_t)cap) vec.resize(cap);
-            tw_compare_ignore(ctx, r0.expect, r0.ew, r0.eh, r0.target, r0.tw, r0.th, &p->param, p->threshold, p->span, r0.ignore.data(),
-                              (int)r0.ignore.size(), vec.data(), cap, &res[0]);
+            tw_compare_mask(ctx, r0.expect, r0.ew, r0.eh, r0.target, r0.tw, r0.th, &p->param, p->threshold, p->span, r0.ignore.data(),
+                            (int)r0.ignore.size(), r0.mask, vec.data(), cap, &res[0]);
             publish(p, r0.id, res[0], vec.data(), std::min(res[0].n_vectors, cap));
             p->cv_res.notify_all();
             continue;
         }
         const int n = (int)work.size();
-        bool any_ignore = false; // pairs with and without regions share a batch; one with regions runs the ignore form
+        // pairs with and without regions / masks share a batch; one with regions runs the ignore form, one with a mask the mask form
+        bool any_ignore = false, any_mask = false;
         for (int i = 0; i < n; i++) {
             ex[i] = work[i].expect; tg[i] = work[i].target;
             ig[i] = work[i].ignore.data(); nig[i] = (int)work[i].ignore.size();
+            mk[i] = work[i].mask;
             any_ignore |= nig[i] > 0;
+            any_mask |= mk[i] != nullptr;
         }
         if (!inflight.empty() && (inflight.back().work[0].ew != r0.ew || inflight.back().work[0].eh != r0.eh))
             while (!inflight.empty()) collect_oldest(); // a new size rebuilds the plan: nothing may be in flight
         if (tw_pipe_pending(ctx) >= 2) collect_oldest();
-        int rc = tw_pipe_submit_ignore(ctx, n, ex.data(), tg.data(), r0.ew, r0.eh, r0.ew, &p->param, p->threshold, p->span, ig.data(),
-                                       any_ignore ? nig.data() : nullptr);
+        int rc = tw_pipe_submit_mask(ctx, n, ex.data(), tg.data(), r0.ew, r0.eh, r0.ew, &p->param, p->threshold, p->span, ig.data(),
+                                     any_ignore ? nig.data() : nullptr, any_mask ? mk.data() : nullptr);
         if (rc != TW_OK) {
             tw_result e;
             fill_error(&e, rc, tw_last_error(ctx));
@@ -397,8 +416,8 @@ tw_pool *tw_pool_create(const int *devices, int n_devices, int max_w, int max_h,
     return p;
 }
 
-long long tw_pool_submit_ignore(tw_pool *p, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
-                                const tw_rect *ignore, int n_ignore)
+long long tw_pool_submit_mask(tw_pool *p, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
+                              const tw_rect *ignore, int n_ignore, const uint8_t *mask)
 {
     if (!p) return -1;
     const std::string bad = check_ignore(ignore, n_ignore);
@@ -409,10 +428,17 @@ long long tw_pool_submit_ignore(tw_pool *p, const uint8_t *expect, int ew, int e
         if (!new_request(p, id, bad)) { p->cv_res.notify_all(); return id; }
         Request r{id, expect, target, ew, eh, tw_, th_};
         if (n_ignore > 0) r.ignore.assign(ignore, ignore + n_ignore);
+        r.mask = mask;
         p->queue.push_back(std::move(r));
     }
     p->cv_req.notify_one();
     return id;
+}
+
+long long tw_pool_submit_ignore(tw_pool *p, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_,
+                                const tw_rect *ignore, int n_ignore)
+{
+    return tw_pool_submit_mask(p, expect, ew, eh, target, tw_, th_, ignore, n_ignore, nullptr);
 }
 
 long long tw_pool_submit(tw_pool *p, const uint8_t *expect, int ew, int eh, const uint8_t *target, int tw_, int th_)
@@ -422,7 +448,8 @@ long long tw_pool_submit(tw_pool *p, const uint8_t *expect, int ew, int eh, cons
 
 // Manager::request as the reference has it (src/manager.cpp:68-78): two image PATHS.  The files are read and decoded on the pool's
 // decoder threads (cv::imread(IMREAD_GRAYSCALE), src/opticalflow.cpp:37,44 -> tw_decode_gray), started on first use.
-long long tw_pool_submit_files_ignore(tw_pool *p, const char *expect_path, const char *target_path, const tw_rect *ignore, int n_ignore)
+long long tw_pool_submit_files_mask(tw_pool *p, const char *expect_path, const char *target_path, const char *mask_path,
+                                    const tw_rect *ignore, int n_ignore)
 {
     if (!p) return -1;
     const std::string bad = check_ignore(ignore, n_ignore);
@@ -435,12 +462,17 @@ long long tw_pool_submit_files_ignore(tw_pool *p, const char *expect_path, const
             for (int i = 0; i < n; i++) p->decoders.emplace_back(decoder_main, p);
         }
         if (!new_request(p, id, bad)) { p->cv_res.notify_all(); return id; }
-        FileJob job{id, expect_path ? expect_path : "", target_path ? target_path : "", {}};
+        FileJob job{id, expect_path ? expect_path : "", target_path ? target_path : "", {}, mask_path ? mask_path : ""};
         if (n_ignore > 0) job.ignore.assign(ignore, ignore + n_ignore);
         p->files.push_back(std::move(job));
     }
     p->cv_file.notify_one();
     return id;
+}
+
+long long tw_pool_submit_files_ignore(tw_pool *p, const char *expect_path, const char *target_path, const tw_rect *ignore, int n_ignore)
+{
+    return tw_pool_submit_files_mask(p, expect_path, target_path, nullptr, ignore, n_ignore);
 }
 
 long long tw_pool_submit_files(tw_pool *p, const char *expect_path, const char *target_path)

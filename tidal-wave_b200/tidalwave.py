@@ -6,7 +6,12 @@ to the default :190-209) on top of the dispatcher (tw_pool_*).  Two options of t
 ``ignoreRegions`` (a list of ``{x, y, width, height}`` in expected-image pixels, for every pair) and ``getIgnoreRegions(shortPath)``
 (a callable like ``getExpectedPath`` returning a pair's own list, or something falsy): parts of the page that are expected to change
 and are left out of the comparison (include/tidalwave_b200.h, tw_compare_ignore).  A pair's regions are the union of the two; a
-malformed region makes that pair an 'error' event rather than a comparison of the region it asked to ignore.  Files are decoded with ``imread_gray`` (PNG / JPEG / PGM,
+malformed region makes that pair an 'error' event rather than a comparison of the region it asked to ignore.  Ignore masks (per-pixel,
+nonzero = ignore, the expected image's size; tw_compare_mask) come from ``ignoreMaskDir`` (a directory holding a mask image at the same
+short path as the target; a pair with no file there has no mask) or, if that is not a string, from ``getIgnoreMaskPath(shortPath)``
+(a callable returning a mask path, or something falsy for none).  A pair's mask and regions are ignored together; a mask file that
+cannot be decoded, or of another size than the expected image, makes that pair an 'error' event.  Wrong-typed values of these
+options mean "no mask", as for the reference's options.  Files are decoded with ``imread_gray`` (PNG / JPEG / PGM,
 bit-exact to cv::imread IMREAD_GRAYSCALE); a file that cannot be decoded becomes the reference's "Can't open <path>" error.
 """
 from __future__ import annotations
@@ -41,6 +46,8 @@ class TidalWave:
             flags=_int32(o, "flags", 256))
         self.ignoreRegions = o.get("ignoreRegions")
         self.getIgnoreRegions = o.get("getIgnoreRegions") if callable(o.get("getIgnoreRegions")) else None
+        self.ignoreMaskDir = o.get("ignoreMaskDir") if isinstance(o.get("ignoreMaskDir"), str) else None
+        self.getIgnoreMaskPath = o.get("getIgnoreMaskPath") if callable(o.get("getIgnoreMaskPath")) else None
         self._handlers = {"data": [], "error": [], "finish": []}
         self._pending = []   # (request id | None, expect path, target path, immediate error | None)
         self._report = {"request": 0, "data": 0, "error": 0}
@@ -81,6 +88,19 @@ class TidalWave:
             regions += [rect(r) for r in src]
         return regions
 
+    def ignore_mask_path(self, shortPath):
+        """The ignore-mask file of the pair whose target is ``shortPath`` (relative to targetDir), or None: the file at the same short
+        path under ``ignoreMaskDir`` if there is one there, else (without ``ignoreMaskDir``) what ``getIgnoreMaskPath(shortPath)``
+        returns if it is a non-empty path."""
+        if self.ignoreMaskDir is not None:
+            path = os.path.abspath(os.path.join(self.ignoreMaskDir, shortPath))
+            return path if os.path.isfile(path) else None
+        if self.getIgnoreMaskPath is not None:
+            path = self.getIgnoreMaskPath(shortPath)
+            if isinstance(path, (str, os.PathLike)) and os.fspath(path):
+                return os.fspath(path)
+        return None
+
     def reject(self, expected: str, target: str, reason: str):
         """Counts a request that is answered with an 'error' event without being computed."""
         if self._disposed:
@@ -88,9 +108,10 @@ class TidalWave:
         self._report["request"] += 1
         self._pending.append((None, expected, target, reason))
 
-    def calc(self, expected: str, target: str, ignore=None):
+    def calc(self, expected: str, target: str, ignore=None, ignore_mask=None):
         """Broker::requestCalc -> Manager::request (src/broker.cpp:125-150, src/manager.cpp:68-78).  ignore: regions of the
-        expected image left out of the comparison (see ignore_regions)."""
+        expected image left out of the comparison (see ignore_regions); ignore_mask: the path of a mask image (see
+        ignore_mask_path) or None."""
         if self._disposed:
             return
         self._report["request"] += 1
@@ -102,7 +123,10 @@ class TidalWave:
         # Manager::request with the two paths: the imreads run on the dispatcher's C++ decoder threads (numThreads of them, as the
         # reference decodes inside its numThreads consumers, src/consumer.cpp:54), the pair joins the compute queue when both are in
         pool = self._ensure_pool(0, 0)
-        rid = pool.request_files(expected, target, ignore=ignore) if ignore else pool.request_files(expected, target)
+        if ignore_mask:
+            rid = pool.request_files(expected, target, ignore=ignore or None, ignore_mask=ignore_mask)
+        else:
+            rid = pool.request_files(expected, target, ignore=ignore) if ignore else pool.request_files(expected, target)
         self._pending.append((rid, expected, target, None))
 
     def flush(self):
@@ -169,7 +193,7 @@ def _calc_all(t: TidalWave, targetDir, getExpectedPath):
         except ValueError as e:
             t.reject(expected, target, str(e))
             continue
-        t.calc(expected, target, regions)  # FS.exists' answer is ignored by the reference too (index.js:57-58)
+        t.calc(expected, target, regions, t.ignore_mask_path(short))  # FS.exists' answer is ignored by the reference too (index.js:57-58)
     t.dispose()
     return t
 
