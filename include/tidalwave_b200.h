@@ -194,6 +194,37 @@ int tw_pipe_submit_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const 
                         int stride, const tw_flow_param *param, double threshold, int span,
                         const tw_rect *const *ignore, const int *n_ignore, const uint8_t *const *mask);
 
+/* ---- change regions: where a page changed, as connected groups of its suspicious sample points (option "change_regions") ----
+ * Grid: the sample points are (i * span, j * span) for 0 <= i < ceil(W / span), 0 <= j < ceil(H / span), in EXPECTED-image pixels
+ * (after the +-5 px resize, as for vectors).  A point is suspicious when it yields a vector.  Points under ignore regions or masks
+ * yield none, so they belong to no region and do not connect regions: a mask stripe through a changed area splits it in two.
+ * Connectivity: two suspicious points are connected when their grid indices differ by at most 1 on each axis (8-connectivity); a
+ * change region is a connected component.  Per region:
+ *   rect       the bounding box of the span cells its points stand for: point (x, y) stands for [x, min(x + span, W)) x
+ *              [y, min(y + span, H)), so rect = (min x, min y, min(max x + span, W) - min x, min(max y + span, H) - min y);
+ *   n_vectors  the number of its points;
+ *   peak       its vector (x, y, dx, dy as in the vector list) with the largest len = f32(f32(dx * dx) + f32(dy * dy)), the value
+ *              the classification computes; a tie goes to the earlier point in scan order.
+ * Order: by first point in row-major scan order (the order of their first vectors in the vector list), which is the label order of
+ * scipy.ndimage.label(grid, structure=np.ones((3, 3))).  n_regions is always the full count; the first TW_MAX_CHANGE_REGIONS in
+ * that order are stored.  Sum of n_vectors over the regions == tw_result.n_vectors whenever n_regions <= TW_MAX_CHANGE_REGIONS.
+ * OK pairs, ERROR pairs and runs with span <= 0 have 0 regions.  Regions do not depend on the caller's vector cap: they are labelled
+ * on the device from the full vector list.  The output is a function of the vector set alone: eager runs and graph replays, the
+ * dense and sparse last iteration, the window kernels and both arithmetics (wherever their vectors agree) give identical bytes.
+ * The rect is an ignore region's type: accepting a change for the next run is a copy of it into the pair's ignore list. */
+#define TW_MAX_CHANGE_REGIONS 1024
+typedef struct tw_change_region {
+    tw_rect rect;      /* expected-image pixels, the same type as an ignore region */
+    int n_vectors;
+    tw_vector peak;    /* offset 24; sizeof 48 on LP64 */
+} tw_change_region;
+
+/* The change regions of pair `pair` of the batch that the last tw_compare*, tw_batch_fetch or tw_pipe_collect answered (those calls
+ * copy them to the host when "change_regions" was 1 for that batch): min(cap, n_regions, TW_MAX_CHANGE_REGIONS) entries to out
+ * (out may be NULL when cap is 0), the full count to *n_regions.  TW_BAD_PARAMETER if that batch ran without the option or pair is
+ * out of range.  Set the option with tw_set_option(ctx, "change_regions", 1); it is refused while pipe batches are pending. */
+int tw_change_regions(tw_ctx *ctx, int pair, tw_change_region *out, int cap, int *n_regions);
+
 /* ---- split phases of tw_compare_batch (same stream; used by the dispatcher to overlap, and by the
  * benchmark to time the device-resident pass separately from the PCIe legs).  They take no ignore regions and no ignore masks:
  * painting changes the resident target, so only the whole-call entry points above apply them.  tw_batch_flow after a run with
@@ -237,7 +268,10 @@ const char *tw_last_error(tw_ctx *ctx);
  *   "polyexp_tma" = 1: interior input tiles of the relaxed polynomial expansion are staged by one TMA tensor-map copy instead of
  *                     per-thread loads (bit-identical; measured 5 % slower, hence opt-in; TW_POLY_TMA=1 sets the default).
  *   "level_generic", "level_unfused", "tight_pitch", "box_unfused": alternative code paths (also the fall-backs of unusual
- *                     options) that the parity tests force. */
+ *                     options) that the parity tests force.
+ *   "change_regions" = 1: each run with span > 0 also groups every pair's vectors into change regions on the device (one more
+ *                     launch, after the sample kernel; tw_change_regions reads them).  Default 0.  TW_BAD_PARAMETER while pipe
+ *                     batches are pending. */
 int tw_set_option(tw_ctx *ctx, const char *name, int value);
 /* Process-wide default of "arithmetic" for contexts created afterwards (the dispatcher's consumers included). */
 int tw_set_default_arithmetic(int relaxed);
@@ -304,8 +338,15 @@ long long tw_pool_submit_mask(tw_pool *pool, const uint8_t *expect, int ew, int 
 long long tw_pool_submit_files_mask(tw_pool *pool, const char *expect_path, const char *target_path, const char *mask_path,
                                     const tw_rect *ignore, int n_ignore);
 int tw_pool_set_decoders(tw_pool *pool, int n);
+/* on = 1: every consumer runs with "change_regions" and keeps each request's regions (tw_pool_wait_regions), whatever vector_cap
+ * is.  Valid before the first submit (TW_OK), TW_BAD_PARAMETER after. */
+int tw_pool_set_change_regions(tw_pool *pool, int on);
 /* Blocks until request `id` is answered; copies up to cap vectors.  Returns res->code, or <0 if dropped. */
 int tw_pool_wait(tw_pool *pool, long long id, tw_vector *out, int cap, tw_result *res);
+/* tw_pool_wait plus the request's change regions: up to region_cap of them to regions, the full count to *n_regions (0 for an
+ * ERROR request and for a pool without change regions). */
+int tw_pool_wait_regions(tw_pool *pool, long long id, tw_vector *out, int cap, tw_result *res, tw_change_region *regions,
+                         int region_cap, int *n_regions);
 /* Blocks until request `id` is answered and copies its result WITHOUT taking it (res->n_vectors = the room tw_pool_wait needs).
  * Returns res->code, or <0 if dropped / unknown. */
 int tw_pool_peek(tw_pool *pool, long long id, tw_result *res);

@@ -24,6 +24,7 @@ HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "tidalwave_b200.h"
 OK, BAD_PARAMETER, BAD_IMAGE_FORMAT, DONT_MATCH_SIZE, CUDA_ERROR, UNSUPPORTED = range(6)
 STATUS_NAMES = {0: "OK", 1: "SUSPICIOUS", 2: "ERROR"}
 MAX_IGNORE = 32  # TW_MAX_IGNORE: ignore regions per pair
+MAX_CHANGE_REGIONS = 1024  # TW_MAX_CHANGE_REGIONS: change regions stored per pair
 
 
 class tw_flow_param(C.Structure):
@@ -43,6 +44,17 @@ class tw_result(C.Structure):
 class tw_rect(C.Structure):
     """An ignore region in expected-image pixels: [x, x + width) x [y, y + height)."""
     _fields_ = [("x", C.c_int), ("y", C.c_int), ("width", C.c_int), ("height", C.c_int)]
+
+
+class tw_change_region(C.Structure):
+    """A change region: the bounding box of a connected group of suspicious sample points (expected-image pixels), their count
+    and the vector with the largest length among them (include/tidalwave_b200.h, tw_change_regions)."""
+    _fields_ = [("rect", tw_rect), ("n_vectors", C.c_int), ("peak", tw_vector)]
+
+
+def _region_dicts(regs, n) -> list[dict]:
+    return [{"x": r.rect.x, "y": r.rect.y, "width": r.rect.width, "height": r.rect.height, "n_vectors": r.n_vectors,
+             "peak": {"x": r.peak.x, "y": r.peak.y, "dx": r.peak.dx, "dy": r.peak.dy}} for r in regs[:n]]
 
 
 def _int(v) -> int:
@@ -149,6 +161,7 @@ def load() -> C.CDLL:
                                         C.c_double, C.c_int, rpp, C.POINTER(C.c_int)]
     L.tw_pipe_submit_mask.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
                                       C.c_double, C.c_int, rpp, C.POINTER(C.c_int), u8pp]
+    L.tw_change_regions.argtypes = [C.c_void_p, C.c_int, C.POINTER(tw_change_region), C.c_int, C.POINTER(C.c_int)]
     L.tw_pipe_collect.argtypes = [C.c_void_p, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
     L.tw_pipe_pending.argtypes = [C.c_void_p]
     L.tw_pipe_ready.argtypes = [C.c_void_p]
@@ -196,6 +209,9 @@ def load() -> C.CDLL:
     L.tw_pool_set_decoders.argtypes = [C.c_void_p, C.c_int]
     L.tw_pool_peek.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_result)]
     L.tw_pool_wait.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
+    L.tw_pool_set_change_regions.argtypes = [C.c_void_p, C.c_int]
+    L.tw_pool_wait_regions.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result),
+                                       C.POINTER(tw_change_region), C.c_int, C.POINTER(C.c_int)]
     L.tw_pool_poll.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
     L.tw_pool_report.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
     L.tw_pool_stop.argtypes = [C.c_void_p]
@@ -263,6 +279,7 @@ class OpticalFlow:
         if not self.ctx:
             raise RuntimeError("tw_create failed: " + err.value.decode())
         self.max_batch = max_batch
+        self.change_regions = False  # set_option("change_regions", 1): responses carry "regions" and "n_regions"
 
     def close(self):
         if getattr(self, "ctx", None):
@@ -274,6 +291,22 @@ class OpticalFlow:
     def set_option(self, name: str, value: int):
         if self.lib.tw_set_option(self.ctx, name.encode(), int(value)) != 0:
             raise ValueError(self.last_error())
+        if name == "change_regions":
+            self.change_regions = bool(value)
+
+    def regions(self, pair: int = 0):
+        """(regions as dicts, n_regions) of pair ``pair`` of the last answered batch (tw_change_regions); raises ValueError if that
+        batch ran without the "change_regions" option."""
+        regs = (tw_change_region * MAX_CHANGE_REGIONS)()
+        n = C.c_int()
+        if self.lib.tw_change_regions(self.ctx, pair, regs, MAX_CHANGE_REGIONS, C.byref(n)) != 0:
+            raise ValueError(self.last_error())
+        return _region_dicts(regs, min(n.value, MAX_CHANGE_REGIONS)), n.value
+
+    def _with_regions(self, resp: dict, pair: int) -> dict:
+        if self.change_regions and resp["status"] != "ERROR":
+            resp["regions"], resp["n_regions"] = self.regions(pair)
+        return resp
 
     def last_error(self) -> str:
         return self.lib.tw_last_error(self.ctx).decode()
@@ -330,7 +363,7 @@ class OpticalFlow:
             self.lib.tw_compare_ignore(self.ctx, a.ctypes.data if a is not None else None, ew, eh,
                                        b.ctypes.data if b is not None else None, tw, th, C.byref(p), threshold, span, rs, nr,
                                        vec, cap, C.byref(res))
-        return _response(res, vec, min(res.n_vectors, cap), span, threshold, expect_image, target_image)
+        return self._with_regions(_response(res, vec, min(res.n_vectors, cap), span, threshold, expect_image, target_image), 0)
 
     def calculate_batch(self, pairs, param: OpticalFlowParameter = OpticalFlowParameter(), threshold: float = 5.0,
                         span: int = 10, cap: int | None = None, ignore=None, ignore_mask=None) -> list[dict]:
@@ -369,7 +402,7 @@ class OpticalFlow:
         out = []
         for i in range(n):
             sub = (tw_vector * cap).from_buffer(vec, i * cap * C.sizeof(tw_vector))
-            out.append(_response(res[i], sub, min(res[i].n_vectors, cap), span, threshold))
+            out.append(self._with_regions(_response(res[i], sub, min(res[i].n_vectors, cap), span, threshold), i))
         return out
 
     def batch_flow(self, pair: int, w: int, h: int):
@@ -407,9 +440,10 @@ class Pool:
     """Manager + Consumer pool (src/manager.cpp:40-98): one consumer thread per entry of ``devices``."""
 
     def __init__(self, devices, param: OpticalFlowParameter = OpticalFlowParameter(), threshold: float = 5.0, span: int = 10,
-                 max_w: int = 0, max_h: int = 0, batch: int = 1, vector_cap: int = 0):
+                 max_w: int = 0, max_h: int = 0, batch: int = 1, vector_cap: int = 0, change_regions: bool = False):
         """max_w / max_h = 0: no bound on the image size; vector_cap = 0: every vector of every request is returned (the capacity
-        follows each request's own sampling grid), > 0: at most that many (``n_vectors`` still holds the full count)."""
+        follows each request's own sampling grid), > 0: at most that many (``n_vectors`` still holds the full count).
+        change_regions: wait() answers also carry "regions" and "n_regions" (tw_pool_set_change_regions), whatever vector_cap is."""
         self.lib = load()
         self.span, self.threshold, self.cap = span, threshold, vector_cap
         err = C.create_string_buffer(256)
@@ -419,6 +453,11 @@ class Pool:
                                             err, 256)
         if not self.pool:
             raise RuntimeError("tw_pool_create failed: " + err.value.decode())
+        self.change_regions = bool(change_regions)
+        if self.change_regions:
+            if self.lib.tw_pool_set_change_regions(self.pool, 1) != OK:
+                self.close()
+                raise RuntimeError("tw_pool_set_change_regions refused: the pool has taken requests already")
         self._keep = {}
 
     def request(self, expectImg, targetImg, ignore=None, ignore_mask=None) -> int:
@@ -474,11 +513,19 @@ class Pool:
                 cap = max(1, info.n_vectors)
         vec = (tw_vector * cap)()
         res = tw_result()
-        rc = self.lib.tw_pool_wait(self.pool, rid, vec, cap, C.byref(res))
+        if not self.change_regions:
+            rc = self.lib.tw_pool_wait(self.pool, rid, vec, cap, C.byref(res))
+        else:
+            regs = (tw_change_region * MAX_CHANGE_REGIONS)()
+            nreg = C.c_int()
+            rc = self.lib.tw_pool_wait_regions(self.pool, rid, vec, cap, C.byref(res), regs, MAX_CHANGE_REGIONS, C.byref(nreg))
         self._keep.pop(rid, None)
         if rc < 0:
             return None
-        return _response(res, vec, min(res.n_vectors, cap), self.span, self.threshold)
+        resp = _response(res, vec, min(res.n_vectors, cap), self.span, self.threshold)
+        if self.change_regions and resp["status"] != "ERROR":
+            resp["regions"], resp["n_regions"] = _region_dicts(regs, min(nreg.value, MAX_CHANGE_REGIONS)), nreg.value
+        return resp
 
     def report(self) -> dict:
         a = C.c_int(); b = C.c_int(); c = C.c_int()

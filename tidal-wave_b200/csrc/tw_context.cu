@@ -19,10 +19,10 @@ using namespace tw;
 
 namespace {
 
-enum Family { F_LEVEL = 0, F_POLY, F_FIRST, F_GITER, F_GLAST, F_BVSUM, F_BITER, F_BLAST, F_BUPD, F_SAMPLE, F_PAINT, F_MASK, F_COUNT };
+enum Family { F_LEVEL = 0, F_POLY, F_FIRST, F_GITER, F_GLAST, F_BVSUM, F_BITER, F_BLAST, F_BUPD, F_SAMPLE, F_PAINT, F_MASK, F_REGIONS, F_COUNT };
 const char *kFamilyNames[F_COUNT] = {"level_image", "polyexp", "first_update", "gauss_iter", "gauss_last",
                                      "box_vsum", "box_hscan", "box_hscan_last", "box_update", "sample", "ignore_paint",
-                                     "mask_paint"};
+                                     "mask_paint", "change_regions"};
 
 struct Scale {
     int k, ksize;
@@ -49,10 +49,11 @@ struct LaunchOptions {
                           // bit-identical and measured 1-7 % slower (DESIGN.md section 4.2)
     int box_unfused = 0;  // 1: the three-launch box iteration (V plane through HBM), kept for the parity tests
     int level_generic = 0, level_unfused = 0;
+    int change_regions = 0; // 1: the change-region kernel runs after the sample kernel
     bool operator==(const LaunchOptions &o) const
     {
         return arith == o.arith && sparse_last == o.sparse_last && window_tiles == o.window_tiles && box_unfused == o.box_unfused &&
-               level_generic == o.level_generic && level_unfused == o.level_unfused;
+               level_generic == o.level_generic && level_unfused == o.level_unfused && change_regions == o.change_regions;
     }
 };
 
@@ -124,7 +125,15 @@ struct tw_ctx {
     int *h_mask_has = nullptr; // page-locked [max_batch]: which pairs of the batch have a mask (the plan holds the planes)
     void *d_vectors = nullptr;
     int dev_cap = 0;
-    int last_n = 0, last_w = 0, last_h = 0;
+    // change regions ("change_regions"): scratch [max_batch][2][reg_cap] int, sized with d_vectors (reg_cap == dev_cap when in use),
+    // the region counts [max_batch] and the regions [max_batch][kMaxChangeRegions] with their page-locked mirrors
+    int *d_reg_scratch = nullptr;
+    int reg_cap = 0;
+    int *d_nreg = nullptr, *h_nreg = nullptr;
+    tw_change_region *d_regions = nullptr, *h_regions = nullptr;
+    int reg_pairs = -1; // pairs of the last answered batch whose regions the mirror holds; -1: that batch ran without the option
+    int last_n = 0, last_w = 0, last_h = 0, last_span = 0;
+    bool last_regions = false; // the last run had "change_regions" on
     bool ran = false;
     // profiling
     bool profiling = false;
@@ -145,6 +154,10 @@ struct tw_ctx {
         int *h_mask_has = nullptr; // page-locked [max_batch]: which pairs of this batch have a mask
         size_t vec_bytes = 0;
         int n = 0, w = 0, h = 0, dev_cap = 0;
+        // change regions of this batch (regions: it ran with the option): device snapshot of the counts and regions, counts on the host
+        bool regions = false;
+        int *d_nreg = nullptr, *h_nreg = nullptr;
+        tw_change_region *d_regions = nullptr;
     };
     struct Pipe {
         cudaStream_t copy = nullptr, fetch = nullptr;
@@ -597,6 +610,43 @@ bool ensure_results(tw_ctx *ctx, int cap)
     return true;
 }
 
+static_assert(kMaxChangeRegions == TW_MAX_CHANGE_REGIONS && sizeof(tw_change_region) == 48, "tw_change_region as the kernel writes it");
+
+// The region counts and regions of the context (tw_ctx::d_nreg, d_regions) and their page-locked mirrors: allocated on first use,
+// at a fixed size, and kept until the context goes.
+bool ensure_region_mirrors(tw_ctx *ctx)
+{
+    if (ctx->h_regions) return true;
+    const size_t bytes = (size_t)ctx->max_batch * kMaxChangeRegions * sizeof(tw_change_region);
+    CK(cudaMalloc(&ctx->d_nreg, sizeof(int) * ctx->max_batch));
+    CK(cudaMallocHost(&ctx->h_nreg, sizeof(int) * ctx->max_batch));
+    CK(cudaMalloc(&ctx->d_regions, bytes));
+    CK(cudaMallocHost(&ctx->h_regions, bytes));
+    return true;
+}
+
+// Those and the scratch of the region kernel, for dev_cap.  The scratch follows the result buffer: it is reallocated only when
+// dev_cap changes, which changes the graph key as well, so no captured graph keeps a freed scratch.
+bool ensure_region_buffers(tw_ctx *ctx)
+{
+    if (!ensure_region_mirrors(ctx)) return false;
+    if (ctx->d_reg_scratch && ctx->reg_cap == ctx->dev_cap) return true;
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ctx->d_reg_scratch) cudaFree(ctx->d_reg_scratch);
+    ctx->d_reg_scratch = nullptr;
+    CK(cudaMalloc(&ctx->d_reg_scratch, (size_t)ctx->max_batch * 2 * ctx->dev_cap * sizeof(int)));
+    ctx->reg_cap = ctx->dev_cap;
+    return true;
+}
+
+// The host mirror now answers for a batch of n pairs: with 0 regions each if `on`, else for no pair (tw_change_regions refuses).
+void answer_regions(tw_ctx *ctx, int n, bool on)
+{
+    n = std::max(0, std::min(n, ctx->max_batch));
+    ctx->reg_pairs = on && ensure_region_mirrors(ctx) ? n : -1;
+    if (ctx->reg_pairs > 0) memset(ctx->h_nreg, 0, sizeof(int) * n);
+}
+
 // Region buffer (tw_ctx::d_ignore, h_ignore, the pipe's staging tail): [max_batch][kMaxIgnore] int4, then [max_batch] int.
 size_t ignore_bytes(int max_batch) { return (size_t)max_batch * (kMaxIgnore * sizeof(int4) + sizeof(int)); }
 
@@ -782,6 +832,13 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span, bool ignore, bool m
                                                      ignore_masks(pl)));
         else if (ignore) LAUNCH(F_SAMPLE, 0.0, launch_sample_ignore(ctx->stream, sa, ignore_regions(ctx->d_ignore, ctx->max_batch)));
         else LAUNCH(F_SAMPLE, 0.0, launch_sample(ctx->stream, sa));
+        if (ctx->opt.change_regions) {
+            if (!ensure_region_buffers(ctx)) return false;
+            ChangeRegionArgs ca{};
+            ca.vectors = ctx->d_vectors; ca.counts = ctx->d_counts; ca.cap = ctx->dev_cap; ca.w = f.d.w; ca.h = f.d.h; ca.span = span;
+            ca.scratch = ctx->d_reg_scratch; ca.n_regions = ctx->d_nreg; ca.regions = ctx->d_regions; ca.batch = n;
+            LAUNCH(F_REGIONS, 0.0, launch_change_regions(ctx->stream, ca));
+        }
     }
     return true;
 }
@@ -939,6 +996,11 @@ void tw_destroy(tw_ctx *ctx)
     if (ctx->h_ignore) cudaFreeHost(ctx->h_ignore);
     if (ctx->h_mask_has) cudaFreeHost(ctx->h_mask_has);
     if (ctx->d_vectors) cudaFree(ctx->d_vectors);
+    if (ctx->d_reg_scratch) cudaFree(ctx->d_reg_scratch);
+    if (ctx->d_nreg) cudaFree(ctx->d_nreg);
+    if (ctx->h_nreg) cudaFreeHost(ctx->h_nreg);
+    if (ctx->d_regions) cudaFree(ctx->d_regions);
+    if (ctx->h_regions) cudaFreeHost(ctx->h_regions);
     if (ctx->flush_buf) cudaFree(ctx->flush_buf);
     if (ctx->rs_buf) cudaFree(ctx->rs_buf);
     {
@@ -957,6 +1019,9 @@ void tw_destroy(tw_ctx *ctx)
             if (s.h_ignore) cudaFreeHost(s.h_ignore);
             if (s.h_mask_has) cudaFreeHost(s.h_mask_has);
             if (s.d_vec) cudaFree(s.d_vec);
+            if (s.d_nreg) cudaFree(s.d_nreg);
+            if (s.h_nreg) cudaFreeHost(s.h_nreg);
+            if (s.d_regions) cudaFree(s.d_regions);
         }
     }
     if (ctx->ev_t0) cudaEventDestroy(ctx->ev_t0);
@@ -1114,6 +1179,7 @@ static int run_batch(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *para
     if (!run_sequence(ctx, n, threshold, span, ignore, mask)) return TW_CUDA_ERROR;
     cudaEventRecord(ctx->ev_r1, ctx->stream);
     ctx->last_n = n; ctx->last_w = w; ctx->last_h = h; ctx->ran = true;
+    ctx->last_span = span; ctx->last_regions = ctx->opt.change_regions != 0;
     ctx->last_sparse = sparse_in_effect(ctx, span);
     return TW_OK;
 }
@@ -1128,9 +1194,13 @@ int tw_batch_fetch(tw_ctx *ctx, int n, tw_vector *out, int cap, tw_result *res)
     if (!ctx || !res) return TW_BAD_PARAMETER;
     if (!ctx->ran || n != ctx->last_n) { ctx->err = "tw_batch_fetch: nothing to fetch"; return TW_BAD_PARAMETER; }
     cudaSetDevice(ctx->device);
+    answer_regions(ctx, n, ctx->last_regions);
+    const bool labelled = ctx->last_regions && ctx->last_span > 0;
     cudaError_t e = cudaMemcpyAsync(ctx->h_counts, ctx->d_counts, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && labelled) e = cudaMemcpyAsync(ctx->h_nreg, ctx->d_nreg, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) {
+        answer_regions(ctx, n, ctx->last_regions);
         set_err(ctx, "fetch", e);
         for (int i = 0; i < n; i++) fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str());
         return TW_CUDA_ERROR;
@@ -1151,6 +1221,13 @@ int tw_batch_fetch(tw_ctx *ctx, int n, tw_vector *out, int cap, tw_result *res)
                                 sizeof(tw_vector) * ncopy, cudaMemcpyDeviceToHost, ctx->stream);
             if (e != cudaSuccess) { set_err(ctx, "fetch vectors", e); fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str()); }
         }
+        const int nreg = labelled ? std::min(ctx->h_nreg[i], kMaxChangeRegions) : 0;
+        if (nreg > 0 && res[i].code == TW_OK) {
+            e = cudaMemcpyAsync(ctx->h_regions + (size_t)i * kMaxChangeRegions, ctx->d_regions + (size_t)i * kMaxChangeRegions,
+                                sizeof(tw_change_region) * nreg, cudaMemcpyDeviceToHost, ctx->stream);
+            if (e != cudaSuccess) { set_err(ctx, "fetch regions", e); fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str()); }
+        }
+        if (res[i].code != TW_OK && ctx->reg_pairs > 0) ctx->h_nreg[i] = 0;
     }
     e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) { set_err(ctx, "fetch sync", e); return TW_CUDA_ERROR; }
@@ -1199,6 +1276,7 @@ int tw_compare_batch_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, cons
                           const uint8_t *const *mask, tw_vector *out, int cap, tw_result *res)
 {
     if (!ctx || !res) return TW_BAD_PARAMETER;
+    answer_regions(ctx, n, ctx->opt.change_regions != 0); // what an ERROR answer leaves: 0 regions per pair
     auto fail_all = [&](int code, const char *msg) {
         for (int i = 0; i < n; i++) fill_error(&res[i], code, msg);
         return code;
@@ -1332,6 +1410,7 @@ int tw_pipe_submit_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const 
     if (!run_sequence(ctx, n, threshold, span, any, any_mask)) return TW_CUDA_ERROR;
     cudaEventRecord(s.r1, ctx->stream);
     ctx->last_n = n; ctx->last_w = w; ctx->last_h = h; ctx->ran = true;
+    ctx->last_span = span; ctx->last_regions = ctx->opt.change_regions != 0;
     ctx->last_sparse = sparse_in_effect(ctx, span);
     // snapshot of the compact results (counts + vectors), then the counts to the host
     const size_t vbytes = (size_t)n * ctx->dev_cap * sizeof(tw_vector);
@@ -1344,6 +1423,19 @@ int tw_pipe_submit_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const 
     e = cudaMemcpyAsync(s.d_counts, ctx->d_counts, sizeof(int) * n, cudaMemcpyDeviceToDevice, ctx->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(s.d_vec, ctx->d_vectors, vbytes, cudaMemcpyDeviceToDevice, ctx->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_counts, s.d_counts, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
+    s.regions = ctx->last_regions;
+    if (e == cudaSuccess && s.regions) { // the change regions likewise: the host reads them on the fetch stream in tw_pipe_collect
+        if ((!s.d_nreg && (e = cudaMalloc(&s.d_nreg, sizeof(int) * ctx->max_batch)) != cudaSuccess) ||
+            (!s.h_nreg && (e = cudaMallocHost(&s.h_nreg, sizeof(int) * ctx->max_batch)) != cudaSuccess) ||
+            (!s.d_regions && (e = cudaMalloc(&s.d_regions, sizeof(tw_change_region) * ctx->max_batch * kMaxChangeRegions)) != cudaSuccess)) {
+            set_err(ctx, "cudaMalloc snapshot", e);
+            return TW_CUDA_ERROR;
+        }
+        e = cudaMemcpyAsync(s.d_nreg, ctx->d_nreg, sizeof(int) * n, cudaMemcpyDeviceToDevice, ctx->stream);
+        if (e == cudaSuccess)
+            e = cudaMemcpyAsync(s.d_regions, ctx->d_regions, sizeof(tw_change_region) * n * kMaxChangeRegions, cudaMemcpyDeviceToDevice, ctx->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_nreg, s.d_nreg, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
+    }
     if (e != cudaSuccess) { set_err(ctx, "snapshot", e); return TW_CUDA_ERROR; }
     cudaEventRecord(s.done, ctx->stream);
     s.n = n; s.w = w; s.h = h; s.dev_cap = ctx->dev_cap;
@@ -1372,6 +1464,7 @@ int tw_pipe_collect(tw_ctx *ctx, tw_vector *out, int cap, tw_result *res)
     tw_ctx::PipeSlot &s = pp.slot[pp.head];
     pp.head ^= 1; pp.count--;
     const int n = s.n;
+    answer_regions(ctx, n, s.regions);
     cudaError_t e = cudaEventSynchronize(s.done);
     if (e != cudaSuccess) {
         set_err(ctx, "collect", e);
@@ -1396,6 +1489,14 @@ int tw_pipe_collect(tw_ctx *ctx, tw_vector *out, int cap, tw_result *res)
             if (e != cudaSuccess) { set_err(ctx, "collect vectors", e); fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str()); }
             copied = true;
         }
+        const int nreg = s.regions ? std::min(s.h_nreg[i], kMaxChangeRegions) : 0;
+        if (nreg > 0 && res[i].code == TW_OK) {
+            e = cudaMemcpyAsync(ctx->h_regions + (size_t)i * kMaxChangeRegions, s.d_regions + (size_t)i * kMaxChangeRegions,
+                                sizeof(tw_change_region) * nreg, cudaMemcpyDeviceToHost, pp.fetch);
+            if (e != cudaSuccess) { set_err(ctx, "collect regions", e); fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str()); }
+            copied = true;
+        }
+        if (s.regions) ctx->h_nreg[i] = res[i].code == TW_OK ? s.h_nreg[i] : 0;
     }
     if (copied && (e = cudaStreamSynchronize(pp.fetch)) != cudaSuccess) { set_err(ctx, "collect sync", e); return TW_CUDA_ERROR; }
     return TW_OK;
@@ -1407,6 +1508,7 @@ int tw_compare_mask(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const ui
 {
     if (!res) return TW_BAD_PARAMETER;
     if (!ctx) { fill_error(res, TW_BAD_PARAMETER, "null context"); return res->code; }
+    answer_regions(ctx, 1, ctx->opt.change_regions != 0); // what an ERROR answer leaves: 0 regions
     // src/opticalflow.cpp:37-49: an image that cannot be opened is BadImageFormat
     if (!expect || ew < 1 || eh < 1) { fill_error(res, TW_BAD_IMAGE_FORMAT, "Can't open expected image"); return res->code; }
     if (!target || tw_ < 1 || th_ < 1) { fill_error(res, TW_BAD_IMAGE_FORMAT, "Can't open target image"); return res->code; }
@@ -1521,6 +1623,18 @@ int tw_profile_read(tw_ctx *ctx, int max_n, const char **names, float *ms, int *
 
 long long tw_launch_count(tw_ctx *ctx) { return ctx ? ctx->launches : 0; }
 
+int tw_change_regions(tw_ctx *ctx, int pair, tw_change_region *out, int cap, int *n_regions)
+{
+    if (!ctx) return TW_BAD_PARAMETER;
+    if (ctx->reg_pairs < 0) { ctx->err = "tw_change_regions: the last answered batch ran without \"change_regions\""; return TW_BAD_PARAMETER; }
+    if (pair < 0 || pair >= ctx->reg_pairs) { ctx->err = "tw_change_regions: pair out of range"; return TW_BAD_PARAMETER; }
+    const int total = ctx->h_nreg[pair];
+    const int k = std::min(std::min(cap, total), kMaxChangeRegions);
+    if (out && k > 0) memcpy(out, ctx->h_regions + (size_t)pair * kMaxChangeRegions, sizeof(tw_change_region) * k);
+    if (n_regions) *n_regions = total;
+    return TW_OK;
+}
+
 int tw_set_option(tw_ctx *ctx, const char *name, int value)
 {
     if (!ctx || !name) return TW_BAD_PARAMETER;
@@ -1543,6 +1657,11 @@ int tw_set_option(tw_ctx *ctx, const char *name, int value)
     if (!strcmp(name, "window_tiles")) { ctx->opt.window_tiles = value ? 1 : 0; return TW_OK; }
     if (!strcmp(name, "level_generic")) { ctx->opt.level_generic = value ? 1 : 0; return TW_OK; }
     if (!strcmp(name, "level_unfused")) { ctx->opt.level_unfused = value ? 1 : 0; return TW_OK; }
+    if (!strcmp(name, "change_regions")) { // the batches in flight were submitted with the other setting
+        if (ctx->pipe.count > 0) { ctx->err = "change_regions: collect the pending pipe batches first"; return TW_BAD_PARAMETER; }
+        ctx->opt.change_regions = value ? 1 : 0;
+        return TW_OK;
+    }
     if (!strcmp(name, "tight_pitch")) {
         ctx->opt_tight_pitch = value ? 1 : 0;
         ctx->plan.valid = false;

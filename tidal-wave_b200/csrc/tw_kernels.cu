@@ -2399,25 +2399,10 @@ struct SkipRegions {
     }
 };
 
-template <class Skip>
-__device__ __forceinline__ void sample_body(const SampleArgs &a, const int b, const Skip &skip)
+// Block-wide exclusive scan of one count per thread (blockDim.x a multiple of 32): returns the sum of the counts of the threads
+// before this one and leaves the block's sum in *total.  warp_sums[32] and *total are the caller's shared memory.
+__device__ __forceinline__ int block_exclusive_scan(const int cnt, int *warp_sums, int *total)
 {
-    __shared__ int warp_sums[32];
-    __shared__ int total;
-    const float *fxp = a.flow + (size_t)b * 2 * a.d.plane, *fyp = fxp + a.d.plane;
-    const int nsx = (a.d.w + a.span - 1) / a.span, nsy = (a.d.h + a.span - 1) / a.span, ns = nsx * nsy;
-    const int per = (ns + blockDim.x - 1) / blockDim.x;
-    const int i0 = min(threadIdx.x * per, ns), i1 = min(i0 + per, ns);
-    int cnt = 0;
-    for (int i = i0; i < i1; i++) {
-        int sy = i / nsx, sx = i - sy * nsx;
-        if (skip(sx * a.span, sy * a.span)) continue;
-        size_t o = (size_t)(sy * a.span) * a.d.pitch + sx * a.span;
-        float dx = fxp[o], dy = fyp[o];
-        float len = (dx * dx) + (dy * dy);
-        cnt += ((double)len > a.thr2) ? 1 : 0;
-    }
-    // block exclusive scan of cnt
     int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     int incl = cnt;
 #pragma unroll
@@ -2436,10 +2421,31 @@ __device__ __forceinline__ void sample_body(const SampleArgs &a, const int b, co
             if (lane >= off) s += u;
         }
         warp_sums[lane] = s - v; // exclusive
-        if (lane == 31) total = s;
+        if (lane == 31) *total = s;
     }
     __syncthreads();
-    int pos = warp_sums[wid] + incl - cnt;
+    return warp_sums[wid] + incl - cnt;
+}
+
+template <class Skip>
+__device__ __forceinline__ void sample_body(const SampleArgs &a, const int b, const Skip &skip)
+{
+    __shared__ int warp_sums[32];
+    __shared__ int total;
+    const float *fxp = a.flow + (size_t)b * 2 * a.d.plane, *fyp = fxp + a.d.plane;
+    const int nsx = (a.d.w + a.span - 1) / a.span, nsy = (a.d.h + a.span - 1) / a.span, ns = nsx * nsy;
+    const int per = (ns + blockDim.x - 1) / blockDim.x;
+    const int i0 = min(threadIdx.x * per, ns), i1 = min(i0 + per, ns);
+    int cnt = 0;
+    for (int i = i0; i < i1; i++) {
+        int sy = i / nsx, sx = i - sy * nsx;
+        if (skip(sx * a.span, sy * a.span)) continue;
+        size_t o = (size_t)(sy * a.span) * a.d.pitch + sx * a.span;
+        float dx = fxp[o], dy = fyp[o];
+        float len = (dx * dx) + (dy * dy);
+        cnt += ((double)len > a.thr2) ? 1 : 0;
+    }
+    int pos = block_exclusive_scan(cnt, warp_sums, &total);
     if (threadIdx.x == 0) a.counts[b] = total;
     if (cnt == 0) return;
     DevVector *out = reinterpret_cast<DevVector *>(a.vectors) + (size_t)b * a.cap;
@@ -2522,6 +2528,158 @@ cudaError_t launch_sample_ignore(cudaStream_t s, const SampleArgs &a, const Igno
 cudaError_t launch_sample_mask(cudaStream_t s, const SampleArgs &a, const IgnoreRegions &g, const IgnoreMasks &k)
 {
     sample_mask_kernel<<<a.batch, 1024, 0, s>>>(a, g, k);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------------
+// Change regions: the 8-connected components of a pair's suspicious sample points, labelled from its compact vector list, so every
+// last-iteration and sample form feeds it alike.  One CTA per pair; thread t owns the run [t * per, (t + 1) * per) of vector indices,
+// as sample_body owns sample points.
+//   1. the cell -> vector index map over the pair's sample grid.  It is not cleared: an entry counts only if the vector it names
+//      is in range and stands at that cell, which holds exactly for the cells that have a vector in this run.  A vector whose W
+//      neighbour is the previous vector of the same thread's run takes that run's parent directly (no global find);
+//   2. union-find (Playne and Hawick) over the neighbours W (first vector of a run), N, NW and NE, with the usual 8-connectivity
+//      decision: N alone if it is there (NW and NE are its row neighbours), else NW unless W is there (W reaches it through its
+//      own N), and NE; roots are joined by atomicMin on the parent of the larger one, so the root of a component is its smallest
+//      vector index -- its first point in scan order -- whatever the scheduling;
+//   3. flatten; the roots, in index order, take the region slots 0, 1, ... (block scan), and the slot of a root is kept in the map;
+//   4. each vector folds its point into its region if that is stored (slot < kMaxChangeRegions): atomicMin / atomicMax of the
+//      corners and atomicAdd of the count, summed over a thread's run of one region first; the peak is a 64-bit atomicMax of
+//      (len bits << 32 | ~index), held in peak.dx until step 5 (len >= 0 orders as its bits; the tie goes to the smaller index);
+//   5. one thread per stored region turns the corners into a rectangle clipped to the frame and the peak key into the vector.
+// Parents change under the other threads' atomics, so they are read through L2 (__ldcg); the region fields likewise in step 5.
+// ------------------------------------------------------------------------------------------------
+struct DevChangeRegion { int x, y, w, h, n, pad; DevVector peak; }; // tw_change_region
+
+__device__ __forceinline__ int uf_find(const int *par, int i)
+{
+    for (int q = __ldcg(par + i); q != i; q = __ldcg(par + i)) i = q;
+    return i;
+}
+
+__device__ __forceinline__ void uf_union(int *par, int a, int b)
+{
+    for (;;) {
+        a = uf_find(par, a); b = uf_find(par, b);
+        if (a == b) return;
+        if (a > b) { const int t = a; a = b; b = t; }
+        const int old = atomicMin(par + b, a);
+        if (old == b) return; // b was still a root: it now hangs below a
+        b = old;              // b was linked meanwhile: join a with where it went
+    }
+}
+
+__device__ __forceinline__ void fold_region(DevChangeRegion *r, int x0, int y0, int x1, int y1, int n, unsigned long long key)
+{
+    atomicMin(&r->x, x0); atomicMin(&r->y, y0);
+    atomicMax(&r->w, x1); atomicMax(&r->h, y1);
+    atomicAdd(&r->n, n);
+    atomicMax(reinterpret_cast<unsigned long long *>(&r->peak.dx), key);
+}
+
+__global__ void __launch_bounds__(1024) change_regions_kernel(ChangeRegionArgs a)
+{
+    __shared__ int warp_sums[32];
+    __shared__ int total;
+    const int b = blockIdx.x;
+    const int nv = min(a.counts[b], a.cap);
+    if (nv == 0) { // block-uniform: an OK pair has no region
+        if (threadIdx.x == 0) a.n_regions[b] = 0;
+        return;
+    }
+    const DevVector *v = reinterpret_cast<const DevVector *>(a.vectors) + (size_t)b * a.cap;
+    int *cell = a.scratch + (size_t)b * 2 * a.cap, *par = cell + a.cap;
+    DevChangeRegion *reg = reinterpret_cast<DevChangeRegion *>(a.regions) + (size_t)b * kMaxChangeRegions;
+    const int span = a.span, nsx = (a.w + span - 1) / span;
+    const int per = (nv + blockDim.x - 1) / blockDim.x;
+    const int i0 = min((int)threadIdx.x * per, nv), i1 = min(i0 + per, nv);
+    // the vector i's W neighbour is vector i - 1 (scan order) if that one stands one span to its left
+    auto has_w = [&](int i, int x, int y) { return i > 0 && v[i - 1].y == y && v[i - 1].x == x - span; };
+    // the vector at cell c, which is (x, y), or -1
+    auto at = [&](int c, int x, int y) {
+        const int j = cell[c];
+        return (j >= 0 && j < nv && v[j].x == x && v[j].y == y) ? j : -1;
+    };
+    // 1.
+    for (int i = i0, head = i0; i < i1; i++) {
+        const int x = v[i].x, y = v[i].y;
+        cell[(y / span) * nsx + x / span] = i;
+        if (!(i > i0 && has_w(i, x, y))) head = i;
+        par[i] = head;
+    }
+    __syncthreads();
+    // 2. the cells W, NW, N, NE come before i in scan order
+    for (int i = i0; i < i1; i++) {
+        const int x = v[i].x, y = v[i].y;
+        const bool w = has_w(i, x, y);
+        if (w && i == i0) uf_union(par, i, i - 1);
+        if (y == 0) continue;
+        const int cx = x / span, c = (y / span) * nsx + cx - nsx;
+        const int n = at(c, x, y - span), nw = cx > 0 ? at(c - 1, x - span, y - span) : -1;
+        if (n >= 0) {
+            if (!(w && nw >= 0)) uf_union(par, i, n);
+        } else {
+            if (nw >= 0 && !w) uf_union(par, i, nw);
+            const int ne = cx + 1 < nsx ? at(c + 1, x + span, y - span) : -1;
+            if (ne >= 0) uf_union(par, i, ne);
+        }
+    }
+    __syncthreads();
+    // 3.
+    int roots = 0;
+    for (int i = i0; i < i1; i++) {
+        const int r = uf_find(par, i);
+        par[i] = r;
+        roots += r == i;
+    }
+    int slot = block_exclusive_scan(roots, warp_sums, &total); // its barrier also ends the flattening
+    if (threadIdx.x == 0) a.n_regions[b] = total;
+    for (int i = i0; i < i1 && roots > 0; i++) {
+        if (par[i] != i) continue;
+        cell[i] = slot; // the map is not read any more: from here on it holds the slot of each root
+        if (slot < kMaxChangeRegions) {
+            DevChangeRegion &r = reg[slot];
+            r.x = 0x7fffffff; r.y = 0x7fffffff; r.w = -1; r.h = -1; r.n = 0;
+            *reinterpret_cast<unsigned long long *>(&r.peak.dx) = 0ull;
+        }
+        slot++;
+        roots--;
+    }
+    __syncthreads();
+    // 4.
+    int cur = -1, x0 = 0, y0 = 0, x1 = 0, y1 = 0, n = 0;
+    unsigned long long key = 0;
+    for (int i = i0; i < i1; i++) {
+        const int s = cell[par[i]];
+        if (s >= kMaxChangeRegions) continue;
+        if (s != cur) {
+            if (cur >= 0) fold_region(reg + cur, x0, y0, x1, y1, n, key);
+            cur = s; x0 = 0x7fffffff; y0 = 0x7fffffff; x1 = -1; y1 = -1; n = 0; key = 0;
+        }
+        const DevVector p = v[i];
+        const float dx = (float)p.dx, dy = (float)p.dy;
+        const float len = (dx * dx) + (dy * dy); // the sample kernel's len (this unit is built with -fmad=false)
+        x0 = min(x0, p.x); y0 = min(y0, p.y); x1 = max(x1, p.x); y1 = max(y1, p.y); n++;
+        const unsigned long long k = ((unsigned long long)__float_as_uint(len) << 32) | (unsigned)~i;
+        key = k > key ? k : key;
+    }
+    if (cur >= 0) fold_region(reg + cur, x0, y0, x1, y1, n, key);
+    __syncthreads();
+    // 5.
+    for (int s = threadIdx.x; s < min(total, kMaxChangeRegions); s += blockDim.x) {
+        DevChangeRegion &r = reg[s];
+        const int rx = __ldcg(&r.x), ry = __ldcg(&r.y), mx = __ldcg(&r.w), my = __ldcg(&r.h);
+        const unsigned long long k = __ldcg(reinterpret_cast<const unsigned long long *>(&r.peak.dx));
+        r.w = min(mx + span, a.w) - rx;
+        r.h = min(my + span, a.h) - ry;
+        r.pad = 0;
+        r.peak = v[~(unsigned)k];
+    }
+}
+
+cudaError_t launch_change_regions(cudaStream_t s, const ChangeRegionArgs &a)
+{
+    change_regions_kernel<<<a.batch, 1024, 0, s>>>(a);
     return cudaGetLastError();
 }
 

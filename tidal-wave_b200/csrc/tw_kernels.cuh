@@ -188,4 +188,21 @@ cudaError_t launch_mask_paint(cudaStream_t s, uint8_t *src, const IgnoreMasks &k
 // arguments as launch_sample_ignore.
 cudaError_t launch_sample_mask(cudaStream_t s, const SampleArgs &a, const IgnoreRegions &g, const IgnoreMasks &k);
 
+// Change regions (tw_change_regions): the 8-connected components of each pair's sample points that yielded a vector, read from the
+// compact vector list the sample kernel wrote (never from the flow).  Regions are stored in the order of their first vector; at
+// most kMaxChangeRegions per pair, n_regions[b] is the full count.  One CTA per pair.
+constexpr int kMaxChangeRegions = 1024; // TW_MAX_CHANGE_REGIONS
+struct ChangeRegionArgs {
+    const void *vectors; // [B][cap] tw_vector, as SampleArgs::vectors
+    const int *counts;   // [B] vectors per pair (after the sample kernel)
+    int cap;
+    int w, h, span;      // frame (expected-image pixels) and sample spacing
+    int *scratch;        // [B][2][cap] int: cell -> vector index map (never cleared: entries are checked against the vectors), then
+                         // union-find parents
+    int *n_regions;      // [B]
+    void *regions;       // [B][kMaxChangeRegions] tw_change_region
+    int batch;
+};
+cudaError_t launch_change_regions(cudaStream_t s, const ChangeRegionArgs &a);
+
 } // namespace tw

@@ -49,6 +49,8 @@ struct Slot {
     bool done = false, dropped = false;
     tw_result res{};
     std::vector<tw_vector> vectors;
+    std::vector<tw_change_region> regions; // the first TW_MAX_CHANGE_REGIONS of n_regions (pools with change regions)
+    int n_regions = 0;
 };
 
 } // namespace
@@ -67,6 +69,7 @@ struct tw_pool {
     std::condition_variable cv_file;
     int decoding = 0;                     // jobs a decoder thread is working on
     int n_decoders = 0;                   // 0: one per host core (at most 32)
+    bool change_regions = false;          // fixed by the first submit (tw_pool_set_change_regions)
     std::unordered_map<long long, Slot> slots;
     bool running = true;
     long long next_id = 0;
@@ -94,12 +97,17 @@ void fill_error(tw_result *r, int code, const char *msg)
     snprintf(r->reason, sizeof r->reason, "%s", msg);
 }
 
-void publish(tw_pool *p, long long id, const tw_result &res, const tw_vector *vec, int nvec)
+void publish(tw_pool *p, long long id, const tw_result &res, const tw_vector *vec, int nvec, const tw_change_region *reg = nullptr,
+             int n_regions = 0)
 {
     std::lock_guard<std::mutex> lk(p->mu);
     Slot &s = p->slots[id];
     s.res = res;
     if (nvec > 0) s.vectors.assign(vec, vec + nvec);
+    if (reg && n_regions > 0) {
+        s.n_regions = n_regions;
+        s.regions.assign(reg, reg + std::min(n_regions, TW_MAX_CHANGE_REGIONS));
+    }
     s.done = true;
     if (res.status == TW_STATUS_ERROR) p->error_count++; else p->data_count++; // Manager::notify, src/manager.cpp:109-114
 }
@@ -272,6 +280,15 @@ void consumer_main(tw_pool *p, int idx)
     std::vector<const tw_rect *> ig(p->batch);
     std::vector<int> nig(p->batch);
     std::vector<const uint8_t *> mk(p->batch);
+    // change regions: the pool's setting is fixed once a request exists, so it is applied before this consumer's first batch
+    bool regions = false, regions_set = false;
+    std::vector<tw_change_region> reg(TW_MAX_CHANGE_REGIONS);
+    // publishes pair i of the batch the context answered last, with its change regions
+    auto publish_pair = [&](long long id, int i, const tw_result &r, const tw_vector *v, int nv) {
+        int nreg = 0;
+        if (regions && tw_change_regions(ctx, i, reg.data(), TW_MAX_CHANGE_REGIONS, &nreg) != TW_OK) nreg = 0;
+        publish(p, id, r, v, nv, reg.data(), nreg);
+    };
     // Up to two batches are in flight on the context (tw_pipe_*): while batch k runs, this thread pops and uploads batch k + 1
     // and then collects batch k - 1 -- one consumer thread per GPU keeps the device busy (src/consumer.cpp:18-24).
     struct InFlight { std::vector<Request> work; int cap = 0; };
@@ -282,7 +299,7 @@ void consumer_main(tw_pool *p, int idx)
         const int n = (int)f.work.size();
         if (vec.size() < (size_t)n * f.cap) vec.resize((size_t)n * f.cap);
         tw_pipe_collect(ctx, vec.data(), f.cap, res.data());
-        for (int i = 0; i < n; i++) publish(p, f.work[i].id, res[i], vec.data() + (size_t)i * f.cap, std::min(res[i].n_vectors, f.cap));
+        for (int i = 0; i < n; i++) publish_pair(f.work[i].id, i, res[i], vec.data() + (size_t)i * f.cap, std::min(res[i].n_vectors, f.cap));
         p->cv_res.notify_all();
     };
     for (;;) {
@@ -327,6 +344,14 @@ void consumer_main(tw_pool *p, int idx)
             p->cv_res.notify_all();
             continue;
         }
+        if (!regions_set) {
+            {
+                std::lock_guard<std::mutex> lk(p->mu);
+                regions = p->change_regions;
+            }
+            tw_set_option(ctx, "change_regions", regions ? 1 : 0); // nothing in flight yet
+            regions_set = true;
+        }
         int cap = p->vector_cap;
         if (cap <= 0) cap = std::max(1, ((work[0].ew + p->span - 1) / p->span) * ((work[0].eh + p->span - 1) / p->span));
         const Request &r0 = work[0];
@@ -337,7 +362,7 @@ void consumer_main(tw_pool *p, int idx)
             if (vec.size() < (size_t)cap) vec.resize(cap);
             tw_compare_mask(ctx, r0.expect, r0.ew, r0.eh, r0.target, r0.tw, r0.th, &p->param, p->threshold, p->span, r0.ignore.data(),
                             (int)r0.ignore.size(), r0.mask, vec.data(), cap, &res[0]);
-            publish(p, r0.id, res[0], vec.data(), std::min(res[0].n_vectors, cap));
+            publish_pair(r0.id, 0, res[0], vec.data(), std::min(res[0].n_vectors, cap));
             p->cv_res.notify_all();
             continue;
         }
@@ -371,13 +396,17 @@ void consumer_main(tw_pool *p, int idx)
     if (ctx) tw_destroy(ctx);
 }
 
-int take(tw_pool *p, std::unordered_map<long long, Slot>::iterator it, tw_vector *out, int cap, tw_result *res)
+int take(tw_pool *p, std::unordered_map<long long, Slot>::iterator it, tw_vector *out, int cap, tw_result *res,
+         tw_change_region *regions = nullptr, int region_cap = 0, int *n_regions = nullptr)
 {
     Slot &s = it->second;
     if (s.dropped) { p->slots.erase(it); return -1; }
     if (res) *res = s.res;
     int n = std::min<int>((int)s.vectors.size(), cap);
     if (out && n > 0) memcpy(out, s.vectors.data(), sizeof(tw_vector) * n);
+    const int k = std::min<int>((int)s.regions.size(), region_cap);
+    if (regions && k > 0) memcpy(regions, s.regions.data(), sizeof(tw_change_region) * k);
+    if (n_regions) *n_regions = s.n_regions;
     int code = s.res.code;
     p->slots.erase(it);
     return code;
@@ -489,7 +518,17 @@ int tw_pool_set_decoders(tw_pool *p, int n)
     return TW_OK;
 }
 
-int tw_pool_wait(tw_pool *p, long long id, tw_vector *out, int cap, tw_result *res)
+int tw_pool_set_change_regions(tw_pool *p, int on)
+{
+    if (!p) return TW_BAD_PARAMETER;
+    std::lock_guard<std::mutex> lk(p->mu);
+    if (p->next_id > 0) return TW_BAD_PARAMETER; // a consumer may already run with the old setting
+    p->change_regions = on != 0;
+    return TW_OK;
+}
+
+int tw_pool_wait_regions(tw_pool *p, long long id, tw_vector *out, int cap, tw_result *res, tw_change_region *regions, int region_cap,
+                         int *n_regions)
 {
     if (!p) return -1;
     std::unique_lock<std::mutex> lk(p->mu);
@@ -497,7 +536,12 @@ int tw_pool_wait(tw_pool *p, long long id, tw_vector *out, int cap, tw_result *r
     if (it == p->slots.end()) return -1;
     p->cv_res.wait(lk, [&] { it = p->slots.find(id); return it == p->slots.end() || it->second.done || it->second.dropped; });
     if (it == p->slots.end()) return -1;
-    return take(p, it, out, cap, res);
+    return take(p, it, out, cap, res, regions, region_cap, n_regions);
+}
+
+int tw_pool_wait(tw_pool *p, long long id, tw_vector *out, int cap, tw_result *res)
+{
+    return tw_pool_wait_regions(p, id, out, cap, res, nullptr, 0, nullptr);
 }
 
 // Blocks until request `id` is answered and copies its tw_result WITHOUT taking it: res->n_vectors tells the caller how many

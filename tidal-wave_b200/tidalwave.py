@@ -11,7 +11,9 @@ nonzero = ignore, the expected image's size; tw_compare_mask) come from ``ignore
 short path as the target; a pair with no file there has no mask) or, if that is not a string, from ``getIgnoreMaskPath(shortPath)``
 (a callable returning a mask path, or something falsy for none).  A pair's mask and regions are ignored together; a mask file that
 cannot be decoded, or of another size than the expected image, makes that pair an 'error' event.  Wrong-typed values of these
-options mean "no mask", as for the reference's options.  Files are decoded with ``imread_gray`` (PNG / JPEG / PGM,
+options mean "no mask", as for the reference's options.  ``changeRegions`` (only ``True`` turns it on) adds ``regions`` and
+``n_regions`` to every 'data' event: where the page changed, as connected groups of its suspicious sample points
+(include/tidalwave_b200.h, tw_change_regions).  Files are decoded with ``imread_gray`` (PNG / JPEG / PGM,
 bit-exact to cv::imread IMREAD_GRAYSCALE); a file that cannot be decoded becomes the reference's "Can't open <path>" error.
 """
 from __future__ import annotations
@@ -48,6 +50,7 @@ class TidalWave:
         self.getIgnoreRegions = o.get("getIgnoreRegions") if callable(o.get("getIgnoreRegions")) else None
         self.ignoreMaskDir = o.get("ignoreMaskDir") if isinstance(o.get("ignoreMaskDir"), str) else None
         self.getIgnoreMaskPath = o.get("getIgnoreMaskPath") if callable(o.get("getIgnoreMaskPath")) else None
+        self.changeRegions = o.get("changeRegions") is True
         self._handlers = {"data": [], "error": [], "finish": []}
         self._pending = []   # (request id | None, expect path, target path, immediate error | None)
         self._report = {"request": 0, "data": 0, "error": 0}
@@ -72,7 +75,8 @@ class TidalWave:
             ndev = max(1, load().tw_device_count())
             devices = self._devices or [i % ndev for i in range(max(1, self.numThreads))]  # consumer i <-> GPU i % count
             # screenshot directories mix page sizes: no size bound, and every vector of every pair comes back whatever its size
-            self._pool = Pool(devices, self.param, self.threshold, self.span, max_w=0, max_h=0, batch=self._batch, vector_cap=0)
+            self._pool = Pool(devices, self.param, self.threshold, self.span, max_w=0, max_h=0, batch=self._batch, vector_cap=0,
+                              change_regions=self.changeRegions)
             load().tw_pool_set_decoders(self._pool.pool, max(1, self.numThreads))
         return self._pool
 
