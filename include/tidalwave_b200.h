@@ -225,6 +225,37 @@ typedef struct tw_change_region {
  * out of range.  Set the option with tw_set_option(ctx, "change_regions", 1); it is refused while pipe batches are pending. */
 int tw_change_regions(tw_ctx *ctx, int pair, tw_change_region *out, int cap, int *n_regions);
 
+/* ---- intensity cells: where a page's pixels changed without moving, per span cell (option "intensity_threshold" = t) ----
+ * The flow only sees structure that moves: a block darkened in place, a button re-coloured or a label erased leaves it at 0 and
+ * the pair OK.  With t in 1 .. 255 gray levels, every run with span > 0 also tests each span cell for a change in place:
+ *   cells      cell (i, j) has its sample point at (x, y) = (i * span, j * span) and covers [x, min(x + span, W)) x
+ *              [y, min(y + span, H)) in EXPECTED-image pixels: the grid and cells of change regions.  E is the expected image,
+ *              T the target after the +-5 px resize and after ignore painting -- the pair the flow was computed on;
+ *   shift      (dx, dy) is the float flow at the cell's sample point (the value the classification reads);
+ *              sx = rint(clamp(dx, -W, W)), sy = rint(clamp(dy, -H, H)), rounding half to even; a non-finite component is 0;
+ *   residual   for a pixel p = (px, py) of the cell, r(p) = min over u, v in {-1, 0, 1} of
+ *              |E(p) - T(clamp(px + sx + u, 0, W - 1), clamp(py + sy + v, 0, H - 1))|, an integer: the integer shift absorbs the
+ *              motion the flow found, the 3 x 3 minimum its sub-pixel remainder and anti-aliasing;
+ *   test       n = the cell's pixels not ignored (under no ignore region and no nonzero mask byte), S = the sum of r over them.
+ *              The cell is an intensity cell when n > 0 and S > t * n (strict, as the vector rule).  Integer arithmetic
+ *              throughout: exact and order-free.
+ * A pair with at least one intensity cell is SUSPICIOUS even with 0 vectors; n_vectors, the vectors and the change regions do not
+ * change (regions describe vectors only).  ERROR pairs and runs with span <= 0 have 0 cells.  n_cells is always the full count;
+ * the first TW_MAX_INTENSITY_CELLS in row-major scan order are stored.  The output is a function of (E, T, the flow at the sample
+ * points, the ignored set) alone: eager runs and graph replays, the dense and sparse last iteration and the tile and strip window
+ * kernels (which write bit-identical sample-point flows) give identical bytes. */
+#define TW_MAX_INTENSITY_CELLS 4096
+typedef struct tw_intensity_cell {
+    int x, y;       /* the cell's sample point, expected-image pixels */
+    int n_pixels;   /* n */
+    int residual;   /* S (the mean residual is S / n); saturates at INT_MAX, which only a cell of more than 8 421 504 pixels reaches */
+} tw_intensity_cell;
+
+/* The intensity cells of pair `pair` of the batch that the last tw_compare*, tw_batch_fetch or tw_pipe_collect answered (copied to
+ * the host when "intensity_threshold" was on for that batch): min(cap, n_cells, TW_MAX_INTENSITY_CELLS) entries to out (out may be
+ * NULL when cap is 0), the full count to *n_cells.  TW_BAD_PARAMETER if that batch ran without the option or pair is out of range. */
+int tw_intensity_cells(tw_ctx *ctx, int pair, tw_intensity_cell *out, int cap, int *n_cells);
+
 /* ---- split phases of tw_compare_batch (same stream; used by the dispatcher to overlap, and by the
  * benchmark to time the device-resident pass separately from the PCIe legs).  They take no ignore regions and no ignore masks:
  * painting changes the resident target, so only the whole-call entry points above apply them.  tw_batch_flow after a run with
@@ -271,7 +302,10 @@ const char *tw_last_error(tw_ctx *ctx);
  *                     options) that the parity tests force.
  *   "change_regions" = 1: each run with span > 0 also groups every pair's vectors into change regions on the device (one more
  *                     launch, after the sample kernel; tw_change_regions reads them).  Default 0.  TW_BAD_PARAMETER while pipe
- *                     batches are pending. */
+ *                     batches are pending.
+ *   "intensity_threshold" = t: 0 (default) off; 1 .. 255: each run with span > 0 also finds every pair's intensity cells (three more
+ *                     launches after the sample kernel; tw_intensity_cells reads them) and counts them toward the status.  Any
+ *                     other value, or a change while pipe batches are pending, answers TW_BAD_PARAMETER. */
 int tw_set_option(tw_ctx *ctx, const char *name, int value);
 /* Process-wide default of "arithmetic" for contexts created afterwards (the dispatcher's consumers included). */
 int tw_set_default_arithmetic(int relaxed);
@@ -341,12 +375,19 @@ int tw_pool_set_decoders(tw_pool *pool, int n);
 /* on = 1: every consumer runs with "change_regions" and keeps each request's regions (tw_pool_wait_regions), whatever vector_cap
  * is.  Valid before the first submit (TW_OK), TW_BAD_PARAMETER after. */
 int tw_pool_set_change_regions(tw_pool *pool, int on);
+/* t = 1 .. 255: every consumer runs with "intensity_threshold" = t and keeps each request's intensity cells
+ * (tw_pool_wait_intensity); 0: off.  Valid before the first submit (TW_OK); TW_BAD_PARAMETER after, and for t outside 0 .. 255. */
+int tw_pool_set_intensity(tw_pool *pool, int t);
 /* Blocks until request `id` is answered; copies up to cap vectors.  Returns res->code, or <0 if dropped. */
 int tw_pool_wait(tw_pool *pool, long long id, tw_vector *out, int cap, tw_result *res);
 /* tw_pool_wait plus the request's change regions: up to region_cap of them to regions, the full count to *n_regions (0 for an
  * ERROR request and for a pool without change regions). */
 int tw_pool_wait_regions(tw_pool *pool, long long id, tw_vector *out, int cap, tw_result *res, tw_change_region *regions,
                          int region_cap, int *n_regions);
+/* tw_pool_wait_regions plus the request's intensity cells: up to cell_cap of them to cells, the full count to *n_cells (0 for an
+ * ERROR request and for a pool without the option).  regions / n_regions may be NULL and region_cap 0. */
+int tw_pool_wait_intensity(tw_pool *pool, long long id, tw_vector *out, int cap, tw_result *res, tw_change_region *regions,
+                           int region_cap, int *n_regions, tw_intensity_cell *cells, int cell_cap, int *n_cells);
 /* Blocks until request `id` is answered and copies its result WITHOUT taking it (res->n_vectors = the room tw_pool_wait needs).
  * Returns res->code, or <0 if dropped / unknown. */
 int tw_pool_peek(tw_pool *pool, long long id, tw_result *res);

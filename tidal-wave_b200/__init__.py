@@ -9,5 +9,6 @@ operator interface), synth.py (seeded synthetic screenshot pairs).
 """
 from . import dist, synth, tidalwave  # noqa: F401
 from .tidalwave import TidalWave, create, run  # noqa: F401
-from .api import (LIB_PATH, MAX_CHANGE_REGIONS, MAX_IGNORE, imread_gray, OpticalFlow, OpticalFlowParameter, Pool, declared_symbols, load,  # noqa: F401
-                  set_default_arithmetic, tw_change_region, tw_flow_param, tw_rect, tw_result, tw_vector)
+from .api import (LIB_PATH, MAX_CHANGE_REGIONS, MAX_IGNORE, MAX_INTENSITY_CELLS, imread_gray, OpticalFlow, OpticalFlowParameter, Pool,  # noqa: F401
+                  declared_symbols, load, set_default_arithmetic, tw_change_region, tw_flow_param, tw_intensity_cell, tw_rect, tw_result,
+                  tw_vector)

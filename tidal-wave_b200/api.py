@@ -25,6 +25,7 @@ OK, BAD_PARAMETER, BAD_IMAGE_FORMAT, DONT_MATCH_SIZE, CUDA_ERROR, UNSUPPORTED = 
 STATUS_NAMES = {0: "OK", 1: "SUSPICIOUS", 2: "ERROR"}
 MAX_IGNORE = 32  # TW_MAX_IGNORE: ignore regions per pair
 MAX_CHANGE_REGIONS = 1024  # TW_MAX_CHANGE_REGIONS: change regions stored per pair
+MAX_INTENSITY_CELLS = 4096  # TW_MAX_INTENSITY_CELLS: intensity cells stored per pair
 
 
 class tw_flow_param(C.Structure):
@@ -50,6 +51,16 @@ class tw_change_region(C.Structure):
     """A change region: the bounding box of a connected group of suspicious sample points (expected-image pixels), their count
     and the vector with the largest length among them (include/tidalwave_b200.h, tw_change_regions)."""
     _fields_ = [("rect", tw_rect), ("n_vectors", C.c_int), ("peak", tw_vector)]
+
+
+class tw_intensity_cell(C.Structure):
+    """An intensity cell: a span cell whose pixels changed where the flow found no motion -- its sample point, its n pixels that
+    are not ignored and the sum S of their residuals (include/tidalwave_b200.h, tw_intensity_cells)."""
+    _fields_ = [("x", C.c_int), ("y", C.c_int), ("n_pixels", C.c_int), ("residual", C.c_int)]
+
+
+def _cell_dicts(cells, n) -> list[dict]:
+    return [{"x": c.x, "y": c.y, "n_pixels": c.n_pixels, "residual": c.residual} for c in cells[:n]]
 
 
 def _region_dicts(regs, n) -> list[dict]:
@@ -162,6 +173,7 @@ def load() -> C.CDLL:
     L.tw_pipe_submit_mask.argtypes = [C.c_void_p, C.c_int, u8pp, u8pp, C.c_int, C.c_int, C.c_int, C.POINTER(tw_flow_param),
                                       C.c_double, C.c_int, rpp, C.POINTER(C.c_int), u8pp]
     L.tw_change_regions.argtypes = [C.c_void_p, C.c_int, C.POINTER(tw_change_region), C.c_int, C.POINTER(C.c_int)]
+    L.tw_intensity_cells.argtypes = [C.c_void_p, C.c_int, C.POINTER(tw_intensity_cell), C.c_int, C.POINTER(C.c_int)]
     L.tw_pipe_collect.argtypes = [C.c_void_p, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
     L.tw_pipe_pending.argtypes = [C.c_void_p]
     L.tw_pipe_ready.argtypes = [C.c_void_p]
@@ -212,6 +224,10 @@ def load() -> C.CDLL:
     L.tw_pool_set_change_regions.argtypes = [C.c_void_p, C.c_int]
     L.tw_pool_wait_regions.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result),
                                        C.POINTER(tw_change_region), C.c_int, C.POINTER(C.c_int)]
+    L.tw_pool_set_intensity.argtypes = [C.c_void_p, C.c_int]
+    L.tw_pool_wait_intensity.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result),
+                                         C.POINTER(tw_change_region), C.c_int, C.POINTER(C.c_int), C.POINTER(tw_intensity_cell),
+                                         C.c_int, C.POINTER(C.c_int)]
     L.tw_pool_poll.argtypes = [C.c_void_p, C.c_longlong, C.POINTER(tw_vector), C.c_int, C.POINTER(tw_result)]
     L.tw_pool_report.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
     L.tw_pool_stop.argtypes = [C.c_void_p]
@@ -280,6 +296,7 @@ class OpticalFlow:
             raise RuntimeError("tw_create failed: " + err.value.decode())
         self.max_batch = max_batch
         self.change_regions = False  # set_option("change_regions", 1): responses carry "regions" and "n_regions"
+        self.intensity = 0  # set_option("intensity_threshold", t > 0): responses carry "intensity_cells" and "n_intensity_cells"
 
     def close(self):
         if getattr(self, "ctx", None):
@@ -293,6 +310,8 @@ class OpticalFlow:
             raise ValueError(self.last_error())
         if name == "change_regions":
             self.change_regions = bool(value)
+        if name == "intensity_threshold":
+            self.intensity = int(value)
 
     def regions(self, pair: int = 0):
         """(regions as dicts, n_regions) of pair ``pair`` of the last answered batch (tw_change_regions); raises ValueError if that
@@ -303,9 +322,20 @@ class OpticalFlow:
             raise ValueError(self.last_error())
         return _region_dicts(regs, min(n.value, MAX_CHANGE_REGIONS)), n.value
 
+    def intensity_cells(self, pair: int = 0):
+        """(intensity cells as dicts, n_cells) of pair ``pair`` of the last answered batch (tw_intensity_cells); raises ValueError if
+        that batch ran without the "intensity_threshold" option."""
+        cells = (tw_intensity_cell * MAX_INTENSITY_CELLS)()
+        n = C.c_int()
+        if self.lib.tw_intensity_cells(self.ctx, pair, cells, MAX_INTENSITY_CELLS, C.byref(n)) != 0:
+            raise ValueError(self.last_error())
+        return _cell_dicts(cells, min(n.value, MAX_INTENSITY_CELLS)), n.value
+
     def _with_regions(self, resp: dict, pair: int) -> dict:
         if self.change_regions and resp["status"] != "ERROR":
             resp["regions"], resp["n_regions"] = self.regions(pair)
+        if self.intensity and resp["status"] != "ERROR":
+            resp["intensity_cells"], resp["n_intensity_cells"] = self.intensity_cells(pair)
         return resp
 
     def last_error(self) -> str:
@@ -440,10 +470,12 @@ class Pool:
     """Manager + Consumer pool (src/manager.cpp:40-98): one consumer thread per entry of ``devices``."""
 
     def __init__(self, devices, param: OpticalFlowParameter = OpticalFlowParameter(), threshold: float = 5.0, span: int = 10,
-                 max_w: int = 0, max_h: int = 0, batch: int = 1, vector_cap: int = 0, change_regions: bool = False):
+                 max_w: int = 0, max_h: int = 0, batch: int = 1, vector_cap: int = 0, change_regions: bool = False,
+                 intensity_threshold: int = 0):
         """max_w / max_h = 0: no bound on the image size; vector_cap = 0: every vector of every request is returned (the capacity
         follows each request's own sampling grid), > 0: at most that many (``n_vectors`` still holds the full count).
-        change_regions: wait() answers also carry "regions" and "n_regions" (tw_pool_set_change_regions), whatever vector_cap is."""
+        change_regions: wait() answers also carry "regions" and "n_regions" (tw_pool_set_change_regions), whatever vector_cap is.
+        intensity_threshold: t in 1 .. 255 gray levels adds "intensity_cells" and "n_intensity_cells" (tw_pool_set_intensity); 0 off."""
         self.lib = load()
         self.span, self.threshold, self.cap = span, threshold, vector_cap
         err = C.create_string_buffer(256)
@@ -458,6 +490,11 @@ class Pool:
             if self.lib.tw_pool_set_change_regions(self.pool, 1) != OK:
                 self.close()
                 raise RuntimeError("tw_pool_set_change_regions refused: the pool has taken requests already")
+        self.intensity = int(intensity_threshold)
+        if self.intensity:
+            if self.lib.tw_pool_set_intensity(self.pool, self.intensity) != OK:
+                self.close()
+                raise ValueError(f"tw_pool_set_intensity refused {intensity_threshold!r}: 0 (off) or 1 .. 255 gray levels")
         self._keep = {}
 
     def request(self, expectImg, targetImg, ignore=None, ignore_mask=None) -> int:
@@ -513,18 +550,28 @@ class Pool:
                 cap = max(1, info.n_vectors)
         vec = (tw_vector * cap)()
         res = tw_result()
-        if not self.change_regions:
+        if not self.change_regions and not self.intensity:
             rc = self.lib.tw_pool_wait(self.pool, rid, vec, cap, C.byref(res))
-        else:
+        elif not self.intensity:
             regs = (tw_change_region * MAX_CHANGE_REGIONS)()
             nreg = C.c_int()
             rc = self.lib.tw_pool_wait_regions(self.pool, rid, vec, cap, C.byref(res), regs, MAX_CHANGE_REGIONS, C.byref(nreg))
+        else:
+            regs = (tw_change_region * MAX_CHANGE_REGIONS)() if self.change_regions else None
+            nreg = C.c_int()
+            cells = (tw_intensity_cell * MAX_INTENSITY_CELLS)()
+            ncell = C.c_int()
+            rc = self.lib.tw_pool_wait_intensity(self.pool, rid, vec, cap, C.byref(res), regs,
+                                                 MAX_CHANGE_REGIONS if self.change_regions else 0, C.byref(nreg), cells,
+                                                 MAX_INTENSITY_CELLS, C.byref(ncell))
         self._keep.pop(rid, None)
         if rc < 0:
             return None
         resp = _response(res, vec, min(res.n_vectors, cap), self.span, self.threshold)
         if self.change_regions and resp["status"] != "ERROR":
             resp["regions"], resp["n_regions"] = _region_dicts(regs, min(nreg.value, MAX_CHANGE_REGIONS)), nreg.value
+        if self.intensity and resp["status"] != "ERROR":
+            resp["intensity_cells"], resp["n_intensity_cells"] = _cell_dicts(cells, min(ncell.value, MAX_INTENSITY_CELLS)), ncell.value
         return resp
 
     def report(self) -> dict:

@@ -19,10 +19,10 @@ using namespace tw;
 
 namespace {
 
-enum Family { F_LEVEL = 0, F_POLY, F_FIRST, F_GITER, F_GLAST, F_BVSUM, F_BITER, F_BLAST, F_BUPD, F_SAMPLE, F_PAINT, F_MASK, F_REGIONS, F_COUNT };
+enum Family { F_LEVEL = 0, F_POLY, F_FIRST, F_GITER, F_GLAST, F_BVSUM, F_BITER, F_BLAST, F_BUPD, F_SAMPLE, F_PAINT, F_MASK, F_REGIONS, F_INTENSITY, F_COUNT };
 const char *kFamilyNames[F_COUNT] = {"level_image", "polyexp", "first_update", "gauss_iter", "gauss_last",
                                      "box_vsum", "box_hscan", "box_hscan_last", "box_update", "sample", "ignore_paint",
-                                     "mask_paint", "change_regions"};
+                                     "mask_paint", "change_regions", "intensity"};
 
 struct Scale {
     int k, ksize;
@@ -50,10 +50,12 @@ struct LaunchOptions {
     int box_unfused = 0;  // 1: the three-launch box iteration (V plane through HBM), kept for the parity tests
     int level_generic = 0, level_unfused = 0;
     int change_regions = 0; // 1: the change-region kernel runs after the sample kernel
+    int intensity = 0;      // "intensity_threshold" t (1 .. 255): the intensity-cell kernels run after the sample kernel; 0: off
     bool operator==(const LaunchOptions &o) const
     {
         return arith == o.arith && sparse_last == o.sparse_last && window_tiles == o.window_tiles && box_unfused == o.box_unfused &&
-               level_generic == o.level_generic && level_unfused == o.level_unfused && change_regions == o.change_regions;
+               level_generic == o.level_generic && level_unfused == o.level_unfused && change_regions == o.change_regions &&
+               intensity == o.intensity;
     }
 };
 
@@ -132,8 +134,19 @@ struct tw_ctx {
     int *d_nreg = nullptr, *h_nreg = nullptr;
     tw_change_region *d_regions = nullptr, *h_regions = nullptr;
     int reg_pairs = -1; // pairs of the last answered batch whose regions the mirror holds; -1: that batch ran without the option
+    // intensity cells ("intensity_threshold"): per-cell totals [max_batch][int_cap] u64 S, then [max_batch][int_cap] u32 n, then
+    // [max_batch][int_chunks] per-chunk counts, sized with d_vectors like the region scratch; the cell counts [max_batch] and the
+    // cells [max_batch][kMaxIntensityCells] with their page-locked mirrors.  The totals are zero between runs (the compaction clears
+    // them); int_dirty: a run that launched the sums may not have reached the compaction, so they are cleared before the next one
+    void *d_int_acc = nullptr;
+    int int_cap = 0, int_chunks = 0;
+    bool int_dirty = false;
+    int *d_ncell = nullptr, *h_ncell = nullptr;
+    tw_intensity_cell *d_cells = nullptr, *h_cells = nullptr;
+    int cell_pairs = -1; // pairs of the last answered batch whose cells the mirror holds; -1: that batch ran without the option
     int last_n = 0, last_w = 0, last_h = 0, last_span = 0;
     bool last_regions = false; // the last run had "change_regions" on
+    bool last_intensity = false; // the last run had "intensity_threshold" on
     bool ran = false;
     // profiling
     bool profiling = false;
@@ -158,6 +171,10 @@ struct tw_ctx {
         bool regions = false;
         int *d_nreg = nullptr, *h_nreg = nullptr;
         tw_change_region *d_regions = nullptr;
+        // intensity cells of this batch (intensity: it ran with the option), snapshot likewise
+        bool intensity = false;
+        int *d_ncell = nullptr, *h_ncell = nullptr;
+        tw_intensity_cell *d_cells = nullptr;
     };
     struct Pipe {
         cudaStream_t copy = nullptr, fetch = nullptr;
@@ -647,6 +664,56 @@ void answer_regions(tw_ctx *ctx, int n, bool on)
     if (ctx->reg_pairs > 0) memset(ctx->h_nreg, 0, sizeof(int) * n);
 }
 
+static_assert(kMaxIntensityCells == TW_MAX_INTENSITY_CELLS && sizeof(tw_intensity_cell) == 16, "tw_intensity_cell as the kernel writes it");
+
+// The cell counts and cells of the context (tw_ctx::d_ncell, d_cells) and their page-locked mirrors: allocated on first use, at a
+// fixed size, and kept until the context goes.
+bool ensure_cell_mirrors(tw_ctx *ctx)
+{
+    if (ctx->h_cells) return true;
+    const size_t bytes = (size_t)ctx->max_batch * kMaxIntensityCells * sizeof(tw_intensity_cell);
+    CK(cudaMalloc(&ctx->d_ncell, sizeof(int) * ctx->max_batch));
+    CK(cudaMallocHost(&ctx->h_ncell, sizeof(int) * ctx->max_batch));
+    CK(cudaMalloc(&ctx->d_cells, bytes));
+    CK(cudaMallocHost(&ctx->h_cells, bytes));
+    return true;
+}
+
+size_t intensity_acc_bytes(const tw_ctx *ctx)
+{
+    return (size_t)ctx->max_batch * ((size_t)ctx->int_cap * (sizeof(unsigned long long) + sizeof(unsigned)) + ctx->int_chunks * sizeof(int));
+}
+
+// Those and the per-cell totals, for dev_cap (>= the cells of the grid, one vector per sample point).  Like the region scratch, the
+// totals are reallocated only when dev_cap changes, which changes the graph key as well; they are cleared when allocated and
+// after a run that may have left them set.
+bool ensure_intensity_buffers(tw_ctx *ctx)
+{
+    if (!ensure_cell_mirrors(ctx)) return false;
+    if (!ctx->d_int_acc || ctx->int_cap != ctx->dev_cap) {
+        CK(cudaStreamSynchronize(ctx->stream));
+        if (ctx->d_int_acc) cudaFree(ctx->d_int_acc);
+        ctx->d_int_acc = nullptr;
+        ctx->int_cap = ctx->dev_cap;
+        ctx->int_chunks = (ctx->dev_cap + kIntChunk - 1) / kIntChunk;
+        CK(cudaMalloc(&ctx->d_int_acc, intensity_acc_bytes(ctx)));
+        ctx->int_dirty = true;
+    }
+    if (ctx->int_dirty) {
+        CK(cudaMemsetAsync(ctx->d_int_acc, 0, intensity_acc_bytes(ctx), ctx->stream));
+        ctx->int_dirty = false;
+    }
+    return true;
+}
+
+// The host mirror now answers for a batch of n pairs: with 0 cells each if `on`, else for no pair (tw_intensity_cells refuses).
+void answer_cells(tw_ctx *ctx, int n, bool on)
+{
+    n = std::max(0, std::min(n, ctx->max_batch));
+    ctx->cell_pairs = on && ensure_cell_mirrors(ctx) ? n : -1;
+    if (ctx->cell_pairs > 0) memset(ctx->h_ncell, 0, sizeof(int) * n);
+}
+
 // Region buffer (tw_ctx::d_ignore, h_ignore, the pipe's staging tail): [max_batch][kMaxIgnore] int4, then [max_batch] int.
 size_t ignore_bytes(int max_batch) { return (size_t)max_batch * (kMaxIgnore * sizeof(int4) + sizeof(int)); }
 
@@ -839,6 +906,23 @@ bool enqueue(tw_ctx *ctx, int n, double threshold, int span, bool ignore, bool m
             ca.scratch = ctx->d_reg_scratch; ca.n_regions = ctx->d_nreg; ca.regions = ctx->d_regions; ca.batch = n;
             LAUNCH(F_REGIONS, 0.0, launch_change_regions(ctx->stream, ca));
         }
+        if (ctx->opt.intensity) {
+            if (!ensure_intensity_buffers(ctx)) return false;
+            IntensityArgs ta{};
+            ta.src = pl.src; ta.spitch = pl.spitch; ta.flow = f.flow; ta.d = f.d; ta.span = span; ta.t = ctx->opt.intensity;
+            if (ignore) ta.g = ignore_regions(ctx->d_ignore, ctx->max_batch);
+            if (mask) ta.k = ignore_masks(pl);
+            ta.sum = reinterpret_cast<unsigned long long *>(ctx->d_int_acc);
+            ta.cnt = reinterpret_cast<unsigned *>(ta.sum + (size_t)ctx->max_batch * ctx->int_cap);
+            ta.chunk_counts = reinterpret_cast<int *>(ta.cnt + (size_t)ctx->max_batch * ctx->int_cap);
+            ta.cell_cap = ctx->int_cap; ta.max_chunks = ctx->int_chunks; ta.n_cells = ctx->d_ncell; ta.cells = ctx->d_cells; ta.batch = n;
+            ctx->int_dirty = true;
+            // what the sums read: E and T once (the 3 x 3 target taps are staged in shared memory)
+            LAUNCH(F_INTENSITY, n * 2.0 * P0, launch_intensity_sum(ctx->stream, ta));
+            LAUNCH(F_INTENSITY, 0.0, launch_intensity_count(ctx->stream, ta));
+            LAUNCH(F_INTENSITY, 0.0, launch_intensity_compact(ctx->stream, ta));
+            ctx->int_dirty = false;
+        }
     }
     return true;
 }
@@ -1001,6 +1085,11 @@ void tw_destroy(tw_ctx *ctx)
     if (ctx->h_nreg) cudaFreeHost(ctx->h_nreg);
     if (ctx->d_regions) cudaFree(ctx->d_regions);
     if (ctx->h_regions) cudaFreeHost(ctx->h_regions);
+    if (ctx->d_int_acc) cudaFree(ctx->d_int_acc);
+    if (ctx->d_ncell) cudaFree(ctx->d_ncell);
+    if (ctx->h_ncell) cudaFreeHost(ctx->h_ncell);
+    if (ctx->d_cells) cudaFree(ctx->d_cells);
+    if (ctx->h_cells) cudaFreeHost(ctx->h_cells);
     if (ctx->flush_buf) cudaFree(ctx->flush_buf);
     if (ctx->rs_buf) cudaFree(ctx->rs_buf);
     {
@@ -1022,6 +1111,9 @@ void tw_destroy(tw_ctx *ctx)
             if (s.d_nreg) cudaFree(s.d_nreg);
             if (s.h_nreg) cudaFreeHost(s.h_nreg);
             if (s.d_regions) cudaFree(s.d_regions);
+            if (s.d_ncell) cudaFree(s.d_ncell);
+            if (s.h_ncell) cudaFreeHost(s.h_ncell);
+            if (s.d_cells) cudaFree(s.d_cells);
         }
     }
     if (ctx->ev_t0) cudaEventDestroy(ctx->ev_t0);
@@ -1179,7 +1271,7 @@ static int run_batch(tw_ctx *ctx, int n, int w, int h, const tw_flow_param *para
     if (!run_sequence(ctx, n, threshold, span, ignore, mask)) return TW_CUDA_ERROR;
     cudaEventRecord(ctx->ev_r1, ctx->stream);
     ctx->last_n = n; ctx->last_w = w; ctx->last_h = h; ctx->ran = true;
-    ctx->last_span = span; ctx->last_regions = ctx->opt.change_regions != 0;
+    ctx->last_span = span; ctx->last_regions = ctx->opt.change_regions != 0; ctx->last_intensity = ctx->opt.intensity != 0;
     ctx->last_sparse = sparse_in_effect(ctx, span);
     return TW_OK;
 }
@@ -1195,12 +1287,16 @@ int tw_batch_fetch(tw_ctx *ctx, int n, tw_vector *out, int cap, tw_result *res)
     if (!ctx->ran || n != ctx->last_n) { ctx->err = "tw_batch_fetch: nothing to fetch"; return TW_BAD_PARAMETER; }
     cudaSetDevice(ctx->device);
     answer_regions(ctx, n, ctx->last_regions);
+    answer_cells(ctx, n, ctx->last_intensity);
     const bool labelled = ctx->last_regions && ctx->last_span > 0;
+    const bool celled = ctx->last_intensity && ctx->last_span > 0 && ctx->cell_pairs >= 0;
     cudaError_t e = cudaMemcpyAsync(ctx->h_counts, ctx->d_counts, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && labelled) e = cudaMemcpyAsync(ctx->h_nreg, ctx->d_nreg, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && celled) e = cudaMemcpyAsync(ctx->h_ncell, ctx->d_ncell, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) {
         answer_regions(ctx, n, ctx->last_regions);
+        answer_cells(ctx, n, ctx->last_intensity);
         set_err(ctx, "fetch", e);
         for (int i = 0; i < n; i++) fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str());
         return TW_CUDA_ERROR;
@@ -1209,9 +1305,10 @@ int tw_batch_fetch(tw_ctx *ctx, int n, tw_vector *out, int cap, tw_result *res)
     cudaEventElapsedTime(&ms, ctx->ev_r0, ctx->ev_r1);
     for (int i = 0; i < n; i++) {
         int cnt = ctx->h_counts[i];
+        const int ncell = celled ? ctx->h_ncell[i] : 0;
         memset(&res[i], 0, sizeof(tw_result));
         res[i].code = TW_OK;
-        res[i].status = cnt == 0 ? TW_STATUS_OK : TW_STATUS_SUSPICIOUS;
+        res[i].status = cnt == 0 && ncell == 0 ? TW_STATUS_OK : TW_STATUS_SUSPICIOUS;
         res[i].n_vectors = cnt;
         res[i].width = ctx->last_w; res[i].height = ctx->last_h;
         res[i].time = ms * 1e-3f / n;
@@ -1227,7 +1324,14 @@ int tw_batch_fetch(tw_ctx *ctx, int n, tw_vector *out, int cap, tw_result *res)
                                 sizeof(tw_change_region) * nreg, cudaMemcpyDeviceToHost, ctx->stream);
             if (e != cudaSuccess) { set_err(ctx, "fetch regions", e); fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str()); }
         }
+        const int kcell = std::min(ncell, kMaxIntensityCells);
+        if (kcell > 0 && res[i].code == TW_OK) {
+            e = cudaMemcpyAsync(ctx->h_cells + (size_t)i * kMaxIntensityCells, ctx->d_cells + (size_t)i * kMaxIntensityCells,
+                                sizeof(tw_intensity_cell) * kcell, cudaMemcpyDeviceToHost, ctx->stream);
+            if (e != cudaSuccess) { set_err(ctx, "fetch intensity cells", e); fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str()); }
+        }
         if (res[i].code != TW_OK && ctx->reg_pairs > 0) ctx->h_nreg[i] = 0;
+        if (res[i].code != TW_OK && ctx->cell_pairs > 0) ctx->h_ncell[i] = 0;
     }
     e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) { set_err(ctx, "fetch sync", e); return TW_CUDA_ERROR; }
@@ -1277,6 +1381,7 @@ int tw_compare_batch_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, cons
 {
     if (!ctx || !res) return TW_BAD_PARAMETER;
     answer_regions(ctx, n, ctx->opt.change_regions != 0); // what an ERROR answer leaves: 0 regions per pair
+    answer_cells(ctx, n, ctx->opt.intensity != 0);        // and 0 intensity cells
     auto fail_all = [&](int code, const char *msg) {
         for (int i = 0; i < n; i++) fill_error(&res[i], code, msg);
         return code;
@@ -1410,7 +1515,7 @@ int tw_pipe_submit_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const 
     if (!run_sequence(ctx, n, threshold, span, any, any_mask)) return TW_CUDA_ERROR;
     cudaEventRecord(s.r1, ctx->stream);
     ctx->last_n = n; ctx->last_w = w; ctx->last_h = h; ctx->ran = true;
-    ctx->last_span = span; ctx->last_regions = ctx->opt.change_regions != 0;
+    ctx->last_span = span; ctx->last_regions = ctx->opt.change_regions != 0; ctx->last_intensity = ctx->opt.intensity != 0;
     ctx->last_sparse = sparse_in_effect(ctx, span);
     // snapshot of the compact results (counts + vectors), then the counts to the host
     const size_t vbytes = (size_t)n * ctx->dev_cap * sizeof(tw_vector);
@@ -1435,6 +1540,19 @@ int tw_pipe_submit_mask(tw_ctx *ctx, int n, const uint8_t *const *expect, const 
         if (e == cudaSuccess)
             e = cudaMemcpyAsync(s.d_regions, ctx->d_regions, sizeof(tw_change_region) * n * kMaxChangeRegions, cudaMemcpyDeviceToDevice, ctx->stream);
         if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_nreg, s.d_nreg, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
+    }
+    s.intensity = ctx->last_intensity;
+    if (e == cudaSuccess && s.intensity) { // the intensity cells likewise
+        if ((!s.d_ncell && (e = cudaMalloc(&s.d_ncell, sizeof(int) * ctx->max_batch)) != cudaSuccess) ||
+            (!s.h_ncell && (e = cudaMallocHost(&s.h_ncell, sizeof(int) * ctx->max_batch)) != cudaSuccess) ||
+            (!s.d_cells && (e = cudaMalloc(&s.d_cells, sizeof(tw_intensity_cell) * ctx->max_batch * kMaxIntensityCells)) != cudaSuccess)) {
+            set_err(ctx, "cudaMalloc snapshot", e);
+            return TW_CUDA_ERROR;
+        }
+        e = cudaMemcpyAsync(s.d_ncell, ctx->d_ncell, sizeof(int) * n, cudaMemcpyDeviceToDevice, ctx->stream);
+        if (e == cudaSuccess)
+            e = cudaMemcpyAsync(s.d_cells, ctx->d_cells, sizeof(tw_intensity_cell) * n * kMaxIntensityCells, cudaMemcpyDeviceToDevice, ctx->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_ncell, s.d_ncell, sizeof(int) * n, cudaMemcpyDeviceToHost, ctx->stream);
     }
     if (e != cudaSuccess) { set_err(ctx, "snapshot", e); return TW_CUDA_ERROR; }
     cudaEventRecord(s.done, ctx->stream);
@@ -1465,6 +1583,7 @@ int tw_pipe_collect(tw_ctx *ctx, tw_vector *out, int cap, tw_result *res)
     pp.head ^= 1; pp.count--;
     const int n = s.n;
     answer_regions(ctx, n, s.regions);
+    answer_cells(ctx, n, s.intensity);
     cudaError_t e = cudaEventSynchronize(s.done);
     if (e != cudaSuccess) {
         set_err(ctx, "collect", e);
@@ -1476,9 +1595,10 @@ int tw_pipe_collect(tw_ctx *ctx, tw_vector *out, int cap, tw_result *res)
     bool copied = false;
     for (int i = 0; i < n; i++) {
         const int cnt = s.h_counts[i];
+        const int ncell = s.intensity ? s.h_ncell[i] : 0;
         memset(&res[i], 0, sizeof(tw_result));
         res[i].code = TW_OK;
-        res[i].status = cnt == 0 ? TW_STATUS_OK : TW_STATUS_SUSPICIOUS;
+        res[i].status = cnt == 0 && ncell == 0 ? TW_STATUS_OK : TW_STATUS_SUSPICIOUS;
         res[i].n_vectors = cnt;
         res[i].width = s.w; res[i].height = s.h;
         res[i].time = ms * 1e-3f / n;
@@ -1497,6 +1617,14 @@ int tw_pipe_collect(tw_ctx *ctx, tw_vector *out, int cap, tw_result *res)
             copied = true;
         }
         if (s.regions) ctx->h_nreg[i] = res[i].code == TW_OK ? s.h_nreg[i] : 0;
+        const int kcell = std::min(ncell, kMaxIntensityCells);
+        if (kcell > 0 && res[i].code == TW_OK && ctx->cell_pairs > 0) {
+            e = cudaMemcpyAsync(ctx->h_cells + (size_t)i * kMaxIntensityCells, s.d_cells + (size_t)i * kMaxIntensityCells,
+                                sizeof(tw_intensity_cell) * kcell, cudaMemcpyDeviceToHost, pp.fetch);
+            if (e != cudaSuccess) { set_err(ctx, "collect intensity cells", e); fill_error(&res[i], TW_CUDA_ERROR, ctx->err.c_str()); }
+            copied = true;
+        }
+        if (ctx->cell_pairs > 0) ctx->h_ncell[i] = res[i].code == TW_OK ? ncell : 0;
     }
     if (copied && (e = cudaStreamSynchronize(pp.fetch)) != cudaSuccess) { set_err(ctx, "collect sync", e); return TW_CUDA_ERROR; }
     return TW_OK;
@@ -1509,6 +1637,7 @@ int tw_compare_mask(tw_ctx *ctx, const uint8_t *expect, int ew, int eh, const ui
     if (!res) return TW_BAD_PARAMETER;
     if (!ctx) { fill_error(res, TW_BAD_PARAMETER, "null context"); return res->code; }
     answer_regions(ctx, 1, ctx->opt.change_regions != 0); // what an ERROR answer leaves: 0 regions
+    answer_cells(ctx, 1, ctx->opt.intensity != 0);        // and 0 intensity cells
     // src/opticalflow.cpp:37-49: an image that cannot be opened is BadImageFormat
     if (!expect || ew < 1 || eh < 1) { fill_error(res, TW_BAD_IMAGE_FORMAT, "Can't open expected image"); return res->code; }
     if (!target || tw_ < 1 || th_ < 1) { fill_error(res, TW_BAD_IMAGE_FORMAT, "Can't open target image"); return res->code; }
@@ -1635,6 +1764,18 @@ int tw_change_regions(tw_ctx *ctx, int pair, tw_change_region *out, int cap, int
     return TW_OK;
 }
 
+int tw_intensity_cells(tw_ctx *ctx, int pair, tw_intensity_cell *out, int cap, int *n_cells)
+{
+    if (!ctx) return TW_BAD_PARAMETER;
+    if (ctx->cell_pairs < 0) { ctx->err = "tw_intensity_cells: the last answered batch ran without \"intensity_threshold\""; return TW_BAD_PARAMETER; }
+    if (pair < 0 || pair >= ctx->cell_pairs) { ctx->err = "tw_intensity_cells: pair out of range"; return TW_BAD_PARAMETER; }
+    const int total = ctx->h_ncell[pair];
+    const int k = std::min(std::min(cap, total), kMaxIntensityCells);
+    if (out && k > 0) memcpy(out, ctx->h_cells + (size_t)pair * kMaxIntensityCells, sizeof(tw_intensity_cell) * k);
+    if (n_cells) *n_cells = total;
+    return TW_OK;
+}
+
 int tw_set_option(tw_ctx *ctx, const char *name, int value)
 {
     if (!ctx || !name) return TW_BAD_PARAMETER;
@@ -1660,6 +1801,12 @@ int tw_set_option(tw_ctx *ctx, const char *name, int value)
     if (!strcmp(name, "change_regions")) { // the batches in flight were submitted with the other setting
         if (ctx->pipe.count > 0) { ctx->err = "change_regions: collect the pending pipe batches first"; return TW_BAD_PARAMETER; }
         ctx->opt.change_regions = value ? 1 : 0;
+        return TW_OK;
+    }
+    if (!strcmp(name, "intensity_threshold")) {
+        if (value < 0 || value > 255) { ctx->err = "intensity_threshold: 0 (off) or 1 .. 255 gray levels"; return TW_BAD_PARAMETER; }
+        if (ctx->pipe.count > 0) { ctx->err = "intensity_threshold: collect the pending pipe batches first"; return TW_BAD_PARAMETER; }
+        ctx->opt.intensity = value;
         return TW_OK;
     }
     if (!strcmp(name, "tight_pitch")) {

@@ -2684,6 +2684,211 @@ cudaError_t launch_change_regions(cudaStream_t s, const ChangeRegionArgs &a)
 }
 
 // ------------------------------------------------------------------------------------------------
+// Intensity cells.  Step 1, intensity_sum_kernel: one CTA per 64 x 32 pixel tile of a pair; thread = one column of the tile and 8
+// consecutive rows, so its cell column (one division) is fixed and its cell row advances by comparison.  Before the pixels:
+//   - each cell the tile meets gets its shift from the flow at its sample point (clamped to the frame, rounded half to even, 0 for a
+//     non-finite component), once, into shared memory;
+//   - the target around the tile is staged in shared memory, clamped to the frame as the definition clamps it: rows y0 - 9 ..
+//     y0 + 40, columns x0 - 12 .. x0 + 75 (whole words where the columns lie in the frame).  A cell whose shift is at most 8 rows
+//     and 11 columns reads its 3 x 3 taps there at fixed offsets; a larger shift reads them from global memory with clamps;
+//   - the ignore test runs per pixel only when the pair has a mask or a region meets the tile.
+// The tile of E is staged too, so that every global load of the tile is issued before the first pixel waits on one.
+// A pixel's residual is the least |E - T| over the taps.  Each thread sums its pixels per cell and adds them to 32-bit shared bins
+// (a tile holds 2048 pixels of at most 255 each) when its cell changes; the bins go to the pair's per-cell totals with one global
+// atomic per (tile, cell) and total.  Integer atomics commute, so the totals do not depend on the scheduling.
+// Steps 2 and 3 read the totals in chunks of kIntChunk cells, one CTA per (chunk, pair), thread = 8 consecutive cells: step 2
+// counts the intensity cells of each chunk, step 3 adds up the counts of the chunks before its own and writes its cells from there
+// in scan order (block scan, as sample_body).  Step 3 also clears the totals it read: they are zero between runs (they are cleared
+// once when allocated), so no memset runs per step.
+// ------------------------------------------------------------------------------------------------
+constexpr int kIntTileW = 64, kIntTileH = 32, kIntRows = 8;            // 64 columns x 4 row groups = 256 threads
+constexpr int kIntHaloY = 9, kIntHaloX = 12;                          // staged rows / columns on each side of the tile
+constexpr int kIntStageW = kIntTileW + 2 * kIntHaloX, kIntStageH = kIntTileH + 2 * kIntHaloY;
+
+__device__ __forceinline__ int intensity_shift(float f, int lim)
+{
+    if (!isfinite(f)) return 0;
+    return __float2int_rn(fminf(fmaxf(f, (float)-lim), (float)lim));
+}
+
+__global__ void __launch_bounds__(256) intensity_sum_kernel(IntensityArgs a)
+{
+    __shared__ unsigned bin_s[kIntTileW * kIntTileH], bin_n[kIntTileW * kIntTileH];
+    __shared__ int2 bin_shift[kIntTileW * kIntTileH];
+    __shared__ __align__(16) uint8_t st[kIntStageH * kIntStageW];
+    __shared__ __align__(16) uint8_t se[kIntTileH * kIntTileW];
+    __shared__ int4 rects[kMaxIgnore];
+    const int b = blockIdx.z, w = a.d.w, h = a.d.h, span = a.span;
+    const int x0 = blockIdx.x * kIntTileW, y0 = blockIdx.y * kIntTileH;
+    const int x1 = min(x0 + kIntTileW, w), y1 = min(y0 + kIntTileH, h);
+    const int cx0 = x0 / span, cy0 = y0 / span;
+    const int ncx = (x1 - 1) / span - cx0 + 1, ncy = (y1 - 1) / span - cy0 + 1; // the tile's cells: at most 64 x 32
+    const int tid = threadIdx.y * blockDim.x + threadIdx.x;
+    const float *fxp = a.flow + (size_t)b * 2 * a.d.plane, *fyp = fxp + a.d.plane;
+    for (int i = tid; i < ncx * ncy; i += 256) {
+        bin_s[i] = 0; bin_n[i] = 0;
+        const size_t o = (size_t)((cy0 + i / ncx) * span) * a.d.pitch + (size_t)(cx0 + i % ncx) * span;
+        bin_shift[i] = make_int2(intensity_shift(__ldg(fxp + o), w), intensity_shift(__ldg(fyp + o), h));
+    }
+    const int nr = a.g.n ? min(a.g.n[b], kMaxIgnore) : 0;
+    bool meets = false;
+    if (tid < nr) {
+        const int4 q = a.g.rects[(size_t)b * kMaxIgnore + tid];
+        rects[tid] = q;
+        meets = q.x < x1 && q.z > x0 && q.y < y1 && q.w > y0;
+    }
+    const uint8_t *mask = a.k.m && a.k.has[b] ? a.k.m + (size_t)b * a.k.H * a.k.spitch : nullptr;
+    const uint8_t *E = a.src + (size_t)b * 2 * h * a.spitch, *T = E + (size_t)h * a.spitch;
+    const int sx0 = x0 - kIntHaloX, sy0 = y0 - kIntHaloY;
+    if (sx0 >= 0 && sx0 + kIntStageW <= w) { // whole words: x0 and spitch are multiples of 16
+        for (int i = tid; i < kIntStageH * (kIntStageW / 4); i += 256) {
+            const int r = i / (kIntStageW / 4), c = i - r * (kIntStageW / 4);
+            const int gy = min(max(sy0 + r, 0), h - 1);
+            reinterpret_cast<unsigned *>(st)[i] = __ldg(reinterpret_cast<const unsigned *>(T + (size_t)gy * a.spitch + sx0) + c);
+        }
+    } else {
+        for (int i = tid; i < kIntStageH * kIntStageW; i += 256) {
+            const int r = i / kIntStageW, c = i - r * kIntStageW;
+            st[i] = __ldg(T + (size_t)min(max(sy0 + r, 0), h - 1) * a.spitch + min(max(sx0 + c, 0), w - 1));
+        }
+    }
+    for (int i = tid; i < kIntTileH * (kIntTileW / 4); i += 256) { // E: whole words of the tile's rows, up to the row pitch
+        const int r = i / (kIntTileW / 4), c = 4 * (i - r * (kIntTileW / 4));
+        if (y0 + r < h && x0 + c < a.spitch)
+            reinterpret_cast<unsigned *>(se)[i] = __ldg(reinterpret_cast<const unsigned *>(E + (size_t)(y0 + r) * a.spitch + x0 + c));
+    }
+    const bool test_ignore = __syncthreads_or(meets || mask != nullptr);
+    const SkipRegions in_region{rects, nr};
+    const int x = x0 + threadIdx.x, ya = y0 + threadIdx.y * kIntRows;
+    if (x < w && ya < h) {
+        const int cx = x / span, yb = min(ya + kIntRows, h);
+        int cy = ya / span, next = (cy + 1) * span;
+        int bin = (cy - cy0) * ncx + (cx - cx0);
+        int2 sh = bin_shift[bin];
+        bool near = abs(sh.x) < kIntHaloX && abs(sh.y) < kIntHaloY;
+        unsigned s = 0, n = 0;
+        for (int y = ya; y < yb; y++) {
+            if (y >= next) { // the next cell down
+                if (n > 0) { atomicAdd(&bin_s[bin], s); atomicAdd(&bin_n[bin], n); }
+                s = 0; n = 0;
+                cy++; next += span; bin += ncx;
+                sh = bin_shift[bin];
+                near = abs(sh.x) < kIntHaloX && abs(sh.y) < kIntHaloY;
+            }
+            if (test_ignore && ((mask && mask[(size_t)y * a.k.spitch + x]) || in_region(x, y))) continue;
+            const int e = se[(y - y0) * kIntTileW + threadIdx.x];
+            int r = 255;
+            if (near) {
+                const uint8_t *c = st + (y - sy0 + sh.y) * kIntStageW + (x - sx0 + sh.x);
+#pragma unroll
+                for (int v = -1; v <= 1; v++)
+#pragma unroll
+                    for (int u = -1; u <= 1; u++) r = min(r, abs(e - (int)c[v * kIntStageW + u]));
+            } else {
+#pragma unroll
+                for (int v = -1; v <= 1; v++) {
+                    const uint8_t *row = T + (size_t)min(max(y + sh.y + v, 0), h - 1) * a.spitch;
+#pragma unroll
+                    for (int u = -1; u <= 1; u++) r = min(r, abs(e - (int)__ldg(row + min(max(x + sh.x + u, 0), w - 1))));
+                }
+            }
+            s += r; n++;
+        }
+        if (n > 0) { atomicAdd(&bin_s[bin], s); atomicAdd(&bin_n[bin], n); }
+    }
+    __syncthreads();
+    const int nsx = (w + span - 1) / span;
+    for (int i = tid; i < ncx * ncy; i += 256) {
+        const unsigned bn = bin_n[i];
+        if (bn == 0) continue;
+        const size_t c = (size_t)b * a.cell_cap + (size_t)(cy0 + i / ncx) * nsx + cx0 + i % ncx;
+        atomicAdd(a.sum + c, (unsigned long long)bin_s[i]);
+        atomicAdd(a.cnt + c, bn);
+    }
+}
+
+struct DevIntensityCell { int x, y, n, residual; }; // tw_intensity_cell
+
+// Flags of the 8 cells [i0, i0 + 8) of a pair (bit j: cell i0 + j; cells past ns are not flagged).
+__device__ __forceinline__ unsigned intensity_flags(const IntensityArgs &a, const unsigned long long *sum, const unsigned *cnt, int i0, int ns)
+{
+    unsigned f = 0;
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+        const int i = i0 + j;
+        const unsigned n = i < ns ? cnt[i] : 0u;
+        const unsigned long long s = i < ns ? sum[i] : 0ull;
+        f |= (n > 0 && s > (unsigned long long)a.t * n) ? 1u << j : 0u;
+    }
+    return f;
+}
+
+__global__ void __launch_bounds__(1024) intensity_count_kernel(IntensityArgs a)
+{
+    __shared__ int warp_sums[32];
+    __shared__ int total;
+    const int b = blockIdx.y, k = blockIdx.x;
+    const int ns = ((a.d.w + a.span - 1) / a.span) * ((a.d.h + a.span - 1) / a.span);
+    const int i0 = k * kIntChunk + threadIdx.x * 8;
+    const unsigned f = intensity_flags(a, a.sum + (size_t)b * a.cell_cap, a.cnt + (size_t)b * a.cell_cap, i0, ns);
+    block_exclusive_scan(__popc(f), warp_sums, &total);
+    if (threadIdx.x == 0) a.chunk_counts[(size_t)b * a.max_chunks + k] = total;
+}
+
+__global__ void __launch_bounds__(1024) intensity_compact_kernel(IntensityArgs a)
+{
+    __shared__ int warp_sums[32];
+    __shared__ int total;
+    const int b = blockIdx.y, k = blockIdx.x;
+    const int nsx = (a.d.w + a.span - 1) / a.span, ns = nsx * ((a.d.h + a.span - 1) / a.span);
+    // the cells of the chunks before this one
+    int before = 0;
+    for (int j = threadIdx.x; j < k; j += blockDim.x) before += a.chunk_counts[(size_t)b * a.max_chunks + j];
+    block_exclusive_scan(before, warp_sums, &total);
+    const int base = total;
+    __syncthreads(); // every thread has read `total` before the next scan writes it
+    unsigned long long *sum = a.sum + (size_t)b * a.cell_cap;
+    unsigned *cnt = a.cnt + (size_t)b * a.cell_cap;
+    const int i0 = k * kIntChunk + threadIdx.x * 8;
+    unsigned f = intensity_flags(a, sum, cnt, i0, ns);
+    int pos = base + block_exclusive_scan(__popc(f), warp_sums, &total);
+    if (k == gridDim.x - 1 && threadIdx.x == 0) a.n_cells[b] = base + total;
+    DevIntensityCell *out = reinterpret_cast<DevIntensityCell *>(a.cells) + (size_t)b * kMaxIntensityCells;
+    for (; f && pos < kMaxIntensityCells; f &= f - 1, pos++) {
+        const int i = i0 + __ffs(f) - 1;
+        const int sy = i / nsx, sx = i - sy * nsx;
+        out[pos] = DevIntensityCell{sx * a.span, sy * a.span, (int)cnt[i], (int)min(sum[i], 0x7fffffffull)};
+    }
+    __syncthreads(); // the chunk's totals are read (above, by the thread that owns each cell) before they are cleared, coalesced
+    for (int i = k * kIntChunk + threadIdx.x; i < min((k + 1) * kIntChunk, ns); i += blockDim.x) { sum[i] = 0; cnt[i] = 0; }
+}
+
+int intensity_chunks(int w, int h, int span)
+{
+    const int ns = ((w + span - 1) / span) * ((h + span - 1) / span);
+    return (ns + kIntChunk - 1) / kIntChunk;
+}
+
+cudaError_t launch_intensity_sum(cudaStream_t s, const IntensityArgs &a)
+{
+    const dim3 grid((a.d.w + kIntTileW - 1) / kIntTileW, (a.d.h + kIntTileH - 1) / kIntTileH, a.batch);
+    intensity_sum_kernel<<<grid, dim3(kIntTileW, kIntTileH / kIntRows), 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_intensity_count(cudaStream_t s, const IntensityArgs &a)
+{
+    intensity_count_kernel<<<dim3(intensity_chunks(a.d.w, a.d.h, a.span), a.batch), kIntChunk / 8, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_intensity_compact(cudaStream_t s, const IntensityArgs &a)
+{
+    intensity_compact_kernel<<<dim3(intensity_chunks(a.d.w, a.d.h, a.span), a.batch), kIntChunk / 8, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------------
 // Ignore regions, step 1: the expected pixels inside each region replace the target's (after the +-5 px resize, before the level
 // images).  One CTA per (region, pair); warp = row, lane = 16-byte column where the row segment is aligned, bytes at its ends.
 // The expected and target slots of a pair share their alignment (spitch and H * spitch are multiples of 16).  Overlapping regions

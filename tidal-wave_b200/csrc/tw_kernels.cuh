@@ -205,4 +205,35 @@ struct ChangeRegionArgs {
 };
 cudaError_t launch_change_regions(cudaStream_t s, const ChangeRegionArgs &a);
 
+// Intensity cells (tw_intensity_cells): the span cells whose pixels changed where the flow found no motion.  Cell (i, j) is
+// [i * span, min(i * span + span, w)) x [j * span, min(j * span + span, h)); its shift is the rounded flow at its sample point.
+// launch_intensity_sum sums, per cell, the residual r(p) = min over the 3 x 3 neighbours of the shifted target pixel of
+// |E(p) - T| and the count of pixels not ignored (regions, mask); launch_intensity_count counts the cells with n > 0 and S > t * n
+// per chunk of kIntChunk cells, and launch_intensity_compact writes them in scan order and clears the totals it read.  All
+// arithmetic is integer, so the sums are exact whatever the order of the atomics.
+constexpr int kMaxIntensityCells = 4096; // TW_MAX_INTENSITY_CELLS
+constexpr int kIntChunk = 8192;          // cells per CTA of the count and compact steps
+struct IntensityArgs {
+    const uint8_t *src;       // [B][2][h][spitch]: expected, then the target as the flow saw it (resized, painted)
+    int spitch;
+    const float *flow;        // [B][2] planes of the finest scale: the flow at every sample point
+    LevelDims d;
+    int span;
+    int t;                    // threshold in gray levels, 1 .. 255
+    IgnoreRegions g;          // g.n == NULL: no pair has regions
+    IgnoreMasks k;            // k.m == NULL: no pair has a mask
+    unsigned long long *sum;  // [B][cell_cap] residual sums S: zero before launch_intensity_sum, zero again after the compaction
+    unsigned int *cnt;        // [B][cell_cap] pixel counts n, likewise
+    int cell_cap;             // >= ceil(w / span) * ceil(h / span)
+    int *chunk_counts;        // [B][max_chunks] intensity cells per chunk
+    int max_chunks;           // >= intensity_chunks(w, h, span)
+    int *n_cells;             // [B] flagged cells (full count)
+    void *cells;              // [B][kMaxIntensityCells] tw_intensity_cell
+    int batch;
+};
+int intensity_chunks(int w, int h, int span);
+cudaError_t launch_intensity_sum(cudaStream_t s, const IntensityArgs &a);
+cudaError_t launch_intensity_count(cudaStream_t s, const IntensityArgs &a);
+cudaError_t launch_intensity_compact(cudaStream_t s, const IntensityArgs &a);
+
 } // namespace tw

@@ -51,6 +51,8 @@ struct Slot {
     std::vector<tw_vector> vectors;
     std::vector<tw_change_region> regions; // the first TW_MAX_CHANGE_REGIONS of n_regions (pools with change regions)
     int n_regions = 0;
+    std::vector<tw_intensity_cell> cells;  // the first TW_MAX_INTENSITY_CELLS of n_cells (pools with intensity cells)
+    int n_cells = 0;
 };
 
 } // namespace
@@ -70,6 +72,7 @@ struct tw_pool {
     int decoding = 0;                     // jobs a decoder thread is working on
     int n_decoders = 0;                   // 0: one per host core (at most 32)
     bool change_regions = false;          // fixed by the first submit (tw_pool_set_change_regions)
+    int intensity = 0;                    // "intensity_threshold", fixed likewise (tw_pool_set_intensity)
     std::unordered_map<long long, Slot> slots;
     bool running = true;
     long long next_id = 0;
@@ -98,7 +101,7 @@ void fill_error(tw_result *r, int code, const char *msg)
 }
 
 void publish(tw_pool *p, long long id, const tw_result &res, const tw_vector *vec, int nvec, const tw_change_region *reg = nullptr,
-             int n_regions = 0)
+             int n_regions = 0, const tw_intensity_cell *cells = nullptr, int n_cells = 0)
 {
     std::lock_guard<std::mutex> lk(p->mu);
     Slot &s = p->slots[id];
@@ -107,6 +110,10 @@ void publish(tw_pool *p, long long id, const tw_result &res, const tw_vector *ve
     if (reg && n_regions > 0) {
         s.n_regions = n_regions;
         s.regions.assign(reg, reg + std::min(n_regions, TW_MAX_CHANGE_REGIONS));
+    }
+    if (cells && n_cells > 0) {
+        s.n_cells = n_cells;
+        s.cells.assign(cells, cells + std::min(n_cells, TW_MAX_INTENSITY_CELLS));
     }
     s.done = true;
     if (res.status == TW_STATUS_ERROR) p->error_count++; else p->data_count++; // Manager::notify, src/manager.cpp:109-114
@@ -280,14 +287,18 @@ void consumer_main(tw_pool *p, int idx)
     std::vector<const tw_rect *> ig(p->batch);
     std::vector<int> nig(p->batch);
     std::vector<const uint8_t *> mk(p->batch);
-    // change regions: the pool's setting is fixed once a request exists, so it is applied before this consumer's first batch
+    // change regions and the intensity threshold: the pool's settings are fixed once a request exists, so they are applied before
+    // this consumer's first batch
     bool regions = false, regions_set = false;
+    int intensity = 0;
     std::vector<tw_change_region> reg(TW_MAX_CHANGE_REGIONS);
-    // publishes pair i of the batch the context answered last, with its change regions
+    std::vector<tw_intensity_cell> cells(TW_MAX_INTENSITY_CELLS);
+    // publishes pair i of the batch the context answered last, with its change regions and intensity cells
     auto publish_pair = [&](long long id, int i, const tw_result &r, const tw_vector *v, int nv) {
-        int nreg = 0;
+        int nreg = 0, ncell = 0;
         if (regions && tw_change_regions(ctx, i, reg.data(), TW_MAX_CHANGE_REGIONS, &nreg) != TW_OK) nreg = 0;
-        publish(p, id, r, v, nv, reg.data(), nreg);
+        if (intensity && tw_intensity_cells(ctx, i, cells.data(), TW_MAX_INTENSITY_CELLS, &ncell) != TW_OK) ncell = 0;
+        publish(p, id, r, v, nv, reg.data(), nreg, cells.data(), ncell);
     };
     // Up to two batches are in flight on the context (tw_pipe_*): while batch k runs, this thread pops and uploads batch k + 1
     // and then collects batch k - 1 -- one consumer thread per GPU keeps the device busy (src/consumer.cpp:18-24).
@@ -348,8 +359,10 @@ void consumer_main(tw_pool *p, int idx)
             {
                 std::lock_guard<std::mutex> lk(p->mu);
                 regions = p->change_regions;
+                intensity = p->intensity;
             }
             tw_set_option(ctx, "change_regions", regions ? 1 : 0); // nothing in flight yet
+            tw_set_option(ctx, "intensity_threshold", intensity);
             regions_set = true;
         }
         int cap = p->vector_cap;
@@ -397,7 +410,8 @@ void consumer_main(tw_pool *p, int idx)
 }
 
 int take(tw_pool *p, std::unordered_map<long long, Slot>::iterator it, tw_vector *out, int cap, tw_result *res,
-         tw_change_region *regions = nullptr, int region_cap = 0, int *n_regions = nullptr)
+         tw_change_region *regions = nullptr, int region_cap = 0, int *n_regions = nullptr, tw_intensity_cell *cells = nullptr,
+         int cell_cap = 0, int *n_cells = nullptr)
 {
     Slot &s = it->second;
     if (s.dropped) { p->slots.erase(it); return -1; }
@@ -407,6 +421,9 @@ int take(tw_pool *p, std::unordered_map<long long, Slot>::iterator it, tw_vector
     const int k = std::min<int>((int)s.regions.size(), region_cap);
     if (regions && k > 0) memcpy(regions, s.regions.data(), sizeof(tw_change_region) * k);
     if (n_regions) *n_regions = s.n_regions;
+    const int kc = std::min<int>((int)s.cells.size(), cell_cap);
+    if (cells && kc > 0) memcpy(cells, s.cells.data(), sizeof(tw_intensity_cell) * kc);
+    if (n_cells) *n_cells = s.n_cells;
     int code = s.res.code;
     p->slots.erase(it);
     return code;
@@ -527,8 +544,17 @@ int tw_pool_set_change_regions(tw_pool *p, int on)
     return TW_OK;
 }
 
-int tw_pool_wait_regions(tw_pool *p, long long id, tw_vector *out, int cap, tw_result *res, tw_change_region *regions, int region_cap,
-                         int *n_regions)
+int tw_pool_set_intensity(tw_pool *p, int t)
+{
+    if (!p || t < 0 || t > 255) return TW_BAD_PARAMETER;
+    std::lock_guard<std::mutex> lk(p->mu);
+    if (p->next_id > 0) return TW_BAD_PARAMETER; // a consumer may already run with the old setting
+    p->intensity = t;
+    return TW_OK;
+}
+
+int tw_pool_wait_intensity(tw_pool *p, long long id, tw_vector *out, int cap, tw_result *res, tw_change_region *regions, int region_cap,
+                           int *n_regions, tw_intensity_cell *cells, int cell_cap, int *n_cells)
 {
     if (!p) return -1;
     std::unique_lock<std::mutex> lk(p->mu);
@@ -536,7 +562,13 @@ int tw_pool_wait_regions(tw_pool *p, long long id, tw_vector *out, int cap, tw_r
     if (it == p->slots.end()) return -1;
     p->cv_res.wait(lk, [&] { it = p->slots.find(id); return it == p->slots.end() || it->second.done || it->second.dropped; });
     if (it == p->slots.end()) return -1;
-    return take(p, it, out, cap, res, regions, region_cap, n_regions);
+    return take(p, it, out, cap, res, regions, region_cap, n_regions, cells, cell_cap, n_cells);
+}
+
+int tw_pool_wait_regions(tw_pool *p, long long id, tw_vector *out, int cap, tw_result *res, tw_change_region *regions, int region_cap,
+                         int *n_regions)
+{
+    return tw_pool_wait_intensity(p, id, out, cap, res, regions, region_cap, n_regions, nullptr, 0, nullptr);
 }
 
 int tw_pool_wait(tw_pool *p, long long id, tw_vector *out, int cap, tw_result *res)

@@ -13,7 +13,9 @@ short path as the target; a pair with no file there has no mask) or, if that is 
 cannot be decoded, or of another size than the expected image, makes that pair an 'error' event.  Wrong-typed values of these
 options mean "no mask", as for the reference's options.  ``changeRegions`` (only ``True`` turns it on) adds ``regions`` and
 ``n_regions`` to every 'data' event: where the page changed, as connected groups of its suspicious sample points
-(include/tidalwave_b200.h, tw_change_regions).  Files are decoded with ``imread_gray`` (PNG / JPEG / PGM,
+(include/tidalwave_b200.h, tw_change_regions).  ``intensityThreshold`` (an integer from 1 to 255 gray levels; anything else
+leaves it off) adds ``intensity_cells`` and ``n_intensity_cells`` to every 'data' event and makes a pair with intensity cells
+SUSPICIOUS: the span cells whose pixels changed where the flow found no motion (tw_intensity_cells).  Files are decoded with ``imread_gray`` (PNG / JPEG / PGM,
 bit-exact to cv::imread IMREAD_GRAYSCALE); a file that cannot be decoded becomes the reference's "Can't open <path>" error.
 """
 from __future__ import annotations
@@ -51,6 +53,8 @@ class TidalWave:
         self.ignoreMaskDir = o.get("ignoreMaskDir") if isinstance(o.get("ignoreMaskDir"), str) else None
         self.getIgnoreMaskPath = o.get("getIgnoreMaskPath") if callable(o.get("getIgnoreMaskPath")) else None
         self.changeRegions = o.get("changeRegions") is True
+        t = _int32(o, "intensityThreshold", 0)
+        self.intensityThreshold = t if 1 <= t <= 255 else 0
         self._handlers = {"data": [], "error": [], "finish": []}
         self._pending = []   # (request id | None, expect path, target path, immediate error | None)
         self._report = {"request": 0, "data": 0, "error": 0}
@@ -76,7 +80,7 @@ class TidalWave:
             devices = self._devices or [i % ndev for i in range(max(1, self.numThreads))]  # consumer i <-> GPU i % count
             # screenshot directories mix page sizes: no size bound, and every vector of every pair comes back whatever its size
             self._pool = Pool(devices, self.param, self.threshold, self.span, max_w=0, max_h=0, batch=self._batch, vector_cap=0,
-                              change_regions=self.changeRegions)
+                              change_regions=self.changeRegions, intensity_threshold=self.intensityThreshold)
             load().tw_pool_set_decoders(self._pool.pool, max(1, self.numThreads))
         return self._pool
 
